@@ -17,6 +17,11 @@ replicated-database run of the same shape.  `--shard m` runs only that section (
 --impl reference times the reference's own CPU implementation on the host cores: the UNMODIFIED mvrl/RANGE package
 (oracle/_ref/reference, staged by __graft_entry__.build(); oracle/ref_harness.py) when it is there, else the oracle
 port, on a bounded sample of the same workload.
+
+--dump-outputs DIR (rank 0) writes what the last timed step returned, so that two builds can be compared output for
+output on the same seeded inputs: DIR/embeddings.npy (float32, the step's (N,1280) result) and
+DIR/model_embeddings.npy (float64, the (N,1280) array `model(locs)` returns), both as the same fixed sample of
+DUMP_ROWS rows (dump_rows()), 47 MB in all.
 """
 import argparse
 import contextlib
@@ -45,6 +50,12 @@ METRIC = "RANGE+ embeddings/sec"
 UNIT = "queries/s"
 REF_SAMPLE_QUERIES = 5000       # per step of the reference arm: each N x M fp32 matrix it materialises is 2 GB
 WORKLOAD = f"RANGE+ beta={BETA}, M={M_DB} (range_db_large shape), SatCLIP-L40 H={H} random-init"
+DUMP_ROWS = 3072                # 3072 x 1280 x (4 + 8) B = 47 MB: the dump stays under 64 MB
+
+
+def dump_rows():
+    """the rows --dump-outputs writes: a fixed seeded sample of the N_QUERIES result rows, in increasing order"""
+    return np.sort(np.random.default_rng(0).choice(N_QUERIES, DUMP_ROWS, replace=False))
 
 
 def synthetic_inputs(rank=0, M=M_DB, n=N_QUERIES):
@@ -322,7 +333,12 @@ def main():
     ap.add_argument("--m-sizes", default="", help="comma-separated database sizes of the M-sharded section")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="skip the extras (reference arm: config 1 / port / eager CUDA)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.shard == "m"):
+        ap.error("--dump-outputs writes the outputs of the headline path (--impl range_b200 --shard query)")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -402,6 +418,10 @@ def main():
         clocks.mark_end()
     launches = _lib.launch_count() - launches0
     ms = t0.elapsed_time(t1)
+    dump = {}
+    if args.dump_outputs and rank == 0:
+        rows = dump_rows()
+        dump["embeddings"] = out[torch.from_numpy(rows).to(dev)].cpu().numpy()
     seg = np.array([[e[i].elapsed_time(e[i + 1]) for i in range(3)] + [0.0, e[5].elapsed_time(e[0])]
                     for e in marks]).mean(0)                                   # enc, stats, apply+concat, -, sort
 
@@ -418,6 +438,8 @@ def main():
     barrier()
     e2e_s = (time.perf_counter() - w0)
     assert res.shape == (N_QUERIES, 1280) and res.dtype == np.float64
+    if dump:
+        dump["model_embeddings"] = res[rows]
     host_path = model.host_path if model.host_path != "auto" else "copy"
     del res
     # opt-in (NOT the reference's dtype, not the headline): float32 rows halve the device->host bytes
@@ -513,6 +535,10 @@ def main():
             qps, sec = ref.time("RANGE+", M_DB, n, steps=2, warmup=1)
             line["cpu_baseline"] = {"value": qps, "unit": UNIT, "cores": torch.get_num_threads(), "kind": ref.kind,
                                     "sample": f"{n} of {N_QUERIES} queries x full {M_DB}-entry DB, 2 calls ({sec:.1f} s each)"}
+        if dump:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dump.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
