@@ -179,6 +179,20 @@ int range_retrieve_concat(range_ctx* ctx, int mode, int64_t N, const void* q16, 
                           float geo_temp, float beta, const double* q64, const int32_t* perm, void* out, int out_dtype,
                           void* workspace, size_t workspace_bytes, void* stream);
 
+/* Retrieval neighbours: which database entries an embedding is made of.  The weight of entry j for a query is the
+ * coefficient range/range.py:213-238 multiplies V[j] by - RANGE: softmax(temp S)_j; RANGE+: (1-beta) softmax(geo_temp G)_j
+ * + beta softmax(temp S)_j - computed with the row sums `sums` (N,2) of range_retrieve_stats.  For every query: the k
+ * (1 <= k <= RANGE_TOPK_MAX, k <= M) largest weights over THIS ctx's database rows, descending, equal fp32 weights by
+ * smaller row; idx (N,k) int32 = device database rows 0..M-1 of this ctx (the caller maps them to its own row order),
+ * weight (N,k) fp32.  Row n of the result goes to row perm[n] (perm from range_sort_queries; NULL = identity).  With
+ * the global sums of an M-sharded database each shard returns its local top k, which merge by weight.  A separate
+ * pass over the database: range_retrieve_* are unaffected. */
+#define RANGE_TOPK_MAX 32
+size_t range_topk_workspace_bytes(range_ctx* ctx, int64_t N, int k);
+int range_retrieve_topk(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
+                        float geo_temp, float beta, const float* sums, int k, const int32_t* perm, int32_t* idx,
+                        float* weight, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- M-sharded database (one process per GPU, rank r holds rows [r M/P, (r+1) M/P) of the database) ----
  * The softmax-weighted sums of range/range.py:213-217,231-238 are associative in the database axis: with the fixed
  * offset (|s|,|g| <= 1) the per-shard exp-sums of range_retrieve_stats merge by SUM (one all-reduce of 8 B per query),

@@ -14,6 +14,7 @@ RANGE_MODE_RANGE, RANGE_MODE_RANGE_PLUS = 0, 1
 RANGE_OUT_F64, RANGE_OUT_F32, RANGE_OUT_PACKED = 0, 1, 2
 RANGE_MAX_RANKS = 8
 RANGE_ENC_F64, RANGE_ENC_F16X3 = 0, 1
+RANGE_TOPK_MAX = 32
 
 # every symbol include/range_b200.h declares: name -> (restype, argtypes)
 PROTOTYPES = {
@@ -57,6 +58,9 @@ PROTOTYPES = {
                                c_void_p, c_size_t, c_void_p]),
     "range_retrieve_concat": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float, c_void_p,
                                       c_void_p, c_void_p, c_int, c_void_p, c_size_t, c_void_p]),
+    "range_topk_workspace_bytes": (c_size_t, [c_void_p, c_int64, c_int]),
+    "range_retrieve_topk": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float, c_void_p,
+                                    c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "range_retrieve_apply_routed": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float,
                                             c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "range_combine_concat": (c_int, [c_void_p, c_int64, c_int, POINTER(c_void_p), POINTER(c_float), c_void_p, c_void_p,

@@ -328,6 +328,30 @@ int fill_args(range_ctx* c, int mode, int64_t N, const void* q16, const float* q
   return RANGE_OK;
 }
 
+// Neighbours pass: the statistics plan's database splits (at most kTopkMaxSplits: the merge takes 2 lists per split and
+// CTA), its geo-skip mask, then the partial lists [2 * splits][N][k] (weight, entry).
+struct TopkPlan {
+  RetrievalPlan ret;                        // only the mask fields are used; ret.off_mask is relative to this workspace
+  int splits, tiles_per_split;
+  size_t off_w, off_idx, total;
+};
+
+TopkPlan plan_topk(const range_ctx* c, int64_t N, int k) {
+  TopkPlan t;
+  t.ret = plan_retrieval(c, N);
+  const int64_t tiles = (c->M + kBlockKeys - 1) / kBlockKeys;
+  const int64_t want = std::min<int64_t>(t.ret.stats_splits, kTopkMaxSplits);
+  t.tiles_per_split = int((tiles + want - 1) / want);
+  t.splits = int((tiles + t.tiles_per_split - 1) / t.tiles_per_split);
+  const size_t lists = size_t(2 * t.splits) * size_t(N) * size_t(k) * 4;
+  size_t o = 0;
+  t.ret.off_mask = o; o += c->caps ? align_up(size_t(t.ret.mask_rows) * t.ret.mask_words * 4, 256) : 0;
+  t.off_w = o;        o += align_up(lists, 256);
+  t.off_idx = o;      o += align_up(lists, 256);
+  t.total = o;
+  return t;
+}
+
 }  // namespace
 
 extern "C" {
@@ -921,6 +945,35 @@ int range_retrieve_concat(range_ctx* c, int mode, int64_t N, const void* q16, co
   if (r) return r;
   return range_retrieve_apply_concat(c, mode, N, q16, qxyz, temp, geo_temp, beta, sums, maxs, q64, perm, out, out_dtype,
                                      workspace, workspace_bytes, stream);
+}
+
+size_t range_topk_workspace_bytes(range_ctx* c, int64_t N, int k) {
+  if (!c || !c->Kh || N <= 0 || N > (int64_t(1) << 30) || k < 1 || k > RANGE_TOPK_MAX) return 0;
+  return plan_topk(c, N, k).total + 256;
+}
+
+int range_retrieve_topk(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
+                        float geo_temp, float beta, const float* sums, int k, const int32_t* perm, int32_t* idx,
+                        float* weight, void* workspace, size_t workspace_bytes, void* stream) {
+  static_assert(RANGE_TOPK_MAX == kTopkMax, "topk.cu list buckets");
+  if (!c || !c->Kh) return fail(RANGE_ERR_INVALID, "database not set");
+  if (!q16 || !qxyz || !sums || !idx || !weight || !workspace) return fail(RANGE_ERR_INVALID, "null argument");
+  if (N <= 0) return fail(RANGE_ERR_INVALID, "N must be positive");
+  if (k < 1 || k > RANGE_TOPK_MAX || k > c->M)
+    return fail(RANGE_ERR_INVALID, "k = %d: need 1 <= k <= %d and k <= M = %lld", k, RANGE_TOPK_MAX, (long long)c->M);
+  if (mode == RANGE_MODE_RANGE_PLUS && !(beta >= 0.f && beta <= 1.f))
+    return fail(RANGE_ERR_INVALID, "beta must be in [0,1]");
+  if (workspace_bytes < range_topk_workspace_bytes(c, N, k)) return fail(RANGE_ERR_WORKSPACE, "top-k workspace too small");
+  const TopkPlan t = plan_topk(c, N, k);
+  RetrievalArgs a;
+  char* ws = reinterpret_cast<char*>(align_up(reinterpret_cast<size_t>(workspace), 256));
+  cudaStream_t s = cudaStream_t(stream);
+  int r = fill_args(c, mode, N, q16, qxyz, temp, geo_temp, t.ret, ws, s, &a, sums);     // apply-pass geo-skip mask
+  if (r) return r;
+  CUDA_TRY(launch_topk(a, t.splits, t.tiles_per_split, sums, beta, k, reinterpret_cast<float*>(ws + t.off_w),
+                       reinterpret_cast<int32_t*>(ws + t.off_idx), perm, idx, weight, s));
+  g_launches += 2;
+  return RANGE_OK;
 }
 
 int range_retrieve_apply_routed(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp,

@@ -154,6 +154,25 @@ __device__ __forceinline__ void tmem_st16(uint32_t taddr, const uint32_t (&v)[16
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
+// Q tile (rows q0..q0+127 of q16, 256 halves each) -> TMEM columns [tmem_q, tmem_q+128): lane = row,
+// column = dim / 2 (two fp16 per 32-bit column) - the A-operand layout of kind::f16 for M = 128.
+// 16 warps: warp w writes lanes 32 (w%4).., column group w/4 = dims [64 g, 64 g + 64).
+__device__ __forceinline__ void load_q_to_tmem16(const __half* __restrict__ q16, int q0, int N, uint32_t tmem_q,
+                                                 int warp, int lane) {
+  const int grp = warp >> 2, quarter = warp & 3;
+  const int n = q0 + quarter * 32 + lane;
+  const uint4* src = reinterpret_cast<const uint4*>(q16 + size_t(n < N ? n : 0) * 256 + grp * 64);
+  uint32_t v[32];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) {
+    uint4 x = make_uint4(0u, 0u, 0u, 0u);
+    if (n < N) x = __ldg(src + i);
+    v[4 * i] = x.x; v[4 * i + 1] = x.y; v[4 * i + 2] = x.z; v[4 * i + 3] = x.w;
+  }
+  tmem_st32(tmem_q + (uint32_t(quarter * 32) << 16) + grp * 32, v);
+  tmem_st_wait();
+}
+
 // ------------------------------------------------------------------ UMMA descriptors
 // Shared-memory matrix descriptor, K-major operand, SWIZZLE_128B, dense 8-row groups (1024 B apart).
 // Canonical layout ((8,n),2):((8,SBO),1) in 16-byte units (cute/atom/mma_traits_sm100.hpp make_umma_desc).

@@ -176,4 +176,13 @@ cudaError_t launch_stats_pc(const RetrievalArgs& a, float* part_sum, float* part
 cudaError_t launch_reduce_out(const float* part, size_t split_stride, int splits, size_t total, float* out,
                               cudaStream_t s);
 
+// ---- retrieval neighbours: the k largest retrieval weights per query (topk.cu) ------------------------------------
+constexpr int kTopkMax = 32, kTopkMaxSplits = 64;
+// a.geo selects RANGE+ (a.geo_mask: the apply-pass mask or null); sums (N,2) from the statistics pass.  Database split
+// `split` covers tiles [split * tiles_per_split, ..); partial lists part_w / part_idx [2 * splits][N][k]; result row n
+// (k entries, descending weight, then ascending entry) -> idx / weight row perm[n] (perm null: n)
+cudaError_t launch_topk(const RetrievalArgs& a, int splits, int tiles_per_split, const float* sums, float beta, int k,
+                        float* part_w, int32_t* part_idx, const int32_t* perm, int32_t* idx, float* weight,
+                        cudaStream_t s);
+
 }  // namespace rangeb200

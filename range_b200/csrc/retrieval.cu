@@ -93,25 +93,6 @@ __device__ __forceinline__ void named_bar_sync_softmax() {
   asm volatile("bar.sync 1, %0;" ::"n"(kNumSoftmaxWarps * 32) : "memory");
 }
 
-// Q tile (rows q0..q0+127 of q16, 256 halves each) -> TMEM columns [kTmemQ, kTmemQ+128): lane = row,
-// column = dim / 2 (two fp16 per 32-bit column) - the A-operand layout of kind::f16 for M = 128.
-// 16 warps: warp w writes lanes 32 (w%4).., column group w/4 = dims [64 g, 64 g + 64).
-__device__ __forceinline__ void load_q_to_tmem16(const __half* __restrict__ q16, int q0, int N, uint32_t tmem_base,
-                                                 int warp, int lane) {
-  const int grp = warp >> 2, quarter = warp & 3;
-  const int n = q0 + quarter * 32 + lane;
-  const uint4* src = reinterpret_cast<const uint4*>(q16 + size_t(n < N ? n : 0) * 256 + grp * 64);
-  uint32_t v[32];
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    uint4 x = make_uint4(0u, 0u, 0u, 0u);
-    if (n < N) x = __ldg(src + i);
-    v[4 * i] = x.x; v[4 * i + 1] = x.y; v[4 * i + 2] = x.z; v[4 * i + 3] = x.w;
-  }
-  ptx::tmem_st32(tmem_base + (uint32_t(quarter * 32) << 16) + kTmemQ + grp * 32, v);
-  ptx::tmem_st_wait();
-}
-
 // ---------------------------------------------------------------------------------------------------
 // K2a: row statistics.  Tile = 128 entries = two 32 KB stages (dims 0-127 | 128-255); Q in TMEM (TS-mode).
 // 16 softmax warps (warp w: TMEM lanes 32 (w%4).., 32-entry column group w/4) + producer + MMA issuer.
@@ -180,7 +161,7 @@ range_stats_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __rest
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);
   const uint32_t smem_u = __shfl_sync(0xffffffffu, ptx::smem_u32(smem), 0);
   const uint32_t bars_u = smem_u + L::bars;
-  if (warp < kStatsWarps) load_q_to_tmem16(q16, q0, N, tmem_base, warp, lane);
+  if (warp < kStatsWarps) ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane);
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();

@@ -303,5 +303,18 @@ class DeviceDatabase:
         self.caps = torch.from_numpy(tile_caps(xyz)).to(dev)
         return self
 
+    def file_rows(self, idx):
+        """device rows (e.g. the entries RangeEngine.retrieve_topk returns) -> rows of the database file, so that
+        db['locs'][rows] are the entries' locations: order[row_range[0] + idx], or row_range[0] + idx when the rows keep
+        the file order.  idx: integer tensor on any device; returns int64 on the same device."""
+        idx = torch.as_tensor(idx)
+        rows = idx.long() + self.row_range[0]
+        if self.order is None:
+            return rows
+        cached = getattr(self, "_order_t", None)
+        if cached is None or cached.device != idx.device:
+            cached = self._order_t = torch.from_numpy(np.asarray(self.order, dtype=np.int64)).to(idx.device)
+        return cached[rows]
+
     def nbytes(self):
         return sum(t.numel() * t.element_size() for t in (self.Kh, self.Vt, self.xyz))

@@ -256,6 +256,20 @@ class RangeEngine:
                                                      _ptr(sums), _ptr(maxs), _ptr(ws), ws.numel(), _stream()))
         return sums, maxs
 
+    def retrieve_topk(self, mode, q16, qxyz, temp, geo_temp, beta, sums, k, perm=None):
+        """the k largest retrieval weights of every query (sums from retrieve_stats): (idx (N,k) int32 device database
+        rows, weight (N,k) fp32), descending; row n of the result at row perm[n] (perm from sort_queries)"""
+        N = q16.shape[0]
+        idx = torch.empty(N, k, dtype=torch.int32, device=self.device)
+        weight = torch.empty(N, k, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.index):
+            ws = self._workspace("topk", max(1, self.lib.range_topk_workspace_bytes(self.ctx, N, k)))
+            _lib.check(self.lib.range_retrieve_topk(
+                self.ctx, MODE[mode], N, _ptr(q16), _ptr(qxyz), temp, geo_temp, 0.0 if beta is None else float(beta),
+                _ptr(sums), k, c_void_p(None) if perm is None else _ptr(perm), _ptr(idx), _ptr(weight), _ptr(ws),
+                ws.numel(), _stream()))
+        return idx, weight
+
     def retrieve_apply(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, O=None):
         N = q16.shape[0]
         O = torch.empty(N, 1024, dtype=torch.float32, device=self.device) if O is None else O

@@ -12,6 +12,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
+from . import _lib
 from .checkpoint import load_satclip_location_encoder
 from .database import DeviceDatabase, open_npz
 from .engine import RangeEngine
@@ -143,6 +144,29 @@ class LocationEncoder(nn.Module):
         O_sem = eng.retrieve_apply('RANGE', q16, qxyz, a.temp, 0.0, None, sums, maxs)
         return [eng.combine_concat([O_geo, O_sem], [1.0 - float(b), float(b)], q64, dtype=out_dtype, perm=perm)
                 for b in betas]
+
+    @torch.no_grad()
+    def neighbours(self, coords, k=8):
+        """Which database entries each embedding is made of: coords (N,2) fp64 (lon, lat) degrees -> (index (N,k) int64,
+        weight (N,k) float32) device tensors in the caller's row order.  index holds rows of the database file
+        (db['locs'][index] are the neighbours' locations), weight the coefficient the retrieved feature gives each of
+        them (range/range.py:213-238 with this model's temp, geo_temp and beta), largest first."""
+        eng, a = self.engine, self.args
+        if self.sharded is not None:
+            raise NotImplementedError('neighbours: an unsharded database')
+        k = int(k)
+        if not 1 <= k <= min(_lib.RANGE_TOPK_MAX, eng.db.M):
+            raise ValueError(f'k={k}: expected 1 <= k <= {min(_lib.RANGE_TOPK_MAX, eng.db.M)} (database of {eng.db.M} entries)')
+        coords = coords.to(eng.device, torch.float64).contiguous()
+        name = self.location_model_name
+        geo_temp = float(getattr(a, 'geo_temp', 0.0))
+        perm = None
+        if self._sorts():
+            coords, perm = eng.sort_queries(coords)
+        _, q16, qxyz = eng.encode(coords)
+        sums, _ = eng.retrieve_stats(name, q16, qxyz, a.temp, geo_temp)
+        idx, weight = eng.retrieve_topk(name, q16, qxyz, a.temp, geo_temp, getattr(a, 'beta', None), sums, k, perm=perm)
+        return eng.db.file_rows(idx), weight
 
     @staticmethod
     def _chunks(N, chunk, tail, taper=DEFAULT_TAPER):
