@@ -185,13 +185,31 @@ int range_retrieve_concat(range_ctx* ctx, int mode, int64_t N, const void* q16, 
  * (1 <= k <= RANGE_TOPK_MAX, k <= M) largest weights over THIS ctx's database rows, descending, equal fp32 weights by
  * smaller row; idx (N,k) int32 = device database rows 0..M-1 of this ctx (the caller maps them to its own row order),
  * weight (N,k) fp32.  Row n of the result goes to row perm[n] (perm from range_sort_queries; NULL = identity).  With
- * the global sums of an M-sharded database each shard returns its local top k, which merge by weight.  A separate
- * pass over the database: range_retrieve_* are unaffected. */
+ * the global sums of an M-sharded database each shard returns its local top k, which merge by weight
+ * (range_retrieve_topk_rows, range_topk_merge below).  A separate pass over the database: range_retrieve_* are
+ * unaffected. */
 #define RANGE_TOPK_MAX 32
 size_t range_topk_workspace_bytes(range_ctx* ctx, int64_t N, int k);
 int range_retrieve_topk(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
                         float geo_temp, float beta, const float* sums, int k, const int32_t* perm, int32_t* idx,
                         float* weight, void* workspace, size_t workspace_bytes, void* stream);
+
+/* A shard's list for an M-sharded database: range_retrieve_topk without perm (row n of the result is query n), with
+ * two differences.  Entry j is reported as row0 + j - with row0 = the shard's first row, a row of the whole database,
+ * so equal weights still order by the smaller (global) row: shards are ascending contiguous ranges of it.  k is only
+ * bounded by RANGE_TOPK_MAX: when the shard holds fewer than k entries the tail of each list is entry -1, weight 0.
+ * Needs row0 >= 0 and row0 + M <= INT32_MAX.  Same workspace as range_retrieve_topk. */
+int range_retrieve_topk_rows(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
+                             float geo_temp, float beta, const float* sums, int k, int64_t row0, int32_t* idx,
+                             float* weight, void* workspace, size_t workspace_bytes, void* stream);
+
+/* Merge of n_parts (1 <= n_parts <= RANGE_MAX_RANKS) lists of k entries per query, laid out [n_parts][N][k] (part_w
+ * fp32, part_idx int32), each sorted by weight descending and then by entry, -1 entries (weight 0) allowed at the tail;
+ * the parts hold disjoint entries.  Result: the k entries with the largest weights, same order and same -1 tail, row n
+ * to idx / weight row perm[n] (NULL = identity).  This is what the owner of a query receives from the P shards'
+ * range_retrieve_topk_rows lists.  Device pointers; no workspace. */
+int range_topk_merge(range_ctx* ctx, int n_parts, int64_t N, int k, const float* part_w, const int32_t* part_idx,
+                     const int32_t* perm, int32_t* idx, float* weight, void* stream);
 
 /* ---- M-sharded database (one process per GPU, rank r holds rows [r M/P, (r+1) M/P) of the database) ----
  * The softmax-weighted sums of range/range.py:213-217,231-238 are associative in the database axis: with the fixed

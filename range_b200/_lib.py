@@ -61,6 +61,10 @@ PROTOTYPES = {
     "range_topk_workspace_bytes": (c_size_t, [c_void_p, c_int64, c_int]),
     "range_retrieve_topk": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float, c_void_p,
                                     c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "range_retrieve_topk_rows": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float,
+                                         c_void_p, c_int, c_int64, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "range_topk_merge": (c_int, [c_void_p, c_int, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                 c_void_p]),
     "range_retrieve_apply_routed": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float,
                                             c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "range_combine_concat": (c_int, [c_void_p, c_int64, c_int, POINTER(c_void_p), POINTER(c_float), c_void_p, c_void_p,

@@ -952,15 +952,12 @@ size_t range_topk_workspace_bytes(range_ctx* c, int64_t N, int k) {
   return plan_topk(c, N, k).total + 256;
 }
 
-int range_retrieve_topk(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
-                        float geo_temp, float beta, const float* sums, int k, const int32_t* perm, int32_t* idx,
-                        float* weight, void* workspace, size_t workspace_bytes, void* stream) {
-  static_assert(RANGE_TOPK_MAX == kTopkMax, "topk.cu list buckets");
-  if (!c || !c->Kh) return fail(RANGE_ERR_INVALID, "database not set");
+// range_retrieve_topk (perm, k <= M, device rows) and range_retrieve_topk_rows (no perm, k past M, rows row0 + j)
+static int topk_impl(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp, float geo_temp,
+                     float beta, const float* sums, int k, const int32_t* perm, int64_t row0, int32_t* idx,
+                     float* weight, void* workspace, size_t workspace_bytes, void* stream) {
   if (!q16 || !qxyz || !sums || !idx || !weight || !workspace) return fail(RANGE_ERR_INVALID, "null argument");
   if (N <= 0) return fail(RANGE_ERR_INVALID, "N must be positive");
-  if (k < 1 || k > RANGE_TOPK_MAX || k > c->M)
-    return fail(RANGE_ERR_INVALID, "k = %d: need 1 <= k <= %d and k <= M = %lld", k, RANGE_TOPK_MAX, (long long)c->M);
   if (mode == RANGE_MODE_RANGE_PLUS && !(beta >= 0.f && beta <= 1.f))
     return fail(RANGE_ERR_INVALID, "beta must be in [0,1]");
   if (workspace_bytes < range_topk_workspace_bytes(c, N, k)) return fail(RANGE_ERR_WORKSPACE, "top-k workspace too small");
@@ -971,8 +968,41 @@ int range_retrieve_topk(range_ctx* c, int mode, int64_t N, const void* q16, cons
   int r = fill_args(c, mode, N, q16, qxyz, temp, geo_temp, t.ret, ws, s, &a, sums);     // apply-pass geo-skip mask
   if (r) return r;
   CUDA_TRY(launch_topk(a, t.splits, t.tiles_per_split, sums, beta, k, reinterpret_cast<float*>(ws + t.off_w),
-                       reinterpret_cast<int32_t*>(ws + t.off_idx), perm, idx, weight, s));
+                       reinterpret_cast<int32_t*>(ws + t.off_idx), perm, int(row0), idx, weight, s));
   g_launches += 2;
+  return RANGE_OK;
+}
+
+int range_retrieve_topk(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
+                        float geo_temp, float beta, const float* sums, int k, const int32_t* perm, int32_t* idx,
+                        float* weight, void* workspace, size_t workspace_bytes, void* stream) {
+  static_assert(RANGE_TOPK_MAX == kTopkMax, "topk.cu list buckets");
+  if (!c || !c->Kh) return fail(RANGE_ERR_INVALID, "database not set");
+  if (k < 1 || k > RANGE_TOPK_MAX || k > c->M)
+    return fail(RANGE_ERR_INVALID, "k = %d: need 1 <= k <= %d and k <= M = %lld", k, RANGE_TOPK_MAX, (long long)c->M);
+  return topk_impl(c, mode, N, q16, qxyz, temp, geo_temp, beta, sums, k, perm, 0, idx, weight, workspace,
+                   workspace_bytes, stream);
+}
+
+int range_retrieve_topk_rows(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
+                             float geo_temp, float beta, const float* sums, int k, int64_t row0, int32_t* idx,
+                             float* weight, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!c || !c->Kh) return fail(RANGE_ERR_INVALID, "database not set");
+  if (k < 1 || k > RANGE_TOPK_MAX) return fail(RANGE_ERR_INVALID, "k = %d: need 1 <= k <= %d", k, RANGE_TOPK_MAX);
+  if (row0 < 0 || row0 + c->M > int64_t(INT32_MAX))
+    return fail(RANGE_ERR_INVALID, "row0 = %lld: rows row0 .. row0 + M - 1 must be int32", (long long)row0);
+  return topk_impl(c, mode, N, q16, qxyz, temp, geo_temp, beta, sums, k, nullptr, row0, idx, weight, workspace,
+                   workspace_bytes, stream);
+}
+
+int range_topk_merge(range_ctx* c, int n_parts, int64_t N, int k, const float* part_w, const int32_t* part_idx,
+                     const int32_t* perm, int32_t* idx, float* weight, void* stream) {
+  if (!c || !part_w || !part_idx || !idx || !weight) return fail(RANGE_ERR_INVALID, "null argument");
+  if (n_parts < 1 || n_parts > RANGE_MAX_RANKS) return fail(RANGE_ERR_INVALID, "n_parts must be in [1, %d]", RANGE_MAX_RANKS);
+  if (N <= 0 || N > (int64_t(1) << 30)) return fail(RANGE_ERR_INVALID, "N must be in [1, 2^30]");
+  if (k < 1 || k > RANGE_TOPK_MAX) return fail(RANGE_ERR_INVALID, "k = %d: need 1 <= k <= %d", k, RANGE_TOPK_MAX);
+  CUDA_TRY(launch_topk_merge(part_w, part_idx, n_parts, int(N), k, perm, 0, idx, weight, cudaStream_t(stream)));
+  g_launches += 1;
   return RANGE_OK;
 }
 

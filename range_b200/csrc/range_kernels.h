@@ -180,9 +180,13 @@ cudaError_t launch_reduce_out(const float* part, size_t split_stride, int splits
 constexpr int kTopkMax = 32, kTopkMaxSplits = 64;
 // a.geo selects RANGE+ (a.geo_mask: the apply-pass mask or null); sums (N,2) from the statistics pass.  Database split
 // `split` covers tiles [split * tiles_per_split, ..); partial lists part_w / part_idx [2 * splits][N][k]; result row n
-// (k entries, descending weight, then ascending entry) -> idx / weight row perm[n] (perm null: n)
+// (k entries, descending weight, then ascending entry) -> idx / weight row perm[n] (perm null: n); a found entry j is
+// stored as row0 + j, an unfilled slot (fewer than k entries) as -1 with weight 0
 cudaError_t launch_topk(const RetrievalArgs& a, int splits, int tiles_per_split, const float* sums, float beta, int k,
-                        float* part_w, int32_t* part_idx, const int32_t* perm, int32_t* idx, float* weight,
+                        float* part_w, int32_t* part_idx, const int32_t* perm, int row0, int32_t* idx, float* weight,
                         cudaStream_t s);
+// the merge step alone: `parts` lists [parts][N][k], each sorted by weight descending then entry, -1 entries last
+cudaError_t launch_topk_merge(const float* part_w, const int32_t* part_idx, int parts, int N, int k,
+                              const int32_t* perm, int row0, int32_t* idx, float* weight, cudaStream_t s);
 
 }  // namespace rangeb200

@@ -16,6 +16,8 @@
 //                        Entries that pass are handed to a one-copy insertion loop through a per-thread row of shared
 //                        memory (no dynamic register indexing; a warp waits for its busiest lane, not for the union).
 //   topk_merge_kernel    one warp per query: a k-round merge of the (split, half) lists [parts][N][k]; row n -> perm[n].
+//                        Also merges the lists the shards of an M-sharded database send to a query's owner
+//                        (range_topk_merge: one part per rank, entries already in rows of the whole database).
 #include <cstdint>
 #include <cstdio>
 #include <type_traits>
@@ -313,11 +315,12 @@ range_topk_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __restr
 }
 
 // One warp per query: lane l holds the heads of parts l, l + 32, .. (sorted by weight descending, then entry); k rounds
-// of a warp arg-max (larger weight, then smaller entry) - the parts are disjoint, so no duplicates.
+// of a warp arg-max (larger weight, then smaller entry) - the parts are disjoint, so no duplicates.  A found entry is
+// stored as row0 + entry (a shard's rows in the whole database: the order of ties is kept, shards are ascending ranges).
 constexpr int kMergeSlots = 4;      // parts per lane: parts <= 128
 __global__ void __launch_bounds__(256)
 topk_merge_kernel(const float* __restrict__ part_w, const int32_t* __restrict__ part_idx, int parts, int N, int k,
-                  const int32_t* __restrict__ perm, int32_t* __restrict__ idx, float* __restrict__ weight) {
+                  const int32_t* __restrict__ perm, int row0, int32_t* __restrict__ idx, float* __restrict__ weight) {
   const int n = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (n >= N) return;
   int head[kMergeSlots];
@@ -351,7 +354,7 @@ topk_merge_kernel(const float* __restrict__ part_w, const int32_t* __restrict__ 
     }
     if (lane == 0) {
       const bool found = i != 0x7fffffff;
-      idx[size_t(dst) * k + r] = found ? i : -1;
+      idx[size_t(dst) * k + r] = found ? row0 + i : -1;
       weight[size_t(dst) * k + r] = found ? w : 0.f;
     }
   }
@@ -381,7 +384,7 @@ cudaError_t launch_bucket(dim3 grid, const rangeb200::RetrievalArgs& a, int tile
 namespace rangeb200 {
 
 cudaError_t launch_topk(const RetrievalArgs& a, int splits, int tiles_per_split, const float* sums, float beta, int k,
-                        float* part_w, int32_t* part_idx, const int32_t* perm, int32_t* idx, float* weight,
+                        float* part_w, int32_t* part_idx, const int32_t* perm, int row0, int32_t* idx, float* weight,
                         cudaStream_t s) {
   if (k < 1 || k > kTopkMax || 2 * splits > 32 * kMergeSlots) return cudaErrorInvalidValue;
   const dim3 grid((a.N + kBlockQ - 1) / kBlockQ, splits, 1);
@@ -390,7 +393,13 @@ cudaError_t launch_topk(const RetrievalArgs& a, int splits, int tiles_per_split,
   else if (k <= 16) e = launch_bucket<16>(grid, a, tiles_per_split, sums, beta, k, part_w, part_idx, s);
   else e = launch_bucket<32>(grid, a, tiles_per_split, sums, beta, k, part_w, part_idx, s);
   if (e != cudaSuccess) return e;
-  topk_merge_kernel<<<(a.N + 7) / 8, 256, 0, s>>>(part_w, part_idx, 2 * splits, a.N, k, perm, idx, weight);
+  return launch_topk_merge(part_w, part_idx, 2 * splits, a.N, k, perm, row0, idx, weight, s);
+}
+
+cudaError_t launch_topk_merge(const float* part_w, const int32_t* part_idx, int parts, int N, int k,
+                              const int32_t* perm, int row0, int32_t* idx, float* weight, cudaStream_t s) {
+  if (k < 1 || k > kTopkMax || parts < 1 || parts > 32 * kMergeSlots) return cudaErrorInvalidValue;
+  topk_merge_kernel<<<(N + 7) / 8, 256, 0, s>>>(part_w, part_idx, parts, N, k, perm, row0, idx, weight);
   return cudaGetLastError();
 }
 

@@ -308,12 +308,18 @@ class DeviceDatabase:
         db['locs'][rows] are the entries' locations: order[row_range[0] + idx], or row_range[0] + idx when the rows keep
         the file order.  idx: integer tensor on any device; returns int64 on the same device."""
         idx = torch.as_tensor(idx)
-        rows = idx.long() + self.row_range[0]
+        return self.file_rows_global(idx.long() + self.row_range[0])
+
+    def file_rows_global(self, rows):
+        """rows of the WHOLE sorted layout (e.g. what an M-sharded neighbours call returns; every shard holds the full
+        row order) -> rows of the database file: order[rows], or rows when the file order is kept.  rows: integer
+        tensor on any device; returns int64 on the same device."""
+        rows = torch.as_tensor(rows).long()
         if self.order is None:
             return rows
         cached = getattr(self, "_order_t", None)
-        if cached is None or cached.device != idx.device:
-            cached = self._order_t = torch.from_numpy(np.asarray(self.order, dtype=np.int64)).to(idx.device)
+        if cached is None or cached.device != rows.device:
+            cached = self._order_t = torch.from_numpy(np.asarray(self.order, dtype=np.int64)).to(rows.device)
         return cached[rows]
 
     def nbytes(self):

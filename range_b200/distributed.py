@@ -19,6 +19,12 @@ running max and the merge needs no rescaling:
 
 merge='reduce_scatter' replaces the routed epilogue + barrier by a local (N,1024) result and NCCL's reduce_scatter
 (the comparison baseline; also what runs if the peers' buffers cannot be mapped).
+
+neighbours() shares the steps up to the SUM of the exp-sums, then:
+    every rank          top-k lists of all P * slab queries over its shard, entries as rows of the whole database
+                        (range_retrieve_topk_rows)
+    all_to_all          the lists, k x 8 B per query and rank: rank r receives its own queries' lists from every shard
+    every rank          merges its P lists by weight, then row (range_topk_merge)
 """
 import ctypes
 
@@ -114,6 +120,7 @@ class ShardedRetriever:
     passes its own queries (the counts may differ) and gets its own rows back."""
 
     MAX_STEP_ROWS = 131072          # P * slab rows per apply launch (receive buffer: 4 KB per row and rank)
+    TOPK_WORKSPACE_BYTES = 1 << 30  # bound of the top-k workspace of a neighbours step (_topk_step_rows)
 
     def __init__(self, engine, group=None, merge="peer"):
         if merge not in ("peer", "reduce_scatter"):
@@ -125,9 +132,10 @@ class ShardedRetriever:
         self.buffers = None
         self._token = None
         self.collectives = 0            # NCCL calls issued (bench.py reports them)
+        self.trace = None               # developer timing: a list collects CUDA events around neighbours' exchange + merge
 
-    def _slab_for(self, n_max):
-        cap = max(128, self.MAX_STEP_ROWS // self.world // 128 * 128)
+    def _slab_for(self, n_max, step_rows=None):
+        cap = max(128, (step_rows or self.MAX_STEP_ROWS) // self.world // 128 * 128)
         return min(cap, (n_max + 127) // 128 * 128)
 
     def _ensure_buffers(self, slab):
@@ -154,22 +162,13 @@ class ShardedRetriever:
             self.buffers.close()
             self.buffers = None
 
-    def embed(self, mode, coords, temp, geo_temp, beta, sort, out=None, out_dtype=torch.float32):
-        """coords (n,2) fp64 on the device (this rank's queries) -> (n,1280) device tensor (this rank's rows)"""
-        eng, P, me = self.engine, self.world, self.rank
+    def _steps(self, mode, coords, temp, geo_temp, sort, n_max, slab):
+        """the step loop of embed and neighbours: per step of `slab` rows per rank, this rank's rows (padded) sorted and
+        encoded, every rank's compact queries gathered, their statistics over this shard and the SUM of the exp-sums.
+        Yields (lo, rows, perm, q64, q16_all, qxyz_all, sums, maxs): this rank's rows [lo, lo + rows) of the step."""
+        eng, P = self.engine, self.world
         dev = eng.device
         n = coords.shape[0]
-        n_max = torch.tensor([n], device=dev, dtype=torch.int64)
-        dist.all_reduce(n_max, op=dist.ReduceOp.MAX, group=self.group)
-        n_max = int(n_max.item())
-        self.collectives += 1
-        out = _new_out(n, out_dtype, dev) if out is None else out
-        if n_max == 0:
-            return out
-        slab = self._slab_for(n_max)
-        self._ensure_buffers(slab)
-        if self._token is None:
-            self._token = torch.zeros(1, device=dev)
         q16_all = torch.empty(P * slab, 256, dtype=torch.float16, device=dev)
         qxyz_all = torch.empty(P * slab, 4, dtype=torch.float32, device=dev)
         for lo in range(0, n_max, slab):
@@ -186,6 +185,26 @@ class ShardedRetriever:
             sums, maxs = eng.retrieve_stats(mode, q16_all, qxyz_all, temp, geo_temp)
             merge_sums(sums, self.group)
             self.collectives += 3
+            yield lo, rows, perm, q64, q16_all, qxyz_all, sums, maxs
+
+    def embed(self, mode, coords, temp, geo_temp, beta, sort, out=None, out_dtype=torch.float32):
+        """coords (n,2) fp64 on the device (this rank's queries) -> (n,1280) device tensor (this rank's rows)"""
+        eng, P, me = self.engine, self.world, self.rank
+        dev = eng.device
+        n = coords.shape[0]
+        n_max = torch.tensor([n], device=dev, dtype=torch.int64)
+        dist.all_reduce(n_max, op=dist.ReduceOp.MAX, group=self.group)
+        n_max = int(n_max.item())
+        self.collectives += 1
+        out = _new_out(n, out_dtype, dev) if out is None else out
+        if n_max == 0:
+            return out
+        slab = self._slab_for(n_max)
+        self._ensure_buffers(slab)
+        if self._token is None:
+            self._token = torch.zeros(1, device=dev)
+        for lo, rows, perm, q64, q16_all, qxyz_all, sums, maxs in self._steps(mode, coords, temp, geo_temp, sort, n_max,
+                                                                              slab):
             whole = rows == slab
             dst = out[lo:lo + slab] if whole else torch.empty((slab,) + tuple(out.shape[1:]), dtype=out.dtype, device=dev)
             if self.merge == "peer":
@@ -202,4 +221,53 @@ class ShardedRetriever:
             if not whole and rows > 0:
                 out[lo:lo + rows] = dst[:rows]
         return out
+
+    def _topk_step_rows(self, k):
+        """P * slab rows per neighbours step: the top-k pass's workspace is 2 * splits * rows * k * 8 B.  The statistics
+        plan it follows (csrc/capi.cu: plan_retrieval) takes at most 16 database splits from ~6 144 rows up (64 below,
+        at most 0.2 GB), so rows <= 2^30 / (2 * 16 * 8 * k) keeps it within TOPK_WORKSPACE_BYTES (1 GB)."""
+        return min(self.MAX_STEP_ROWS, self.TOPK_WORKSPACE_BYTES // (2 * 16 * 8 * k))
+
+    def neighbours(self, mode, coords, temp, geo_temp, beta, sort, k):
+        """coords (n,2) fp64 on the device (this rank's queries) -> (rows (n,k) int32, weight (n,k)) device tensors in
+        this rank's row order: the k entries of the WHOLE database with the largest retrieval weight, descending, equal
+        weights by the smaller row; rows of the database's sorted layout (DeviceDatabase.file_rows_global maps them to
+        file rows).  A COLLECTIVE call; every rank must pass the same k, 1 <= k <= min(RANGE_TOPK_MAX, entries of the
+        database) (ValueError on every rank when they differ).
+
+        Per step, after embed's statistics and SUM of the exp-sums: this shard's top-k lists of all P * slab gathered
+        queries (entries as global rows), all_to_all of the lists - they are rank-major by owner, so rank r receives
+        [P][slab][k] - and the owner's merge of its P lists.  At most 256 B per query and rank cross the links: no peer
+        buffers, the same path for both merge settings."""
+        eng, P = self.engine, self.world
+        dev = eng.device
+        n, k = coords.shape[0], int(k)
+        head = torch.tensor([n, k, -k], device=dev, dtype=torch.int64)     # max n, and max / min k: the ranks agree?
+        dist.all_reduce(head, op=dist.ReduceOp.MAX, group=self.group)
+        self.collectives += 1
+        n_max, k_max, k_min = int(head[0]), int(head[1]), -int(head[2])
+        if k_max != k_min:
+            raise ValueError(f"neighbours: every rank must pass the same k, got k from {k_min} to {k_max}")
+        if n_max == 0:
+            return (torch.empty(0, k, dtype=torch.int32, device=dev), torch.empty(0, k, dtype=torch.float32, device=dev))
+        slab = self._slab_for(n_max, self._topk_step_rows(k))
+        row0 = eng.db.row_range[0]
+        got_idx, got_w = [], []
+        for lo, rows, perm, _, q16_all, qxyz_all, sums, _ in self._steps(mode, coords, temp, geo_temp, sort, n_max, slab):
+            idx, w = eng.retrieve_topk_rows(mode, q16_all, qxyz_all, temp, geo_temp, beta, sums, k, row0)
+            if self.trace is not None:
+                t0 = torch.cuda.Event(enable_timing=True)
+                t0.record()
+            recv_w, recv_idx = torch.empty_like(w), torch.empty_like(idx)
+            dist.all_to_all_single(recv_w, w, group=self.group)
+            dist.all_to_all_single(recv_idx, idx, group=self.group)
+            self.collectives += 2
+            mi, mw = eng.topk_merge(recv_w.view(P, slab, k), recv_idx.view(P, slab, k), perm=perm)
+            if self.trace is not None:
+                t1 = torch.cuda.Event(enable_timing=True)
+                t1.record()
+                self.trace.append((t0, t1))
+            got_idx.append(mi[:rows])
+            got_w.append(mw[:rows])
+        return torch.cat(got_idx), torch.cat(got_w)
 

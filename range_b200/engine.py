@@ -270,6 +270,36 @@ class RangeEngine:
                 ws.numel(), _stream()))
         return idx, weight
 
+    def retrieve_topk_rows(self, mode, q16, qxyz, temp, geo_temp, beta, sums, k, row0):
+        """retrieve_topk as one shard of an M-sharded database (sums: the global ones): entries are row0 + device row
+        (rows of the whole sorted database with row0 = db.row_range[0]), k may exceed this shard's M (unfilled slots:
+        entry -1, weight 0), row n of the result is query n"""
+        N = q16.shape[0]
+        idx = torch.empty(N, k, dtype=torch.int32, device=self.device)
+        weight = torch.empty(N, k, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.index):
+            ws = self._workspace("topk", max(1, self.lib.range_topk_workspace_bytes(self.ctx, N, k)))
+            _lib.check(self.lib.range_retrieve_topk_rows(
+                self.ctx, MODE[mode], N, _ptr(q16), _ptr(qxyz), temp, geo_temp, 0.0 if beta is None else float(beta),
+                _ptr(sums), k, int(row0), _ptr(idx), _ptr(weight), _ptr(ws), ws.numel(), _stream()))
+        return idx, weight
+
+    def topk_merge(self, part_w, part_idx, perm=None):
+        """(parts, N, k) fp32 / int32 lists (each sorted by weight descending, then entry; -1 entries last) -> the merged
+        (idx (N,k) int32, weight (N,k) fp32), row n at row perm[n]"""
+        parts, N, k = part_w.shape
+        if part_idx.shape != part_w.shape or part_w.dtype != torch.float32 or part_idx.dtype != torch.int32 \
+                or not (part_w.is_contiguous() and part_idx.is_contiguous()):
+            raise ValueError(f"part_w / part_idx must be contiguous (parts, N, k) float32 / int32, got "
+                             f"{part_w.dtype} {tuple(part_w.shape)}, {part_idx.dtype} {tuple(part_idx.shape)}")
+        idx = torch.empty(N, k, dtype=torch.int32, device=self.device)
+        weight = torch.empty(N, k, dtype=torch.float32, device=self.device)
+        with torch.cuda.device(self.index):
+            _lib.check(self.lib.range_topk_merge(self.ctx, parts, N, k, _ptr(part_w), _ptr(part_idx),
+                                                 c_void_p(None) if perm is None else _ptr(perm), _ptr(idx),
+                                                 _ptr(weight), _stream()))
+        return idx, weight
+
     def retrieve_apply(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, O=None):
         N = q16.shape[0]
         O = torch.empty(N, 1024, dtype=torch.float32, device=self.device) if O is None else O

@@ -150,16 +150,21 @@ class LocationEncoder(nn.Module):
         """Which database entries each embedding is made of: coords (N,2) fp64 (lon, lat) degrees -> (index (N,k) int64,
         weight (N,k) float32) device tensors in the caller's row order.  index holds rows of the database file
         (db['locs'][index] are the neighbours' locations), weight the coefficient the retrieved feature gives each of
-        them (range/range.py:213-238 with this model's temp, geo_temp and beta), largest first."""
+        them (range/range.py:213-238 with this model's temp, geo_temp and beta), largest first.
+        With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call: every rank passes its own queries
+        and the same k, and gets the neighbours of its own rows over the whole database (distributed.py)."""
         eng, a = self.engine, self.args
-        if self.sharded is not None:
-            raise NotImplementedError('neighbours: an unsharded database')
         k = int(k)
-        if not 1 <= k <= min(_lib.RANGE_TOPK_MAX, eng.db.M):
-            raise ValueError(f'k={k}: expected 1 <= k <= {min(_lib.RANGE_TOPK_MAX, eng.db.M)} (database of {eng.db.M} entries)')
+        k_max = min(_lib.RANGE_TOPK_MAX, eng.db.M_total)       # the whole database: the same bound on every rank
+        if not 1 <= k <= k_max:
+            raise ValueError(f'k={k}: expected 1 <= k <= {k_max} (database of {eng.db.M_total} entries)')
         coords = coords.to(eng.device, torch.float64).contiguous()
         name = self.location_model_name
         geo_temp = float(getattr(a, 'geo_temp', 0.0))
+        if self.sharded is not None:
+            rows, weight = self.sharded.neighbours(name, coords, a.temp, geo_temp, getattr(a, 'beta', None),
+                                                   self._sorts(), k)
+            return eng.db.file_rows_global(rows), weight
         perm = None
         if self._sorts():
             coords, perm = eng.sort_queries(coords)

@@ -1,7 +1,8 @@
 """Run under torchrun on N >= 2 GPUs: the M-sharded database path (range_b200/distributed.py) against the unsharded one.
 Every rank owns its own queries (ragged counts, one rank's set clustered in a small region, several steps), the database
 is sharded along M; both merges are checked: 'peer' (the apply kernel's epilogue stores partial rows into the owners'
-receive buffers over NVLink) and 'reduce_scatter' (NCCL).  Also: query sharding + all_gather == one GPU.
+receive buffers over NVLink) and 'reduce_scatter' (NCCL).  Also: query sharding + all_gather == one GPU, and the
+M-sharded neighbours(coords, 8) (shard lists exchanged with all_to_all, merged on the owner) against the unsharded one.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/multi_gpu_check.py
 """
 import contextlib, os, sys, time
@@ -50,7 +51,26 @@ def timed(fn, reps=3):
 full = model()
 ref = full.embed(coords)                                            # unsharded database, my queries
 t_full = timed(lambda: full.embed(coords))
-report = {}
+K_NB, TOL = 8, 2e-3
+nb_ref = full.neighbours(coords, K_NB)
+report, nb_report, nb_out = {}, {}, {}
+
+
+def max_all(x):
+    x = torch.tensor([float(x)], device=dev)
+    dist.all_reduce(x, op=dist.ReduceOp.MAX)
+    return float(x[0])
+
+
+def neighbours_vs_full(got):
+    """weights within TOL of the unsharded call position by position; entries only one list holds have weights within
+    TOL of the unsharded k-th weight (near-ties at the cut): (max rel weight diff, entries that differ, worst tie gap)"""
+    (r_sh, w_sh), (r_un, w_un) = got, nb_ref
+    e_w = ((w_sh.double() - w_un.double()).abs() / w_un.double()).max().item() if w_un.numel() else 0.0
+    only = ~(r_sh.unsqueeze(2) == r_un.unsqueeze(1)).any(2)
+    kth = w_un[:, -1:].double().expand_as(w_un)
+    gap = ((w_sh.double() - kth).abs() / kth)[only].max().item() if only.any() else 0.0
+    return e_w, int(only.sum()), gap
 for merge in ("peer", "reduce_scatter"):
     sh = model(db_shard=(rank, world), db_group=None, db_merge=merge)
     sh.sharded.MAX_STEP_ROWS = int(os.environ.get("STEP_ROWS", 16_384 * world))     # several steps per call
@@ -65,6 +85,18 @@ for merge in ("peer", "reduce_scatter"):
     if host is not None:
         assert host.shape == (n_mine, 1280) and np.allclose(host[:, :1024], out[:, :1024].cpu().numpy(), rtol=1e-6, atol=1e-7)
     report[merge] = (sh.sharded.merge, float(err[0]), float(err[1]), bool(same[0] > 0), t)
+    nb = sh.neighbours(coords, K_NB)                                 # collective: every rank, the same k
+    nb_again = sh.neighbours(coords, K_NB)
+    nb_same = max_all(not (torch.equal(nb[0], nb_again[0]) and torch.equal(nb[1], nb_again[1]))) == 0
+    e_w, n_diff, gap = neighbours_vs_full(nb)
+    t_nb = timed(lambda: sh.neighbours(coords, K_NB))
+    sh.sharded.trace = []                                            # CUDA events around the list exchange + owner merge
+    sh.neighbours(coords, K_NB)
+    torch.cuda.synchronize()
+    t_x = sum(a.elapsed_time(b) for a, b in sh.sharded.trace) / 1e3
+    sh.sharded.trace = None
+    nb_out[merge] = nb
+    nb_report[merge] = (max_all(e_w), int(max_all(n_diff)), max_all(gap), nb_same, max_all(t_nb), max_all(t_x), t)
     sh.sharded.close()
     del sh
 lo, hi = shard_rows(N, rank, world)                                # query sharding: my slab of a common set, then gather
@@ -81,4 +113,12 @@ if rank == 0:
         assert e_o < 1e-3 and e_q == 0.0 and same
     print(f"query-sharded + all_gather vs one GPU {e2:.2e}")
     assert e2 < 1e-3
+across = max_all(not all(torch.equal(a, b) for a, b in zip(nb_out["peer"], nb_out["reduce_scatter"]))) == 0
+if rank == 0:
+    for merge, (e_w, n_diff, gap, same, t_nb, t_x, t) in nb_report.items():
+        print(f"M-sharded neighbours k={K_NB} [{merge}] vs unsharded: max rel weight diff {e_w:.2e}, {n_diff} entries differ "
+              f"(weights within {gap:.1e} of the k-th), repeatable {same}, same under both merges {across}; "
+              f"{t_nb*1e3:.1f} ms per call (list exchange + owner merge {t_x*1e3:.2f} ms, {100 * t_x / t_nb:.1f} %) "
+              f"vs {t*1e3:.1f} ms for the sharded embed (world {world}, N={N}+1500 r per rank, M={M})")
+        assert e_w < TOL and gap < TOL and same and across
 dist.destroy_process_group()
