@@ -240,6 +240,20 @@ int range_retrieve_apply_routed(range_ctx* ctx, int mode, int64_t N, const void*
 int range_combine_concat(range_ctx* ctx, int64_t N, int n_parts, const float* const* parts, const float* weights,
                          const double* q64, const int32_t* perm, void* out, int out_dtype, void* stream);
 
+/* The last step of a beta sweep on an M-sharded database, for up to RANGE_SWEEP_MAX_BETAS beta at once:
+ *   outs[b] row perm[n] (NULL = identity) = [ w_sem[b] * S[n] + w_geo[b] * G[n] | q64[n][0:256] ]
+ * G = sum of the n_slots geo slots, S = sum of the n_slots sem slots, each summed in slot order 0 .. n_slots-1 (the
+ * partial rows of the geographic end, beta 0, and of the semantic end, beta 1, that the ranks sent this owner); per
+ * column fmaf(w_sem, s, w_geo * g).  geo / sem: host arrays of n_slots (1 <= n_slots <= RANGE_MAX_RANKS) device pointers
+ * to (N,1024) fp32; w_geo / w_sem: host arrays of n_betas (1 <= n_betas <= RANGE_SWEEP_MAX_BETAS) weights, normally
+ * 1 - beta and beta rounded on the host; outs: host array of n_betas device pointers to (N,1280) results in out_dtype
+ * (RANGE_OUT_F64 or RANGE_OUT_F32).  Every slot is read once, whatever n_betas.  With n_slots = 1 the rows are bit for bit
+ * those of range_combine_concat with parts (G, S) and weights (w_geo, w_sem). */
+#define RANGE_SWEEP_MAX_BETAS 8
+int range_sweep_concat(range_ctx* ctx, int64_t N, int n_slots, const float* const* geo, const float* const* sem,
+                       int n_betas, const float* w_geo, const float* w_sem, const double* q64, const int32_t* perm,
+                       void* const* outs, int out_dtype, void* stream);
+
 /* Receive buffers must be mappable by the other ranks' processes: the one place where the library allocates device
  * memory itself (cudaMalloc + CUDA IPC handle, 64 opaque bytes to hand to the peers, e.g. with all_gather_object).
  * range_peer_open maps a peer's buffer into this process (enables peer access over NVLink), range_peer_close unmaps

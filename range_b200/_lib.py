@@ -15,6 +15,7 @@ RANGE_OUT_F64, RANGE_OUT_F32, RANGE_OUT_PACKED = 0, 1, 2
 RANGE_MAX_RANKS = 8
 RANGE_ENC_F64, RANGE_ENC_F16X3 = 0, 1
 RANGE_TOPK_MAX = 32
+RANGE_SWEEP_MAX_BETAS = 8
 
 # every symbol include/range_b200.h declares: name -> (restype, argtypes)
 PROTOTYPES = {
@@ -69,6 +70,8 @@ PROTOTYPES = {
                                             c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "range_combine_concat": (c_int, [c_void_p, c_int64, c_int, POINTER(c_void_p), POINTER(c_float), c_void_p, c_void_p,
                                      c_void_p, c_int, c_void_p]),
+    "range_sweep_concat": (c_int, [c_void_p, c_int64, c_int, POINTER(c_void_p), POINTER(c_void_p), c_int, POINTER(c_float),
+                                   POINTER(c_float), c_void_p, c_void_p, POINTER(c_void_p), c_int, c_void_p]),
     "range_peer_alloc": (c_int, [c_size_t, POINTER(c_void_p), c_void_p]),
     "range_peer_open": (c_int, [c_void_p, POINTER(c_void_p)]),
     "range_peer_close": (c_int, [c_void_p]),

@@ -1031,6 +1031,36 @@ int range_combine_concat(range_ctx* c, int64_t N, int n_parts, const float* cons
   return RANGE_OK;
 }
 
+int range_sweep_concat(range_ctx* c, int64_t N, int n_slots, const float* const* geo, const float* const* sem,
+                       int n_betas, const float* w_geo, const float* w_sem, const double* q64, const int32_t* perm,
+                       void* const* outs, int out_dtype, void* stream) {
+  static_assert(RANGE_MAX_RANKS == kMaxRanks && RANGE_SWEEP_MAX_BETAS == kSweepMaxBetas, "merge.cu: SweepParts");
+  if (!c || !geo || !sem || !w_geo || !w_sem || !q64 || !outs) return fail(RANGE_ERR_INVALID, "null argument");
+  if (N <= 0 || N > (int64_t(1) << 30)) return fail(RANGE_ERR_INVALID, "N must be in [1, 2^30]");
+  if (n_slots < 1 || n_slots > RANGE_MAX_RANKS) return fail(RANGE_ERR_INVALID, "n_slots must be in [1, %d]", RANGE_MAX_RANKS);
+  if (n_betas < 1 || n_betas > RANGE_SWEEP_MAX_BETAS)
+    return fail(RANGE_ERR_INVALID, "n_betas must be in [1, %d]", RANGE_SWEEP_MAX_BETAS);
+  if (out_dtype != RANGE_OUT_F64 && out_dtype != RANGE_OUT_F32)
+    return fail(RANGE_ERR_INVALID, "out dtype must be RANGE_OUT_F64 or RANGE_OUT_F32");
+  SweepParts sp;
+  sp.n_slots = n_slots;
+  sp.n_betas = n_betas;
+  for (int k = 0; k < n_slots; ++k) {
+    if (!geo[k] || !sem[k]) return fail(RANGE_ERR_INVALID, "slot %d is null", k);
+    sp.geo[k] = geo[k];
+    sp.sem[k] = sem[k];
+  }
+  for (int b = 0; b < n_betas; ++b) {
+    if (!outs[b]) return fail(RANGE_ERR_INVALID, "output %d is null", b);
+    sp.w_geo[b] = w_geo[b];
+    sp.w_sem[b] = w_sem[b];
+    sp.out[b] = outs[b];
+  }
+  CUDA_TRY(launch_sweep_concat(sp, q64, int(N), perm, out_dtype, cudaStream_t(stream)));
+  g_launches += 1;
+  return RANGE_OK;
+}
+
 /* ---- peer memory (receive buffers of an M-sharded database) ---- */
 int range_peer_alloc(size_t bytes, void** dptr, unsigned char* handle64) {
   if (!bytes || !dptr || !handle64) return fail(RANGE_ERR_INVALID, "bad arguments");

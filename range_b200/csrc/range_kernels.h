@@ -118,6 +118,20 @@ cudaError_t launch_combine_concat(const CombineParts& parts, const double* q64, 
                                   int dtype, cudaStream_t s);
 // O (N,1024) fp32 -> the owners' receive buffers
 cudaError_t launch_route_rows(const float* O, int N, const RowRoute& route, cudaStream_t s);
+// a beta sweep's last step: the geographic (beta 0) and semantic (beta 1) ends, each as n_slots partial slots
+constexpr int kSweepMaxBetas = 8;
+struct SweepParts {
+  int n_slots = 0, n_betas = 0;
+  const float* geo[kMaxRanks] = {};
+  const float* sem[kMaxRanks] = {};
+  float w_geo[kSweepMaxBetas] = {};
+  float w_sem[kSweepMaxBetas] = {};
+  void* out[kSweepMaxBetas] = {};
+};
+// G = sum of the geo slots, S = sum of the sem slots (slot order); for every b < n_betas:
+// out[b][perm ? perm[n] : n] = [fmaf(w_sem[b], S[n], w_geo[b] * G[n]) | q64[n]]; dtype 0: fp64 (N,1280), 1: fp32 (N,1280)
+cudaError_t launch_sweep_concat(const SweepParts& parts, const double* q64, int N, const int* perm, int dtype,
+                                cudaStream_t s);
 
 // ---- spatial batching of the queries (sort.cu) ----------------------------------------------------
 size_t sort_workspace_bytes(int N);

@@ -25,6 +25,12 @@ neighbours() shares the steps up to the SUM of the exp-sums, then:
                         (range_retrieve_topk_rows)
     all_to_all          the lists, k x 8 B per query and rank: rank r receives its own queries' lists from every shard
     every rank          merges its P lists by weight, then row (range_topk_merge)
+
+embed_sweep() (RANGE+ for several beta) shares the steps up to the SUM of the exp-sums, then:
+    every rank          apply passes of the geographic end (beta 0) and the semantic end (beta 1), routed into the two
+                        halves of the owners' receive buffers
+    barrier             one for both ends
+    every rank          sums its P slots of each end and writes (1 - beta) G + beta S for every beta (range_sweep_concat)
 """
 import ctypes
 
@@ -91,14 +97,18 @@ class PeerBuffers:
                 self._opened.append(p)
                 self.ptrs.append(p.value)
 
-    def route(self, slab):
-        """range_route of a step of `slab` (<= self.slab) rows per rank: slot r of a buffer starts at r * slab rows"""
-        assert slab <= self.slab
-        return _lib.Route(self.world, self.rank, int(slab), (ctypes.c_void_p * _lib.RANGE_MAX_RANKS)(*self.ptrs))
+    def route(self, slab, half=0):
+        """range_route of a step of `slab` rows per rank: slot r of a buffer starts at r * slab rows.  half=1 (a beta
+        sweep: the two ends of a step, each `slab` <= self.slab / 2 rows per rank): slot r of half h starts at
+        (h * P + r) * slab rows"""
+        assert (half + 1) * slab <= self.slab
+        base = half * self.world * int(slab) * 4096
+        return _lib.Route(self.world, self.rank, int(slab),
+                          (ctypes.c_void_p * _lib.RANGE_MAX_RANKS)(*[p + base for p in self.ptrs]))
 
-    def slots(self, slab):
-        """device addresses of this rank's P slots for a step of `slab` rows per rank"""
-        return [self.local.value + r * int(slab) * 4096 for r in range(self.world)]
+    def slots(self, slab, half=0):
+        """device addresses of this rank's P slots for a step of `slab` rows per rank (in `half`, see route)"""
+        return [self.local.value + (half * self.world + r) * int(slab) * 4096 for r in range(self.world)]
 
     def close(self):
         if getattr(self, "local", None) is None:
@@ -221,6 +231,62 @@ class ShardedRetriever:
             if not whole and rows > 0:
                 out[lo:lo + rows] = dst[:rows]
         return out
+
+    def embed_sweep(self, coords, temp, geo_temp, sort, betas, out_dtype=torch.float32):
+        """RANGE+ for several beta on this rank's queries: coords (n,2) fp64 on the device -> a list of (n,1280) device
+        tensors, one per beta, in this rank's row order.  A COLLECTIVE call: every rank takes every step, whatever its
+        own n and its own beta list (the lists may differ between ranks; an empty one returns []).
+
+        The steps of embed (RANGE+ statistics, SUM of the exp-sums), then TWO apply passes per step whatever the number
+        of beta, as in the unsharded LocationEncoder.embed_sweep: the geographic end (beta 0) and the semantic end (the
+        one-softmax retrieval at temp, with RANGE+'s sums).  Peer merge: the two ends are routed into the two halves of
+        the receive buffer (slot r of half h at row (h P + r) slab, PeerBuffers.route / slots; slab <= MAX_STEP_ROWS / 2P,
+        so the buffer is the one embed allocates), one barrier, then range_sweep_concat over this rank's 2 P slots writes
+        every beta.  The buffer is reused across steps for the same reason as embed's: a rank's apply passes of step i + 1
+        follow its all_gathers of step i + 1 on its stream, which cannot complete before every rank has enqueued - and so,
+        in stream order, finished - its sweep_concat of step i.  merge='reduce_scatter': both ends computed locally, two
+        reduce_scatters, then range_sweep_concat with one slot per end.  Collectives: 1 + 4 per step (peer), 1 + 5
+        (reduce_scatter)."""
+        eng, P, me = self.engine, self.world, self.rank
+        dev = eng.device
+        n = coords.shape[0]
+        betas = [float(b) for b in betas]
+        if out_dtype not in (torch.float64, torch.float32):
+            raise ValueError(f"out_dtype={out_dtype}: expected torch.float64 or torch.float32")
+        n_max = torch.tensor([n], device=dev, dtype=torch.int64)
+        dist.all_reduce(n_max, op=dist.ReduceOp.MAX, group=self.group)
+        n_max = int(n_max.item())
+        self.collectives += 1
+        outs = [_new_out(n, out_dtype, dev) for _ in betas]
+        if n_max == 0:
+            return outs
+        slab = self._slab_for(n_max, self.MAX_STEP_ROWS // 2)
+        self._ensure_buffers(2 * slab)
+        if self._token is None:
+            self._token = torch.zeros(1, device=dev)
+        for lo, rows, perm, q64, q16_all, qxyz_all, sums, maxs in self._steps("RANGE+", coords, temp, geo_temp, sort,
+                                                                              n_max, slab):
+            if self.merge == "peer":
+                bufs = self.buffers
+                eng.retrieve_apply_routed("RANGE+", q16_all, qxyz_all, temp, geo_temp, 0.0, sums, maxs, bufs.route(slab, 0))
+                eng.retrieve_apply_routed("RANGE", q16_all, qxyz_all, temp, 0.0, None, sums, maxs, bufs.route(slab, 1))
+                dist.all_reduce(self._token, group=self.group)                    # barrier: all partial rows have landed
+                self.collectives += 1
+                geo, sem = bufs.slots(slab, 0), bufs.slots(slab, 1)
+            else:
+                O_geo = eng.retrieve_apply("RANGE+", q16_all, qxyz_all, temp, geo_temp, 0.0, sums, maxs)
+                O_sem = eng.retrieve_apply("RANGE", q16_all, qxyz_all, temp, 0.0, None, sums, maxs)
+                geo, sem = [_reduce_scatter(O_geo, P, me, self.group)], [_reduce_scatter(O_sem, P, me, self.group)]
+                self.collectives += 2
+            if not betas:
+                continue
+            whole = rows == slab
+            dst = [o[lo:lo + slab] if whole else torch.empty(slab, 1280, dtype=o.dtype, device=dev) for o in outs]
+            eng.sweep_concat(geo, sem, betas, q64, perm=perm, outs=dst)
+            if not whole and rows > 0:
+                for o, d in zip(outs, dst):
+                    o[lo:lo + rows] = d[:rows]
+        return outs
 
     def _topk_step_rows(self, k):
         """P * slab rows per neighbours step: the top-k pass's workspace is 2 * splits * rows * k * 8 B.  The statistics

@@ -379,3 +379,52 @@ class RangeEngine:
                                                      c_void_p(None) if perm is None else _ptr(perm), _ptr(out),
                                                      _out_code(out), _stream()))
         return out
+
+    def sweep_concat(self, geo_parts, sem_parts, betas, q64, out_dtype=torch.float32, perm=None, outs=None):
+        """[(1 - beta) G[n] + beta S[n] | q64[n]] at row perm[n] for every beta: G / S = the sum of the slots geo_parts /
+        sem_parts (the geographic and semantic ends of a beta sweep; tensors or raw device addresses, (N,1024) fp32),
+        each slot read once per RANGE_SWEEP_MAX_BETAS beta.  Returns a list of (N,1280) tensors in out_dtype (float64 or
+        float32), or fills `outs` (one per beta)."""
+        N = q64.shape[0]
+        if len(geo_parts) != len(sem_parts):
+            raise ValueError(f"{len(geo_parts)} geo slots but {len(sem_parts)} sem slots")
+
+        def addresses(parts):
+            ptrs = []
+            for p in parts:
+                if isinstance(p, int):
+                    ptrs.append(p)
+                    continue
+                if p.dtype != torch.float32 or p.shape != (N, 1024) or not p.is_contiguous():
+                    raise ValueError(f"slots must be contiguous (N,1024) float32, got {p.dtype} {tuple(p.shape)}")
+                ptrs.append(p.data_ptr())
+            return (c_void_p * len(ptrs))(*ptrs)
+
+        G, S = addresses(geo_parts), addresses(sem_parts)
+        betas = [float(b) for b in betas]
+        if outs is None:
+            if out_dtype not in (torch.float64, torch.float32):
+                raise ValueError(f"out_dtype={out_dtype}: expected torch.float64 or torch.float32")
+            outs = [_new_out(N, out_dtype, self.device) for _ in betas]
+        if len(outs) != len(betas):
+            raise ValueError(f"{len(outs)} outputs for {len(betas)} beta")
+        codes = {_out_code(o) for o in outs}
+        if len(codes) > 1:
+            raise ValueError("every output of a sweep must have the same dtype")
+        for o in outs:
+            width = PACKED_ROW_BYTES if _out_code(o) == _lib.RANGE_OUT_PACKED else 1280
+            if o.shape != (N, width) or not o.is_contiguous():
+                raise ValueError(f"outputs must be contiguous ({N}, {width}), got {tuple(o.shape)}")
+        if N == 0:
+            return outs
+        step = _lib.RANGE_SWEEP_MAX_BETAS              # the kernel's limit: longer lists in groups
+        with torch.cuda.device(self.index):
+            for b0 in range(0, len(betas), step):
+                bs, group = betas[b0:b0 + step], outs[b0:b0 + step]
+                n = len(bs)
+                # the weights are rounded to fp32 here, like combine_concat's (1 - beta, beta) in the unsharded sweep
+                _lib.check(self.lib.range_sweep_concat(
+                    self.ctx, N, len(geo_parts), G, S, n, (ctypes.c_float * n)(*[1.0 - b for b in bs]),
+                    (ctypes.c_float * n)(*bs), _ptr(q64), c_void_p(None) if perm is None else _ptr(perm),
+                    (c_void_p * n)(*[o.data_ptr() for o in group]), _out_code(group[0]), _stream()))
+        return outs

@@ -130,10 +130,16 @@ class LocationEncoder(nn.Module):
         """RANGE+ for several beta on the same queries (multi-resolution use, Readme.md:27-31).  range/range.py:238 is
         linear in beta - O(beta) = (1 - beta) O_geo + beta O_sem - so the encoder, the statistics pass and TWO apply
         passes (the geographic and the semantic end) serve any number of beta; each beta then costs one memory-bound
-        blend + concat kernel.  Returns a list of (N,1280) device tensors."""
-        if self.location_model_name != 'RANGE+' or self.sharded is not None:
-            raise NotImplementedError('embed_sweep: RANGE+ with an unsharded database')
+        blend + concat kernel.  Returns a list of (N,1280) device tensors.
+        With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call: every rank passes its own queries
+        and its own beta list (the lists may differ; every rank takes every step) and gets its own rows for each of its
+        beta (distributed.py: two routed apply passes per step, one merge kernel for all beta)."""
+        if self.location_model_name != 'RANGE+':
+            raise NotImplementedError('embed_sweep: only RANGE+ has a beta to sweep')
         eng, a = self.engine, self.args
+        if self.sharded is not None:
+            coords = torch.as_tensor(coords).to(eng.device, torch.float64).contiguous()
+            return self.sharded.embed_sweep(coords, a.temp, a.geo_temp, self._sorts(), betas, out_dtype=out_dtype)
         perm = None
         if self._sorts():
             coords, perm = eng.sort_queries(coords)
@@ -269,6 +275,17 @@ class LocationEncoder(nn.Module):
         lat = torch.as_tensor(lat_axis).to(eng.device, torch.float64).contiguous()
         return dict(H=lat.numel(), W=lon.numel(), buf=None, lon=lon, lat=lat)
 
+    def _raster_lonlat(self, tables, p0, n):
+        """(n,2) fp64 device coordinates of the raster points [p0, p0 + n), built on the device"""
+        eng = self.engine
+        if n == 0:
+            return torch.empty(0, 2, dtype=torch.float64, device=eng.device)
+        if tables['buf'] is None:
+            return self._raster_coords(tables, self._raster_ij(tables['W'], p0, p0 + n)).contiguous()
+        lonlat = torch.empty(n, 2, dtype=torch.float64, device=eng.device)
+        eng.raster_points(tables, p0, n, lonlat=lonlat)
+        return lonlat
+
     def _encode_raster(self, tables, ij):
         eng = self.engine
         if tables['buf'] is None:
@@ -280,11 +297,17 @@ class LocationEncoder(nn.Module):
         """Device-resident dense-grid path (BASELINE config 5): the points [rows[0], rows[1]) of the lat-major raster
         lat_axis x lon_axis (point p = i * W + j, like coord_grid) -> (n, 1280) device tensor in raster order.  The
         harmonics are evaluated separably (once per distinct latitude / longitude, csrc/encoder_raster.cu); results
-        are bit-identical to embed() on the same coordinates."""
+        are bit-identical to embed() on the same coordinates.
+        With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call: every rank passes the same axes and
+        its own rows (e.g. its slab of the raster) and gets those points' rows over the whole database - the sharded
+        embed() of the points' coordinates, built on the device (the per-point encoder: the separable one is no faster
+        there and gives the same bits)."""
         eng = self.engine
         tables = self.raster_tables(lon_axis, lat_axis) if tables is None else tables
         p0, p1 = (0, tables['H'] * tables['W']) if rows is None else rows
         n = p1 - p0
+        if self.sharded is not None:
+            return self.embed(self._raster_lonlat(tables, p0, n), out=out, out_dtype=out_dtype)
         perm = None
         if tables['buf'] is None:              # no separable evaluation: the per-point encoder on the materialised coordinates
             ij = self._raster_ij(tables['W'], p0, p1)
@@ -305,7 +328,9 @@ class LocationEncoder(nn.Module):
     def forward_raster(self, lon_axis, lat_axis, rows=None, out=None):
         """model(coord_grid(...)) without building the coordinate list on the host: numpy float64 (H * W, 1280).
         rows=(p0, p1): only those raster points (a rank's slab); out: the caller's float64 (p1 - p0, 1280) array, e.g.
-        rows of a memory-mapped .npy (filled through the packed path with bounded page-locked memory)."""
+        rows of a memory-mapped .npy (filled through the packed path with bounded page-locked memory).
+        With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call like embed_raster: every rank passes
+        the same axes and its own rows; its points' rows are computed on the device, then copied to the host."""
         tables = self.raster_tables(lon_axis, lat_axis)
         p0, p1 = (0, tables['H'] * tables['W']) if rows is None else rows
         if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float64 and out.shape == (p1 - p0, 1280)
@@ -338,7 +363,10 @@ class LocationEncoder(nn.Module):
         elif path == 'auto':
             path = 'copy' if N * row_bytes <= self.pinned_limit else 'packed'
         if self.sharded is not None:            # collective: distributed.py chunks (every rank must take the same steps)
-            dev = coords.to(eng.device, torch.float64, non_blocking=True)
+            if raster is None:
+                dev = coords.to(eng.device, torch.float64, non_blocking=True)
+            else:
+                dev = self._raster_lonlat(raster, raster_p0, N)
             res = self.embed(dev, out_dtype=tdtype)
             host = torch.empty((N, 1280), dtype=tdtype, pin_memory=N * row_bytes <= self.pinned_limit)
             host.copy_(res)

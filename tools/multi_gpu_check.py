@@ -2,7 +2,9 @@
 Every rank owns its own queries (ragged counts, one rank's set clustered in a small region, several steps), the database
 is sharded along M; both merges are checked: 'peer' (the apply kernel's epilogue stores partial rows into the owners'
 receive buffers over NVLink) and 'reduce_scatter' (NCCL).  Also: query sharding + all_gather == one GPU, and the
-M-sharded neighbours(coords, 8) (shard lists exchanged with all_to_all, merged on the owner) against the unsharded one.
+M-sharded neighbours(coords, 8) (shard lists exchanged with all_to_all, merged on the owner) against the unsharded one,
+the M-sharded embed_sweep (beta 0 .. 1 in 5 steps) against the unsharded sweep, and the M-sharded embed_raster /
+forward_raster of every rank's slab of a small raster against the sharded embed of the same points and the unsharded raster.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 tools/multi_gpu_check.py
 """
 import contextlib, os, sys, time
@@ -53,7 +55,15 @@ ref = full.embed(coords)                                            # unsharded 
 t_full = timed(lambda: full.embed(coords))
 K_NB, TOL = 8, 2e-3
 nb_ref = full.neighbours(coords, K_NB)
-report, nb_report, nb_out = {}, {}, {}
+BETAS = (0.0, 0.25, 0.5, 0.75, 1.0)
+sw_ref = full.embed_sweep(coords, BETAS)
+RH, RW = 90, 180                                                    # a small raster, every rank its own slab of points
+lon_ax, lat_ax = LocationEncoder.coord_grid_axes((RH, RW))
+p0, p1 = shard_rows(RH * RW, rank, world)
+pts_idx = torch.arange(p0, p1)
+raster_pts = torch.stack((lon_ax[pts_idx % RW], lat_ax[pts_idx // RW]), 1).to(dev)
+raster_ref = full.embed_raster(lon_ax, lat_ax, rows=(p0, p1))
+report, nb_report, nb_out, sw_report, ra_report = {}, {}, {}, {}, {}
 
 
 def max_all(x):
@@ -97,6 +107,22 @@ for merge in ("peer", "reduce_scatter"):
     sh.sharded.trace = None
     nb_out[merge] = nb
     nb_report[merge] = (max_all(e_w), int(max_all(n_diff)), max_all(gap), nb_same, max_all(t_nb), max_all(t_x), t)
+    sw = sh.embed_sweep(coords, BETAS)                               # collective: two routed apply passes per step
+    sw_again = sh.embed_sweep(coords, BETAS)
+    e_sw = max(rel(a[:, :1024], b[:, :1024]) for a, b in zip(sw, sw_ref))
+    q_sw = max((a[:, 1024:] - b[:, 1024:]).abs().max().item() for a, b in zip(sw, sw_ref))
+    sw_same = max_all(not all(torch.equal(a, b) for a, b in zip(sw, sw_again))) == 0
+    t_sw = timed(lambda: sh.embed_sweep(coords, BETAS))
+    sw_report[merge] = (max_all(e_sw), max_all(q_sw), sw_same, max_all(t_sw), t)
+    ra = sh.embed_raster(lon_ax, lat_ax, rows=(p0, p1))             # collective: every rank its own points
+    ra_eq = torch.equal(ra, sh.embed(raster_pts))
+    e_ra = rel(ra[:, :1024], raster_ref[:, :1024])
+    q_ra = (ra[:, 1024:] - raster_ref[:, 1024:]).abs().max().item()
+    host = np.empty((p1 - p0, 1280))
+    sh.forward_raster(lon_ax, lat_ax, rows=(p0, p1), out=host)
+    host_eq = np.array_equal(host, sh.embed_raster(lon_ax, lat_ax, rows=(p0, p1), out_dtype=torch.float64).cpu().numpy())
+    t_ra = timed(lambda: sh.embed_raster(lon_ax, lat_ax, rows=(p0, p1)))
+    ra_report[merge] = (max_all(e_ra), max_all(q_ra), max_all(not ra_eq) == 0, max_all(not host_eq) == 0, max_all(t_ra))
     sh.sharded.close()
     del sh
 lo, hi = shard_rows(N, rank, world)                                # query sharding: my slab of a common set, then gather
@@ -121,4 +147,14 @@ if rank == 0:
               f"{t_nb*1e3:.1f} ms per call (list exchange + owner merge {t_x*1e3:.2f} ms, {100 * t_x / t_nb:.1f} %) "
               f"vs {t*1e3:.1f} ms for the sharded embed (world {world}, N={N}+1500 r per rank, M={M})")
         assert e_w < TOL and gap < TOL and same and across
+    for merge, (e_o, e_q, same, t_sw, t) in sw_report.items():
+        print(f"M-sharded sweep beta={BETAS} [{merge}] vs unsharded sweep: max rel-row err {e_o:.2e}, location columns "
+              f"{e_q:.1e}, repeatable {same}; {t_sw*1e3:.1f} ms per call vs {len(BETAS)} x {t*1e3:.1f} = "
+              f"{len(BETAS)*t*1e3:.1f} ms for {len(BETAS)} sharded embed calls (world {world}, N={N}+1500 r per rank, M={M})")
+        assert e_o < 1e-3 and e_q == 0.0 and same
+    for merge, (e_o, e_q, eq, host_eq, t_ra) in ra_report.items():
+        print(f"M-sharded raster {RH}x{RW} [{merge}], a slab of points per rank: equal to the sharded embed of the same "
+              f"coordinates {eq}, vs unsharded embed_raster max rel-row err {e_o:.2e} (location columns {e_q:.1e}), "
+              f"forward_raster(out=) equal to the float64 rows {host_eq}; {t_ra*1e3:.1f} ms per call (world {world}, M={M})")
+        assert eq and host_eq and e_o < 1e-3 and e_q < 1e-3
 dist.destroy_process_group()
