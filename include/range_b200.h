@@ -35,7 +35,10 @@ extern "C" {
 #define RANGE_OUT_F32 1
 #define RANGE_OUT_PACKED 2 /* rows of 6144 B: 1024 fp32 feature columns, then 256 fp64 location columns - every bit of
                               information of the reference's float64 row (its feature columns are fp32 values widened,
-                              range/range.py:222,240) in 60 % of the bytes; range_host_unpack widens on the host */
+                              range/range.py:222,240) in 60 % of the bytes; range_host_unpack widens on the host.
+                              For a database of value width D (range_ctx_set_db_values) a row is 4 round_up(D, 4) bytes
+                              of fp32 features (D columns, then zero padding: the fp64 part stays 16-byte aligned),
+                              then 256 fp64 location columns - 6144 B for D = 1024 */
 
 typedef struct range_ctx range_ctx;
 
@@ -83,9 +86,16 @@ int range_ctx_set_encoder_precision(range_ctx* ctx, int mode);
 
 /* Device-resident database (range_b200/database.py) - replaces the tensors built at range/range.py:78-100.
  *   Kh  (Mpad, 256) fp16 row-major: row-normalised keys, rows >= M zero
- *   Vt  (1024, Mpad) fp16: values transposed (entries contiguous) times vscale, columns >= M zero
+ *   Vt  (Dp, Mpad) fp16: values transposed (entries contiguous) times vscale, columns >= M zero;
+ *       D = value_dim (1 <= D <= RANGE_MAX_VALUE_DIM; RANGE_ERR_INVALID otherwise), Dp = round_up(D, 256), rows >= D zero
  *   xyz (Mpad, 4) fp32: unit vectors (x, y, z, 0)
- * Mpad is a multiple of 128.  Borrowed; must outlive the ctx or the next set_db. */
+ * Mpad is a multiple of 128.  Borrowed; must outlive the ctx or the next set_db.  The value width D sets the shapes
+ * of every entry point below that reads or writes value rows: O and the parts of range_combine_concat /
+ * range_sweep_concat are (N, D) fp32, results are (N, D + 256) or packed rows of 4 round_up(D, 4) + 2048 bytes.
+ * A ctx with no database has D = 1024.  range_ctx_set_db is range_ctx_set_db_values with value_dim = 1024. */
+#define RANGE_MAX_VALUE_DIM 4096
+int range_ctx_set_db_values(range_ctx* ctx, int64_t M, int64_t Mpad, int value_dim, const void* Kh, const void* Vt,
+                            const float* xyz, float vscale);
 int range_ctx_set_db(range_ctx* ctx, int64_t M, int64_t Mpad, const void* Kh, const void* Vt, const float* xyz,
                      float vscale);
 
@@ -150,9 +160,11 @@ int range_encode_raster(range_ctx* ctx, int64_t n_lat, int64_t n_lon, const void
 /* K2: retrieval, range/range.py:213-217 (RANGE) and :213-238 (RANGE+).
  *   stats: sums (N,2) = {sum_j exp(temp (s_j-1)), sum_j exp(geo_temp (g_j-1))}, maxs (N,2) = {max s, max g}
  *          over THIS ctx's database shard; shards merge with SUM / MAX (M-sharding across GPUs).
- *   apply: O (N,1024) fp32 = this shard's contribution to the retrieved feature, normalised with the given
+ *   apply: O (N,D) fp32 = this shard's contribution to the retrieved feature, normalised with the given
  *          (global) sums; shards merge with SUM.
- *   retrieve = stats + apply for an unsharded database. */
+ *   retrieve = stats + apply for an unsharded database.
+ * The workspace size depends on the database's value width D; for D != 1024 the apply pass runs in query chunks that
+ * keep its largest scratch arrays (the partial results of the database splits) within 1 GiB. */
 size_t range_retrieve_workspace_bytes(range_ctx* ctx, int64_t N);
 int range_retrieve_stats(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
                          float geo_temp, float* sums, float* maxs, void* workspace, size_t workspace_bytes,
@@ -164,10 +176,10 @@ int range_retrieve(range_ctx* ctx, int mode, int64_t N, const void* q16, const f
                    float geo_temp, float beta, float* O, void* workspace, size_t workspace_bytes, void* stream);
 
 /* K2 apply + K3 in one call: this shard-less variant writes the retrieved feature straight into the caller's
- * (N,1280) result - row n to out row perm[n] (perm from range_sort_queries, NULL = identity), as fp64
+ * (N,D+256) result - row n to out row perm[n] (perm from range_sort_queries, NULL = identity), as fp64
  * (RANGE_OUT_F64, what range/range.py:222,240 returns) or fp32 - followed by the location columns q64.  For
- * large batches the apply kernel's epilogue does the concat itself (no (N,1024) intermediate); small batches run
- * apply + range_concat_scatter internally. */
+ * large batches of a 1024-wide database the apply kernel's epilogue does the concat itself (no (N,1024)
+ * intermediate); small batches and other widths run apply + range_concat_scatter internally. */
 int range_retrieve_apply_concat(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
                                 float geo_temp, float beta, const float* sums, const float* maxs, const double* q64,
                                 const int32_t* perm, void* out, int out_dtype, void* workspace, size_t workspace_bytes,
@@ -229,12 +241,14 @@ typedef struct range_route {
   int64_t slab_rows;
   float* peer[RANGE_MAX_RANKS];
 } range_route;
+/* Needs a 1024-wide database: RANGE_ERR_UNSUPPORTED for any other value width. */
 int range_retrieve_apply_routed(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
                                 float geo_temp, float beta, const float* sums, const float* maxs,
                                 const range_route* route, void* workspace, size_t workspace_bytes, void* stream);
 
-/* out row perm[n] (NULL = identity) = [ sum_k weights[k] * parts[k][n][0:1024] | q64[n][0:256] ] in out_dtype.
- * parts: host array of n_parts (<= 8) device pointers to (N,1024) fp32; weights: host array or NULL (all 1).
+/* out row perm[n] (NULL = identity) = [ sum_k weights[k] * parts[k][n][0:D] | q64[n][0:256] ] in out_dtype, D the ctx's
+ * value width: (N,D+256) fp64 / fp32 or packed rows.
+ * parts: host array of n_parts (<= 8) device pointers to (N,D) fp32; weights: host array or NULL (all 1).
  * Uses: the slots of an M-sharded receive buffer (weights 1); a beta sweep - range/range.py:238 is linear in beta,
  * so O(beta) = (1-beta) O(0) + beta O(1) serves any number of beta from two apply passes (Readme.md:27-31). */
 int range_combine_concat(range_ctx* ctx, int64_t N, int n_parts, const float* const* parts, const float* weights,
@@ -245,8 +259,8 @@ int range_combine_concat(range_ctx* ctx, int64_t N, int n_parts, const float* co
  * G = sum of the n_slots geo slots, S = sum of the n_slots sem slots, each summed in slot order 0 .. n_slots-1 (the
  * partial rows of the geographic end, beta 0, and of the semantic end, beta 1, that the ranks sent this owner); per
  * column fmaf(w_sem, s, w_geo * g).  geo / sem: host arrays of n_slots (1 <= n_slots <= RANGE_MAX_RANKS) device pointers
- * to (N,1024) fp32; w_geo / w_sem: host arrays of n_betas (1 <= n_betas <= RANGE_SWEEP_MAX_BETAS) weights, normally
- * 1 - beta and beta rounded on the host; outs: host array of n_betas device pointers to (N,1280) results in out_dtype
+ * to (N,D) fp32 (D the ctx's value width); w_geo / w_sem: host arrays of n_betas (1 <= n_betas <= RANGE_SWEEP_MAX_BETAS) weights, normally
+ * 1 - beta and beta rounded on the host; outs: host array of n_betas device pointers to (N,D+256) results in out_dtype
  * (RANGE_OUT_F64 or RANGE_OUT_F32).  Every slot is read once, whatever n_betas.  With n_slots = 1 the rows are bit for bit
  * those of range_combine_concat with parts (G, S) and weights (w_geo, w_sem). */
 #define RANGE_SWEEP_MAX_BETAS 8
@@ -264,11 +278,13 @@ int range_peer_close(void* dptr);
 int range_peer_free(void* dptr);
 
 /* HOST function (no CUDA): widen N packed rows (RANGE_OUT_PACKED, e.g. a pinned staging buffer a device->host copy
- * just filled) into the caller's (N,1280) float64 array - the array range/range.py:222,240 returns - with a thread
- * team of n_threads of its own. */
+ * just filled) of a database of value width value_dim = D (1 <= D <= 4096) into the caller's (N,D+256) float64 array -
+ * the array range/range.py:222,240 returns - with a thread team of n_threads of its own.  range_host_unpack is
+ * range_host_unpack_rows with value_dim = 1024. */
+int range_host_unpack_rows(const void* packed, int64_t N, int value_dim, double* out, int n_threads);
 int range_host_unpack(const void* packed, int64_t N, double* out, int n_threads);
 
-/* K3: out (N,1280) = [O | q64] as fp64 (RANGE_OUT_F64, what the reference returns: range/range.py:222,240)
+/* K3: out (N,D+256) = [O | q64] (O (N,D), D the ctx's value width) as fp64 (RANGE_OUT_F64, what the reference returns: range/range.py:222,240)
  * or fp32. */
 int range_concat(range_ctx* ctx, int64_t N, const float* O, const double* q64, void* out, int out_dtype,
                  void* stream);

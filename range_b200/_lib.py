@@ -16,6 +16,7 @@ RANGE_MAX_RANKS = 8
 RANGE_ENC_F64, RANGE_ENC_F16X3 = 0, 1
 RANGE_TOPK_MAX = 32
 RANGE_SWEEP_MAX_BETAS = 8
+RANGE_MAX_VALUE_DIM = 4096
 
 # every symbol include/range_b200.h declares: name -> (restype, argtypes)
 PROTOTYPES = {
@@ -32,6 +33,7 @@ PROTOTYPES = {
     "range_ctx_prepare_encoder": (c_int, [c_void_p, c_void_p, c_size_t, c_void_p]),
     "range_ctx_set_encoder_precision": (c_int, [c_void_p, c_int]),
     "range_ctx_set_db": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_float]),
+    "range_ctx_set_db_values": (c_int, [c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_float]),
     "range_ctx_set_db_caps": (c_int, [c_void_p, c_int64, c_void_p, c_int64]),
     "range_geo_mask_shape": (c_int, [c_void_p, c_int64, POINTER(c_int32), POINTER(c_int32)]),
     "range_geo_mask": (c_int, [c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p, c_void_p]),
@@ -77,6 +79,7 @@ PROTOTYPES = {
     "range_peer_close": (c_int, [c_void_p]),
     "range_peer_free": (c_int, [c_void_p]),
     "range_host_unpack": (c_int, [c_void_p, c_int64, c_void_p, c_int]),
+    "range_host_unpack_rows": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int]),
     "range_concat": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "range_concat_scatter": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
 }

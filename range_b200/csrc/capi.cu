@@ -37,6 +37,9 @@ int fail(int code, const char* fmt, ...) {
 
 constexpr int kDimK = 256, kDimV = 1024, kBlockQ = 128, kBlockKeys = 128;
 constexpr int64_t kEncodeChunk = 131072;   // queries per encoder pass (bounds the feature workspace)
+// apply pass of a database with value width != 1024: queries per chunk are chosen so that the split partials
+// (splits x rows x D fp32) and the scratch O they are reduced into (rows x D) together stay within this many bytes
+constexpr size_t kApplyChunkBytes = size_t(1) << 30;
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
@@ -97,6 +100,7 @@ struct range_ctx {
   int64_t M = 0, Mpad = 0;
   const void* Kh = nullptr;
   const void* Vt = nullptr;
+  int dim_v = kDimV;               // value width D: Vt is (round_up(D, 256), Mpad)
   const float* xyz = nullptr;
   float vscale = 1.f;
   CUtensorMap tmK128, tmK64, tmV128;
@@ -201,6 +205,7 @@ struct RetrievalPlan {
   int mask_rows, mask_words;                // geo-skip mask: [even-padded query tiles][ceil(tiles / 32)]
   bool pc;                                  // apply with the producer/consumer kernel (retrieval_pc.cu)
   bool stats_pc;                            // statistics with the CTA-pair / four-group kernel (retrieval_pc.cu)
+  int64_t chunk_rows;                       // apply pass in query chunks of this many rows (N for a 1024-wide database)
   size_t off_part_sum, off_part_max, off_sums, off_maxs, off_rowc, off_mask, off_ring, off_flags, off_pc_part, off_pc_scratch, off_part_out, off_O, total;
 };
 
@@ -230,7 +235,7 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   const int64_t qtiles = (N + kBlockQ - 1) / kBlockQ;
   const int64_t tiles = (c->M + kBlockKeys - 1) / kBlockKeys;
   int64_t want = 1;
-  const int64_t ctas = qtiles * 4;
+  const int64_t ctas = qtiles * ((c->dim_v + 255) / 256);    // one CTA per (query tile, 256-wide value slice)
   if (ctas < 2 * c->sm_count) want = (2 * c->sm_count + ctas - 1) / ctas;
   int64_t max_splits = tiles / 8 > 0 ? tiles / 8 : 1;      // at least 8 tiles per split
   if (want > max_splits) want = max_splits;
@@ -276,13 +281,21 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   const int units = apply_pc_units(c->sm_count);
   const int64_t qpairs = (qtiles + 1) / 2;
   const int ov = apply_kernel_override();
-  p.pc = units > 0 && ov != 1 && (ov == 2 || qpairs >= units);
+  // the producer/consumer kernel's consumer pairs cover exactly 1024 value columns: other widths run the CTA pairs
+  p.pc = c->dim_v == kDimV && units > 0 && ov != 1 && (ov == 2 || qpairs >= units);
   p.off_ring = o;     o += p.pc ? align_up(apply_pc_ring_bytes(c->sm_count), 1024) : 0;
   p.off_flags = o;    o += p.pc ? align_up(apply_pc_flag_bytes(c->sm_count, N, c->M), 256) : 0;
   p.off_pc_part = o;  o += p.pc ? align_up(apply_pc_part_bytes(c->sm_count, N, c->M), 256) : 0;
   p.off_pc_scratch = o; o += p.pc ? align_up(apply_pc_scratch_bytes(c->sm_count), 256) : 0;
-  p.off_part_out = o; o += (p.splits > 1 && !p.pc) ? align_up(size_t(p.splits) * N * kDimV * 4, 256) : 0;
-  p.off_O = o;        o += p.pc ? 0 : align_up(size_t(N) * kDimV * 4, 256);   // scratch O of range_retrieve_apply_concat (small batches)
+  p.chunk_rows = N;
+  if (c->dim_v != kDimV) {      // whole CTA pairs of query tiles per chunk
+    const size_t arrays = p.splits > 1 ? p.splits + 1 : 1;     // the split partials and the reduced rows
+    const int64_t rows = int64_t(kApplyChunkBytes / (arrays * c->dim_v * 4)) / 256 * 256;
+    p.chunk_rows = std::min<int64_t>(N, std::max<int64_t>(rows, 256));
+  }
+  const int64_t rows = p.chunk_rows;
+  p.off_part_out = o; o += (p.splits > 1 && !p.pc) ? align_up(size_t(p.splits) * rows * c->dim_v * 4, 256) : 0;
+  p.off_O = o;        o += p.pc ? 0 : align_up(size_t(rows) * c->dim_v * 4, 256);   // scratch O of range_retrieve_apply_concat (small batches)
   p.total = o;
   return p;
 }
@@ -456,21 +469,28 @@ int range_ctx_set_encoder(range_ctx* c, int n_layers, const int32_t* dims, const
   return RANGE_OK;
 }
 
-int range_ctx_set_db(range_ctx* c, int64_t M, int64_t Mpad, const void* Kh, const void* Vt, const float* xyz,
-                     float vscale) {
+int range_ctx_set_db_values(range_ctx* c, int64_t M, int64_t Mpad, int value_dim, const void* Kh, const void* Vt,
+                            const float* xyz, float vscale) {
   if (!c || M <= 0 || Mpad < M || Mpad % kBlockKeys || !Kh || !Vt || !xyz || !(vscale > 0.f))
     return fail(RANGE_ERR_INVALID, "bad database arguments (M=%lld, Mpad=%lld)", (long long)M, (long long)Mpad);
+  if (value_dim < 1 || value_dim > RANGE_MAX_VALUE_DIM)
+    return fail(RANGE_ERR_INVALID, "value_dim = %d: need 1 <= value_dim <= %d", value_dim, RANGE_MAX_VALUE_DIM);
   if (M > (int64_t(1) << 30)) return fail(RANGE_ERR_UNSUPPORTED, "M too large");
   CUDA_TRY(cudaSetDevice(c->device));
   int r = make_tmap(&c->tmK128, Kh, uint64_t(Mpad), kDimK, 128);
   if (r) return r;
   r = make_tmap(&c->tmK64, Kh, uint64_t(Mpad), kDimK, 64);
   if (r) return r;
-  r = make_tmap(&c->tmV128, Vt, kDimV, uint64_t(Mpad), 128);
+  r = make_tmap(&c->tmV128, Vt, uint64_t(value_dim + 255) / 256 * 256, uint64_t(Mpad), 128);
   if (r) return r;
-  c->M = M; c->Mpad = Mpad; c->Kh = Kh; c->Vt = Vt; c->xyz = xyz; c->vscale = vscale;
+  c->M = M; c->Mpad = Mpad; c->Kh = Kh; c->Vt = Vt; c->xyz = xyz; c->vscale = vscale; c->dim_v = value_dim;
   c->caps = nullptr; c->M_total = M;
   return RANGE_OK;
+}
+
+int range_ctx_set_db(range_ctx* c, int64_t M, int64_t Mpad, const void* Kh, const void* Vt, const float* xyz,
+                     float vscale) {
+  return range_ctx_set_db_values(c, M, Mpad, kDimV, Kh, Vt, xyz, vscale);
 }
 
 int range_ctx_set_db_caps(range_ctx* c, int64_t n_tiles, const float* caps, int64_t M_total) {
@@ -818,8 +838,8 @@ int range_retrieve_stats(range_ctx* c, int mode, int64_t N, const void* q16, con
   return RANGE_OK;
 }
 
-// apply pass; the result goes either to O (N,1024) fp32 or, fused with the concat of range/range.py:222,240, to the
-// caller's (N,1280) array `out` (rows through `perm`, fp32 or fp64) together with the location columns q64
+// apply pass; the result goes either to O (N,D) fp32 or, fused with the concat of range/range.py:222,240, to the
+// caller's (N,D+256) array `out` (rows through `perm`, fp32 or fp64) together with the location columns q64
 static bool valid_out_dtype(int d) { return d == RANGE_OUT_F64 || d == RANGE_OUT_F32 || d == RANGE_OUT_PACKED; }
 
 static int check_route(const range_route* r, int64_t N, RowRoute* out) {
@@ -856,6 +876,9 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
   if (out && !valid_out_dtype(out_dtype)) return fail(RANGE_ERR_INVALID, "unknown out dtype");
   RowRoute rr;
   if (int r0 = check_route(route, N, &rr)) return r0;
+  if (route && c->dim_v != kDimV)
+    return fail(RANGE_ERR_UNSUPPORTED, "routed apply (M-sharded database) needs 1024-wide values, this database has %d",
+                c->dim_v);
   const RetrievalPlan p = plan_retrieval(c, N);
   if (workspace_bytes < p.total + 256) return fail(RANGE_ERR_WORKSPACE, "retrieve workspace too small");
   RetrievalArgs a;
@@ -865,7 +888,6 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
   if (r) return r;
   float* rowc = reinterpret_cast<float*>(ws + p.off_rowc);
   CUDA_TRY(launch_row_constants(sums, maxs, qxyz, int(N), a.geo, beta, a.a_sem, a.a_geo, 1.f / c->vscale, rowc, s));
-  const size_t stride = size_t(N) * kDimV;
   const int W = kDimV + kDimK;
   if (p.pc) {
     CUtensorMap tmP;
@@ -893,23 +915,42 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
     g_launches += 2 + (apply_pc_part_bytes(c->sm_count, N, c->M) > 0);
     return RANGE_OK;
   }
-  float* Odst = O ? O : reinterpret_cast<float*>(ws + p.off_O);
-  float* part_out = p.splits > 1 ? reinterpret_cast<float*>(ws + p.off_part_out) : Odst;
-  CUDA_TRY(launch_apply(a, rowc, part_out, stride, s));
-  g_launches += 2;
-  if (p.splits > 1) {
-    CUDA_TRY(launch_reduce_out(part_out, stride, p.splits, stride, Odst, s));
+  // CTA pairs over ceil(D / 256) value slices, in query chunks (plan_retrieval: chunk_rows) that keep the partials of
+  // the database splits within kApplyChunkBytes; one chunk of all N rows for a 1024-wide database
+  const int D = c->dim_v;
+  const size_t out_row = out_dtype == RANGE_OUT_PACKED ? packed_row_bytes(D)
+                                                       : size_t(D + kDimK) * (out_dtype == RANGE_OUT_F64 ? 8 : 4);
+  for (int64_t n0 = 0; n0 < N; n0 += p.chunk_rows) {
+    const int64_t n = std::min(p.chunk_rows, N - n0);
+    RetrievalArgs ac = a;
+    if (n < N) {
+      r = make_tmap(&ac.tmQ, reinterpret_cast<const char*>(q16) + n0 * kDimK * 2, uint64_t(n), kDimK, kBlockQ);
+      if (r) return r;
+      ac.q16 += n0 * kDimK;
+      ac.q_xyz += n0;
+      ac.N = int(n);
+      if (ac.geo_mask) ac.geo_mask += (n0 / kBlockQ) * ac.mask_words;   // n0 is a multiple of 256: whole pairs
+    }
+    float* Odst = O ? O + n0 * D : reinterpret_cast<float*>(ws + p.off_O);
+    float* part_out = p.splits > 1 ? reinterpret_cast<float*>(ws + p.off_part_out) : Odst;
+    CUDA_TRY(launch_apply(ac, rowc + n0 * 8, part_out, size_t(n) * D, D, D, s));
     g_launches += 1;
+    if (p.splits > 1) {
+      CUDA_TRY(launch_reduce_out(part_out, size_t(n) * D, p.splits, size_t(n) * D, Odst, s));
+      g_launches += 1;
+    }
+    if (route) {                  // 1024-wide values only (checked above): one chunk
+      CUDA_TRY(launch_route_rows(Odst, int(N), rr, s));
+      g_launches += 1;
+    } else if (out) {
+      CombineParts one;
+      one.n = 1; one.p[0] = Odst; one.w[0] = 1.f;
+      void* dst = perm ? out : static_cast<char*>(out) + size_t(n0) * out_row;
+      CUDA_TRY(launch_combine_concat(one, q64 + n0 * kDimK, int(n), D, perm ? perm + n0 : nullptr, dst, out_dtype, s));
+      g_launches += 1;
+    }
   }
-  if (route) {
-    CUDA_TRY(launch_route_rows(Odst, int(N), rr, s));
-    g_launches += 1;
-  } else if (out) {
-    CombineParts one;
-    one.n = 1; one.p[0] = Odst; one.w[0] = 1.f;
-    CUDA_TRY(launch_combine_concat(one, q64, int(N), perm, out, out_dtype, s));
-    g_launches += 1;
-  }
+  g_launches += 1;                // row constants
   return RANGE_OK;
 }
 
@@ -1026,7 +1067,7 @@ int range_combine_concat(range_ctx* c, int64_t N, int n_parts, const float* cons
     cp.p[k] = parts[k];
     cp.w[k] = weights ? weights[k] : 1.f;
   }
-  CUDA_TRY(launch_combine_concat(cp, q64, int(N), perm, out, out_dtype, cudaStream_t(stream)));
+  CUDA_TRY(launch_combine_concat(cp, q64, int(N), c->dim_v, perm, out, out_dtype, cudaStream_t(stream)));
   g_launches += 1;
   return RANGE_OK;
 }
@@ -1056,7 +1097,7 @@ int range_sweep_concat(range_ctx* c, int64_t N, int n_slots, const float* const*
     sp.w_sem[b] = w_sem[b];
     sp.out[b] = outs[b];
   }
-  CUDA_TRY(launch_sweep_concat(sp, q64, int(N), perm, out_dtype, cudaStream_t(stream)));
+  CUDA_TRY(launch_sweep_concat(sp, q64, int(N), c->dim_v, perm, out_dtype, cudaStream_t(stream)));
   g_launches += 1;
   return RANGE_OK;
 }
@@ -1120,7 +1161,7 @@ int range_concat_scatter(range_ctx* c, int64_t N, const float* O, const double* 
   if (!valid_out_dtype(out_dtype)) return fail(RANGE_ERR_INVALID, "unknown out dtype");
   CombineParts one;
   one.n = 1; one.p[0] = O; one.w[0] = 1.f;
-  CUDA_TRY(launch_combine_concat(one, q64, int(N), perm, out, out_dtype, cudaStream_t(stream)));
+  CUDA_TRY(launch_combine_concat(one, q64, int(N), c->dim_v, perm, out, out_dtype, cudaStream_t(stream)));
   g_launches += 1;
   return RANGE_OK;
 }

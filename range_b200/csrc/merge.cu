@@ -8,6 +8,7 @@
 //   sweep_concat_kernel     out_b[perm[n]] = [ (1 - beta_b) G[n] + beta_b S[n] | q64[n] ] for up to 8 beta at once - the
 //                           last step of a beta sweep on an M-sharded database: G / S = the sums of the partial slots of
 //                           the geographic (beta 0) and semantic (beta 1) ends; every slot is read once for all beta
+//   *_any_kernel            the two above for a value width D other than 1024: parts (N,D), rows [D | 256]
 //   route_rows_kernel       small batches of an M-sharded database: this rank's (N,1024) partial rows -> the owners'
 //                           receive buffers over NVLink (large batches: the apply kernel's epilogue stores there itself)
 //   peer memory             receive buffers are plain cudaMalloc allocations exported / opened with CUDA IPC handles
@@ -89,6 +90,63 @@ sweep_concat_kernel(const SweepParts parts, const double* __restrict__ q64, int 
   }
 }
 
+// The two kernels above for a value width D != 1024 (the 1024-wide launches keep them): one CTA of 256 threads per row,
+// thread t handles feature columns t, t + 256, ... and location column t.  Per column the same arithmetic.
+// Row of `out`: dtype 0 fp64 / 1 fp32: D + 256 columns; 2 packed: packed_row_bytes(D), fp32 columns [D, round_up(D, 4))
+// written as zero.
+template <int kDtype>
+__device__ __forceinline__ void store_row(void* out, size_t r, int D, int c, float v) {
+  if (kDtype == 0) __stcs(reinterpret_cast<double*>(out) + r * size_t(D + 256) + c, double(v));
+  else if (kDtype == 1) __stcs(reinterpret_cast<float*>(out) + r * size_t(D + 256) + c, v);
+  else __stcs(reinterpret_cast<float*>(reinterpret_cast<char*>(out) + r * rangeb200::packed_row_bytes(D)) + c, v);
+}
+
+template <int kDtype>
+__device__ __forceinline__ void store_q(void* out, size_t r, int D, int t, double q) {
+  if (kDtype == 0) __stcs(reinterpret_cast<double*>(out) + r * size_t(D + 256) + D + t, q);
+  else if (kDtype == 1) __stcs(reinterpret_cast<float*>(out) + r * size_t(D + 256) + D + t, float(q));
+  else __stcs(reinterpret_cast<double*>(reinterpret_cast<char*>(out) + r * rangeb200::packed_row_bytes(D) +
+                                        size_t((D + 3) / 4 * 4) * 4) + t, q);
+}
+
+template <int kDtype>
+__global__ void __launch_bounds__(256)
+combine_concat_any_kernel(const CombineParts parts, const double* __restrict__ q64, int N, int D,
+                          const int* __restrict__ perm, void* __restrict__ out) {
+  const int n = blockIdx.x;
+  const int t = threadIdx.x;
+  const size_t r = perm ? size_t(perm[n]) : size_t(n);
+  const int cols = kDtype == 2 ? (D + 3) / 4 * 4 : D;
+  for (int c = t; c < cols; c += 256) {
+    float a = 0.f;
+    if (c < D)
+      for (int k = 0; k < parts.n; ++k) a = fmaf(parts.w[k], __ldcs(parts.p[k] + size_t(n) * D + c), a);
+    store_row<kDtype>(out, r, D, c, a);
+  }
+  store_q<kDtype>(out, r, D, t, q64[size_t(n) * 256 + t]);
+}
+
+template <int kDtype>      // 0: fp64, 1: fp32
+__global__ void __launch_bounds__(256)
+sweep_concat_any_kernel(const SweepParts parts, const double* __restrict__ q64, int N, int D,
+                        const int* __restrict__ perm) {
+  const int n = blockIdx.x;
+  const int t = threadIdx.x;
+  const size_t r = perm ? size_t(perm[n]) : size_t(n);
+  for (int c = t; c < D; c += 256) {
+    const size_t off = size_t(n) * D + c;
+    float g = __ldcs(parts.geo[0] + off), s = __ldcs(parts.sem[0] + off);
+    for (int k = 1; k < parts.n_slots; ++k) {
+      g += __ldcs(parts.geo[k] + off);
+      s += __ldcs(parts.sem[k] + off);
+    }
+    for (int b = 0; b < parts.n_betas; ++b)
+      store_row<kDtype>(parts.out[b], r, D, c, fmaf(parts.w_sem[b], s, parts.w_geo[b] * g));
+  }
+  const double q = q64[size_t(n) * 256 + t];
+  for (int b = 0; b < parts.n_betas; ++b) store_q<kDtype>(parts.out[b], r, D, t, q);
+}
+
 __global__ void __launch_bounds__(256)
 route_rows_kernel(const float4* __restrict__ O, int N, const RowRoute route) {
   const int n = blockIdx.x;
@@ -100,18 +158,29 @@ route_rows_kernel(const float4* __restrict__ O, int N, const RowRoute route) {
 
 namespace rangeb200 {
 
-cudaError_t launch_combine_concat(const CombineParts& parts, const double* q64, int N, const int* perm, void* out,
+cudaError_t launch_combine_concat(const CombineParts& parts, const double* q64, int N, int D, const int* perm, void* out,
                                   int dtype, cudaStream_t s) {
   if (N <= 0) return cudaSuccess;
+  if (D != 1024) {
+    if (dtype == 0) combine_concat_any_kernel<0><<<N, 256, 0, s>>>(parts, q64, N, D, perm, out);
+    else if (dtype == 1) combine_concat_any_kernel<1><<<N, 256, 0, s>>>(parts, q64, N, D, perm, out);
+    else combine_concat_any_kernel<2><<<N, 256, 0, s>>>(parts, q64, N, D, perm, out);
+    return cudaGetLastError();
+  }
   if (dtype == 0) combine_concat_kernel<0><<<N, 256, 0, s>>>(parts, q64, N, perm, out);
   else if (dtype == 1) combine_concat_kernel<1><<<N, 256, 0, s>>>(parts, q64, N, perm, out);
   else combine_concat_kernel<2><<<N, 256, 0, s>>>(parts, q64, N, perm, out);
   return cudaGetLastError();
 }
 
-cudaError_t launch_sweep_concat(const SweepParts& parts, const double* q64, int N, const int* perm, int dtype,
+cudaError_t launch_sweep_concat(const SweepParts& parts, const double* q64, int N, int D, const int* perm, int dtype,
                                 cudaStream_t s) {
   if (N <= 0) return cudaSuccess;
+  if (D != 1024) {
+    if (dtype == 0) sweep_concat_any_kernel<0><<<N, 256, 0, s>>>(parts, q64, N, D, perm);
+    else sweep_concat_any_kernel<1><<<N, 256, 0, s>>>(parts, q64, N, D, perm);
+    return cudaGetLastError();
+  }
   if (dtype == 0) sweep_concat_kernel<0><<<N, 256, 0, s>>>(parts, q64, N, perm);
   else sweep_concat_kernel<1><<<N, 256, 0, s>>>(parts, q64, N, perm);
   return cudaGetLastError();

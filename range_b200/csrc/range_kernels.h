@@ -112,9 +112,10 @@ struct CombineParts {
   const float* p[kMaxParts] = {};
   float w[kMaxParts] = {};
 };
-// out[perm ? perm[n] : n] = [sum_k w[k] p[k][n][0:1024] | q64[n][0:256]]; dtype 0: fp64 (N,1280), 1: fp32 (N,1280),
-// 2: packed rows of 6144 bytes (1024 fp32 + 256 fp64)
-cudaError_t launch_combine_concat(const CombineParts& parts, const double* q64, int N, const int* perm, void* out,
+// value width D, parts (N,D) fp32: out[perm ? perm[n] : n] = [sum_k w[k] p[k][n][0:D] | q64[n][0:256]]; dtype 0: fp64
+// (N,D+256), 1: fp32 (N,D+256), 2: packed rows of packed_row_bytes(D) (D fp32 padded to a multiple of 4, 256 fp64)
+__host__ __device__ inline size_t packed_row_bytes(int D) { return size_t((D + 3) / 4 * 4) * 4 + 256 * 8; }
+cudaError_t launch_combine_concat(const CombineParts& parts, const double* q64, int N, int D, const int* perm, void* out,
                                   int dtype, cudaStream_t s);
 // O (N,1024) fp32 -> the owners' receive buffers
 cudaError_t launch_route_rows(const float* O, int N, const RowRoute& route, cudaStream_t s);
@@ -129,8 +130,9 @@ struct SweepParts {
   void* out[kSweepMaxBetas] = {};
 };
 // G = sum of the geo slots, S = sum of the sem slots (slot order); for every b < n_betas:
-// out[b][perm ? perm[n] : n] = [fmaf(w_sem[b], S[n], w_geo[b] * G[n]) | q64[n]]; dtype 0: fp64 (N,1280), 1: fp32 (N,1280)
-cudaError_t launch_sweep_concat(const SweepParts& parts, const double* q64, int N, const int* perm, int dtype,
+// out[b][perm ? perm[n] : n] = [fmaf(w_sem[b], S[n], w_geo[b] * G[n]) | q64[n]]; slots (N,D) fp32; dtype 0: fp64
+// (N,D+256), 1: fp32 (N,D+256)
+cudaError_t launch_sweep_concat(const SweepParts& parts, const double* q64, int N, int D, const int* perm, int dtype,
                                 cudaStream_t s);
 
 // ---- spatial batching of the queries (sort.cu) ----------------------------------------------------
@@ -169,8 +171,10 @@ cudaError_t launch_reduce_stats(const float* part_sum, const float* part_max, in
                                 float* maxs, cudaStream_t s);
 cudaError_t launch_row_constants(const float* sums, const float* maxs, const float* q_xyz, int N, int geo,
                                  float beta, float a_sem, float a_geo, float inv_vscale, float* rowc, cudaStream_t s);
-cudaError_t launch_apply(const RetrievalArgs& a, const float* rowc, float* out, size_t out_split_stride,
-                         cudaStream_t s);
+// the CTA-pair apply kernel over ceil(dim_v / 256) value slices (Vt padded to whole slices); row n of split k's
+// result at out + k * out_split_stride + n * out_ld, columns >= dim_v not stored
+cudaError_t launch_apply(const RetrievalArgs& a, const float* rowc, float* out, size_t out_split_stride, int out_ld,
+                         int dim_v, cudaStream_t s);
 // role-specialised persistent apply kernel for large batches (retrieval_pc.cu): P' computed once per tile pair by
 // producer CTAs, handed to the value-slice consumers through an L2-resident ring
 int apply_pc_units(int sm_count);

@@ -23,7 +23,7 @@
 //
 // TMEM (512 columns): apply  [0,128) S/P buf 0 | [128,256) S/P buf 1 | [256,512) O slice    (Q in smem)
 //                     stats  [0,128) Q | [128,256) S buf 0 | [256,384) S buf 1
-// CTA = 128 queries (x one 256-wide slice of the 1024 value dims for apply).  Warp roles: warps 0-7
+// CTA = 128 queries (x one 256-wide slice of the value dims for apply: 4 slices of a 1024-wide database).  Warp roles: warps 0-7
 // softmax/epilogue (warp w owns TMEM lanes 32 (w%4)..+31, group w/4 owns half of a tile's key columns),
 // warp 8 TMA producer, warp 9 MMA issuer + TMEM allocator.
 #include <cstdint>
@@ -367,8 +367,8 @@ __global__ void __launch_bounds__(kPairThreads, 1)
 range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK64,
                         const __grid_constant__ CUtensorMap tmV128, const float4* __restrict__ db_xyz,
                         const float4* __restrict__ rowc, int N, int M, int tiles_per_split, float a_sem,
-                        float* __restrict__ out, size_t out_split_stride, const uint32_t* __restrict__ geo_mask,
-                        int mask_words, long long* __restrict__ prof = nullptr) {
+                        float* __restrict__ out, size_t out_split_stride, int out_ld, int out_cols,
+                        const uint32_t* __restrict__ geo_mask, int mask_words, long long* __restrict__ prof = nullptr) {
   using L = PairSmem;
   constexpr int NS = L::NS, NX = L::NX, kKeys = L::kKeys, kXyzBytes = L::kXyzBytes;
   long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -606,21 +606,31 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
     if (T > 0) {
       ptx::mbar_wait(&bars[L::b_o_full], 0);
       ptx::tc_fence_after();
-      float* orow = out + size_t(split) * out_split_stride + size_t(n) * 1024 + slice * kSliceV + grp * 64;
+      // rows out_ld floats apart; columns >= out_cols (Vt's zero padding rows) are not stored
+      const int col0 = slice * kSliceV + grp * 64;
+      float* orow = out + size_t(split) * out_split_stride + size_t(n) * out_ld + col0;
+      const bool vec = (out_ld & 3) == 0;            // float4 stores need 16-byte aligned rows
 #pragma unroll
       for (int cc = 0; cc < 2; ++cc) {
         uint32_t v[32];
         ptx::tmem_ld32(tmem_o + (uint32_t(quarter * 32) << 16) + grp * 64 + cc * 32, v);
         ptx::tmem_ld_wait();
         if (n < N) {
+          const int left = out_cols - col0 - cc * 32;      // valid columns from orow + cc * 32 on
+          if (vec && left >= 32) {
 #pragma unroll
-          for (int i = 0; i < 32; i += 4) {
-            float4 o;
-            o.x = __uint_as_float(v[i]) * out_scale;
-            o.y = __uint_as_float(v[i + 1]) * out_scale;
-            o.z = __uint_as_float(v[i + 2]) * out_scale;
-            o.w = __uint_as_float(v[i + 3]) * out_scale;
-            *reinterpret_cast<float4*>(orow + cc * 32 + i) = o;
+            for (int i = 0; i < 32; i += 4) {
+              float4 o;
+              o.x = __uint_as_float(v[i]) * out_scale;
+              o.y = __uint_as_float(v[i + 1]) * out_scale;
+              o.z = __uint_as_float(v[i + 2]) * out_scale;
+              o.w = __uint_as_float(v[i + 3]) * out_scale;
+              *reinterpret_cast<float4*>(orow + cc * 32 + i) = o;
+            }
+          } else {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (i < left) orow[cc * 32 + i] = __uint_as_float(v[i]) * out_scale;
           }
         }
       }
@@ -763,6 +773,16 @@ __global__ void reduce_out_kernel(const float4* __restrict__ part, size_t split_
   out[i] = a;
 }
 
+// the same for sizes that are not a multiple of 4 floats (value widths D % 4 != 0)
+__global__ void reduce_out1_kernel(const float* __restrict__ part, size_t split_stride, int splits, size_t total,
+                                   float* __restrict__ out) {
+  const size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  float a = part[i];
+  for (int k = 1; k < splits; ++k) a += part[size_t(k) * split_stride + i];
+  out[i] = a;
+}
+
 template <class K>
 cudaError_t set_smem(K kernel, int bytes) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
@@ -846,8 +866,8 @@ cudaError_t launch_pair(Kern kern, dim3 grid, int bytes, cudaStream_t stream, Ar
   return e;
 }
 
-cudaError_t launch_apply(const RetrievalArgs& a, const float* rowc, float* out, size_t out_split_stride,
-                         cudaStream_t stream) {
+cudaError_t launch_apply(const RetrievalArgs& a, const float* rowc, float* out, size_t out_split_stride, int out_ld,
+                         int dim_v, cudaStream_t stream) {
   cudaError_t e;
   const float4* rc = reinterpret_cast<const float4*>(rowc);
   const int qtiles = (a.N + kBlockQ - 1) / kBlockQ;
@@ -855,25 +875,30 @@ cudaError_t launch_apply(const RetrievalArgs& a, const float* rowc, float* out, 
   const uint32_t* no_mask = nullptr;
   // CTA pairs: cluster (2,1,1) over the query-tile axis (an odd tile count gets one all-padding CTA)
   const int bytes = PairSmem::dynamic_bytes;
-  dim3 grid((qtiles + 1) / 2 * 2, 1024 / kSliceV, a.apply_splits);
+  dim3 grid((qtiles + 1) / 2 * 2, (dim_v + kSliceV - 1) / kSliceV, a.apply_splits);
   if (g_prof_buffer) {   // instrumented build of the same kernel (tools/time_apply.py)
     if ((e = set_smem(range_apply_pair_kernel<true, true>, bytes)) != cudaSuccess) return e;
     return launch_pair(range_apply_pair_kernel<true, true>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.db_xyz,
-                       rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, a.geo_mask, a.mask_words,
-                       g_prof_buffer);
+                       rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v, a.geo_mask,
+                       a.mask_words, g_prof_buffer);
   }
   if ((e = set_smem(range_apply_pair_kernel<true>, bytes)) != cudaSuccess) return e;
   if ((e = set_smem(range_apply_pair_kernel<false>, bytes)) != cudaSuccess) return e;
   if (a.geo)
     return launch_pair(range_apply_pair_kernel<true>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.db_xyz, rc,
-                       a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, a.geo_mask, a.mask_words,
-                       no_prof);
+                       a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v, a.geo_mask,
+                       a.mask_words, no_prof);
   return launch_pair(range_apply_pair_kernel<false>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.db_xyz, rc,
-                     a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, no_mask, 0, no_prof);
+                     a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v, no_mask, 0,
+                     no_prof);
 }
 
 cudaError_t launch_reduce_out(const float* part, size_t split_stride, int splits, size_t total, float* out,
                               cudaStream_t stream) {
+  if (total % 4 || split_stride % 4) {
+    reduce_out1_kernel<<<unsigned((total + 255) / 256), 256, 0, stream>>>(part, split_stride, splits, total, out);
+    return cudaGetLastError();
+  }
   const size_t total4 = total / 4;
   reduce_out_kernel<<<unsigned((total4 + 255) / 256), 256, 0, stream>>>(
       reinterpret_cast<const float4*>(part), split_stride / 4, splits, total4, reinterpret_cast<float4*>(out));

@@ -3,8 +3,10 @@ retrieval kernels stream.
 
 Device layout (what include/range_b200.h:range_ctx_set_db takes):
   Kh  (Mpad, 256)  fp16  row-normalised SatCLIP keys, row-major  -> TMA boxes [128 entries x 64 dims]
-  Vt  (1024, Mpad) fp16  values TRANSPOSED (entries contiguous) x vscale -> TMA boxes [256 dims x 64 entries];
-                         K-major B operand of the P.V tensor-core product, same descriptor as the keys
+  Vt  (Dp, Mpad)   fp16  values TRANSPOSED (entries contiguous) x vscale -> TMA boxes [256 dims x 64 entries];
+                         K-major B operand of the P.V tensor-core product, same descriptor as the keys.  D = value_dim
+                         (1024 for SatMAE features; any width up to MAX_VALUE_DIM), Dp = D rounded up to a whole
+                         256-wide value slice of the apply kernel, rows >= D zero
   xyz (Mpad, 4)    fp32  unit vectors of the entry locations (x, y, z, 0)
   caps (Mpad/128, 4) fp32 bounding cap of every 128-entry tile: (unit centre, angular radius [rad])
 Mpad = M rounded up to 128; padding is zero and masked in-kernel.
@@ -26,6 +28,20 @@ import torch
 from .utils import rad_to_cart
 
 BLOCK = 128
+SLICE_V = 256                   # value dims per CTA of the apply kernel: Vt holds whole slices
+MAX_VALUE_DIM = 4096            # include/range_b200.h: RANGE_MAX_VALUE_DIM
+
+
+def padded_value_dim(D):
+    """rows of Vt for values of width D: D rounded up to a multiple of SLICE_V"""
+    return (D + SLICE_V - 1) // SLICE_V * SLICE_V
+
+
+def value_dim_of(V):
+    """the value width D of an (M, D) image_embeddings array; ValueError unless 1 <= D <= MAX_VALUE_DIM"""
+    if V.ndim != 2 or not 1 <= V.shape[1] <= MAX_VALUE_DIM:
+        raise ValueError(f"RANGE database values must be (M, D) with 1 <= D <= {MAX_VALUE_DIM}, got shape {V.shape}")
+    return int(V.shape[1])
 
 
 def prepare_reference_arrays(db):
@@ -147,8 +163,9 @@ class DeviceDatabase:
         Kraw, V = (a if isinstance(a, np.ndarray) else np.asarray(a)
                    for a in (db["satclip_embeddings"], db["image_embeddings"]))
         self.M_total = xyz.shape[0]
-        if Kraw.ndim != 2 or Kraw.shape[1] != 256 or V.ndim != 2 or V.shape[1] != 1024:
-            raise ValueError(f"RANGE database must have 256-d keys and 1024-d values, got {Kraw.shape[1:]}, {V.shape[1:]}")
+        if Kraw.ndim != 2 or Kraw.shape[1] != 256:
+            raise ValueError(f"RANGE database must have 256-d keys (SatCLIP embeddings), got {Kraw.shape[1:]}")
+        self.value_dim = D = value_dim_of(V)
         if Kraw.shape[0] != self.M_total or V.shape[0] != self.M_total:
             raise ValueError(f"RANGE database arrays disagree on the number of entries: locs {self.M_total}, "
                              f"keys {Kraw.shape[0]}, values {V.shape[0]}")
@@ -170,7 +187,7 @@ class DeviceDatabase:
         vmax = _abs_max_fp32(V[lo:hi] if self.order is None else V)
         self.vscale = 1.0 if vmax == 0.0 or not math.isfinite(vmax) else 2.0 ** math.floor(math.log2(256.0 / vmax))
         self.Kh = torch.zeros(Mpad, 256, dtype=torch.float16, device=dev)
-        self.Vt = torch.zeros(1024, Mpad, dtype=torch.float16, device=dev)
+        self.Vt = torch.zeros(padded_value_dim(D), Mpad, dtype=torch.float16, device=dev)
         step = self.STAGING_ROWS
         for b0 in range(0, M, step):                       # bounded staging memory for 10M-entry databases
             b1 = min(M, b0 + step)
@@ -181,7 +198,7 @@ class DeviceDatabase:
             k = (k / np.linalg.norm(k, ord=2, axis=1, keepdims=True))[back]               # range.py:89
             self.Kh[b0:b1] = torch.from_numpy(np.ascontiguousarray(k)).to(dev).half()
             v = np.asarray(V[idx]).astype(np.float32)[back]                               # range.py:90
-            self.Vt[:, b0:b1] = (torch.from_numpy(np.ascontiguousarray(v)).to(dev) * self.vscale).half().t()
+            self.Vt[:D, b0:b1] = (torch.from_numpy(np.ascontiguousarray(v)).to(dev) * self.vscale).half().t()
         self.xyz = torch.zeros(Mpad, 4, dtype=torch.float32, device=dev)
         self.xyz[:M, :3] = torch.from_numpy(np.ascontiguousarray(xyz)).to(dev)
         self.caps = torch.from_numpy(tile_caps(xyz)).to(dev) if self.order is not None else None
@@ -216,7 +233,7 @@ class DeviceDatabase:
         shard = (-1, -1) if self.shard is None else self.shard
         try:
             with open(tmp, "wb") as f:
-                np.savez(f, version=self.CACHE_VERSION, M=self.M, Mpad=self.Mpad, M_total=self.M_total,
+                np.savez(f, version=self.CACHE_VERSION, M=self.M, Mpad=self.Mpad, M_total=self.M_total, value_dim=self.value_dim,
                          row_range=np.asarray(self.row_range), vscale=self.vscale, shard=np.asarray(shard),
                          fingerprint=np.asarray(fingerprint),
                          Kh=self.Kh.cpu().numpy(), Vt=self.Vt.cpu().numpy(), xyz=self.xyz.cpu().numpy(),
@@ -229,9 +246,10 @@ class DeviceDatabase:
         return path
 
     @classmethod
-    def from_cache(cls, path, device, shard=None, fingerprint=None, spatial_sort=None):
+    def from_cache(cls, path, device, shard=None, fingerprint=None, spatial_sort=None, value_dim=None):
         """load a cache written by save_cache.  Returns None (the caller rebuilds) when the file is missing or was built
-        for another shard, another source (fingerprint, when given) or another row order; raises on a malformed file."""
+        for another shard, another source (fingerprint, when given), another row order or another value width
+        (value_dim, when given; caches without the field hold 1024-wide values); raises on a malformed file."""
         path = cls.cache_path(path, shard)
         if not os.path.exists(path):
             return None
@@ -245,6 +263,9 @@ class DeviceDatabase:
             return None
         if spatial_sort is not None and bool(z["order"].shape[0]) != bool(spatial_sort):
             return None
+        D = int(z["value_dim"]) if "value_dim" in z else 1024
+        if value_dim is not None and D != int(value_dim):
+            return None
         self = cls.__new__(cls)
         dev = torch.device(device)
         self.M, self.Mpad, self.M_total = int(z["M"]), int(z["Mpad"]), int(z["M_total"])
@@ -255,23 +276,26 @@ class DeviceDatabase:
             if self.row_range != (lo, hi):
                 raise ValueError(f"{path}: rows {self.row_range} do not match shard {want} of {self.M_total} entries")
         self.vscale = float(z["vscale"])
+        self.value_dim = D
         self.Kh = torch.from_numpy(z["Kh"]).to(dev)
         self.Vt = torch.from_numpy(z["Vt"]).to(dev)
         self.xyz = torch.from_numpy(z["xyz"]).to(dev)
         self.caps = torch.from_numpy(z["caps"]).to(dev) if z["caps"].shape[0] else None
         self.order = z["order"] if z["order"].shape[0] else None
-        if self.Kh.shape != (self.Mpad, 256) or self.Vt.shape != (1024, self.Mpad) or self.Kh.dtype != torch.float16 \
+        if self.Kh.shape != (self.Mpad, 256) or self.Vt.shape != (padded_value_dim(D), self.Mpad) \
+                or self.Kh.dtype != torch.float16 or not 1 <= D <= MAX_VALUE_DIM \
                 or self.M != self.row_range[1] - self.row_range[0]:
             raise ValueError(f"{path}: malformed database cache")
         return self
 
     @classmethod
-    def synthetic(cls, M, device, seed=0, shard=None):
+    def synthetic(cls, M, device, seed=0, shard=None, value_dim=1024):
         """Benchmark-only: an iid synthetic database (area-uniform locations, N(0,1) keys and values - the worst case
         for the fp16 operands, SURVEY.md 8d) generated block by block straight into the device layout, so 10 M-entry
         databases (25.7 GB in fp16) do not need their 51 GB of fp32 source arrays on the host.
         shard=(rank, world): rows [rank*M/world, (rank+1)*M/world) of the spatially sorted database only - every rank
-        draws the same M locations (same seed) and sorts them the same way, keys / values are iid per entry."""
+        draws the same M locations (same seed) and sorts them the same way, keys / values are iid per entry.
+        value_dim: width D of the values (timing other feature widths)."""
         self = cls.__new__(cls)
         dev = torch.device(device)
         rng = np.random.default_rng(seed)
@@ -281,6 +305,9 @@ class DeviceDatabase:
         xyz = rad_to_cart(locs * math.pi / 180)                                       # range.py:93-95 (fp32)
         self.order = hilbert_order(xyz)
         self.M_total = M
+        self.value_dim = D = int(value_dim)
+        if not 1 <= D <= MAX_VALUE_DIM:
+            raise ValueError(f"value_dim={D}: expected 1 <= value_dim <= {MAX_VALUE_DIM}")
         lo, hi = (0, M) if shard is None else ((M * shard[0]) // shard[1], (M * (shard[0] + 1)) // shard[1])
         self.shard = None if shard is None else (int(shard[0]), int(shard[1]))
         self.row_range = (lo, hi)
@@ -289,15 +316,15 @@ class DeviceDatabase:
         self.Mpad = (m + BLOCK - 1) // BLOCK * BLOCK
         self.vscale = 2.0 ** math.floor(math.log2(256.0 / 6.0))                      # |N(0,1)| < 6
         self.Kh = torch.zeros(self.Mpad, 256, dtype=torch.float16, device=dev)
-        self.Vt = torch.zeros(1024, self.Mpad, dtype=torch.float16, device=dev)
+        self.Vt = torch.zeros(padded_value_dim(D), self.Mpad, dtype=torch.float16, device=dev)
         g = torch.Generator(device=dev).manual_seed(seed if shard is None else seed * 1000003 + 1 + int(shard[0]))
         step = 1 << 18
         for b0 in range(0, m, step):
             b1 = min(m, b0 + step)
             k = torch.randn(b1 - b0, 256, device=dev, generator=g)
             self.Kh[b0:b1] = (k / k.norm(dim=1, keepdim=True)).half()                 # range.py:89
-            v = torch.randn(b1 - b0, 1024, device=dev, generator=g).clamp_(-6.0, 6.0)
-            self.Vt[:, b0:b1] = (v * self.vscale).half().t()
+            v = torch.randn(b1 - b0, D, device=dev, generator=g).clamp_(-6.0, 6.0)
+            self.Vt[:D, b0:b1] = (v * self.vscale).half().t()
         self.xyz = torch.zeros(self.Mpad, 4, dtype=torch.float32, device=dev)
         self.xyz[:m, :3] = torch.from_numpy(np.ascontiguousarray(xyz)).to(dev)
         self.caps = torch.from_numpy(tile_caps(xyz)).to(dev)

@@ -27,21 +27,26 @@ def _stream():
 PACKED_ROW_BYTES = 6144
 
 
-def _out_code(t):
+def packed_row_bytes(D):
+    """bytes of a packed row for values of width D: D fp32 padded to a multiple of 4, then 256 fp64 (6144 for D = 1024)"""
+    return (D + 3) // 4 * 16 + 256 * 8
+
+
+def _out_code(t, D=1024):
     if t.dtype == torch.float64:
         return _lib.RANGE_OUT_F64
     if t.dtype == torch.float32:
         return _lib.RANGE_OUT_F32
-    if t.dtype == torch.uint8 and t.shape[-1] == PACKED_ROW_BYTES:
+    if t.dtype == torch.uint8 and t.shape[-1] == packed_row_bytes(D):
         return _lib.RANGE_OUT_PACKED
-    raise ValueError(f"result tensor must be float64 / float32 (N,1280) or uint8 (N,{PACKED_ROW_BYTES}), got "
+    raise ValueError(f"result tensor must be float64 / float32 (N,{D + 256}) or uint8 (N,{packed_row_bytes(D)}), got "
                      f"{t.dtype} {tuple(t.shape)}")
 
 
-def _new_out(N, dtype, device):
+def _new_out(N, dtype, device, D=1024):
     if dtype == torch.uint8:
-        return torch.empty(N, PACKED_ROW_BYTES, dtype=torch.uint8, device=device)
-    return torch.empty(N, 1280, dtype=dtype, device=device)
+        return torch.empty(N, packed_row_bytes(D), dtype=torch.uint8, device=device)
+    return torch.empty(N, D + 256, dtype=dtype, device=device)
 
 
 class RangeEngine:
@@ -66,6 +71,7 @@ class RangeEngine:
         self.ctx = ctx
         self._ws = {}
         self.db = None
+        self.value_dim = 1024       # width D of the database's values: results are (N, D + 256)
         self.L = int(encoder["L"]) if encoder is not None else int(L)
         # spherical harmonics: the generated polynomials ('analytic', the SatCLIP-L40 checkpoint) or the recurrence
         self.harmonics = harmonics or (encoder or {}).get("harmonics_calculation", "analytic")
@@ -127,11 +133,13 @@ class RangeEngine:
             self.precision = "f16x3"
 
     def set_database(self, db):
-        _lib.check(self.lib.range_ctx_set_db(self.ctx, db.M, db.Mpad, _ptr(db.Kh), _ptr(db.Vt), _ptr(db.xyz),
-                                             float(db.vscale)))
+        D = int(getattr(db, "value_dim", 1024))
+        _lib.check(self.lib.range_ctx_set_db_values(self.ctx, db.M, db.Mpad, D, _ptr(db.Kh), _ptr(db.Vt), _ptr(db.xyz),
+                                                    float(db.vscale)))
         if getattr(db, "caps", None) is not None:
             _lib.check(self.lib.range_ctx_set_db_caps(self.ctx, db.caps.shape[0], _ptr(db.caps), db.M_total))
         self.db = db
+        self.value_dim = D
 
     def _workspace(self, key, nbytes):
         buf = self._ws.get(key)
@@ -238,7 +246,7 @@ class RangeEngine:
 
     def retrieve(self, mode, q16, qxyz, temp, geo_temp, beta, O=None):
         N = q16.shape[0]
-        O = torch.empty(N, 1024, dtype=torch.float32, device=self.device) if O is None else O
+        O = torch.empty(N, self.value_dim, dtype=torch.float32, device=self.device) if O is None else O
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
             _lib.check(self.lib.range_retrieve(self.ctx, MODE[mode], N, _ptr(q16), _ptr(qxyz), temp, geo_temp,
@@ -302,7 +310,7 @@ class RangeEngine:
 
     def retrieve_apply(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, O=None):
         N = q16.shape[0]
-        O = torch.empty(N, 1024, dtype=torch.float32, device=self.device) if O is None else O
+        O = torch.empty(N, self.value_dim, dtype=torch.float32, device=self.device) if O is None else O
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
             _lib.check(self.lib.range_retrieve_apply(self.ctx, MODE[mode], N, _ptr(q16), _ptr(qxyz), temp, geo_temp,
@@ -312,10 +320,10 @@ class RangeEngine:
 
     def retrieve_apply_concat(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, q64, out=None,
                               dtype=torch.float64, perm=None):
-        """apply pass + concat in one call: (N,1280) = [retrieved feature | q64], row n at out[perm[n]]"""
+        """apply pass + concat in one call: (N,D+256) = [retrieved feature | q64], row n at out[perm[n]]"""
         N = q16.shape[0]
-        out = _new_out(N, dtype, self.device) if out is None else out
-        code = _out_code(out)
+        out = _new_out(N, dtype, self.device, self.value_dim) if out is None else out
+        code = _out_code(out, self.value_dim)
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
             _lib.check(self.lib.range_retrieve_apply_concat(
@@ -325,23 +333,23 @@ class RangeEngine:
         return out
 
     def retrieve_concat(self, mode, q16, qxyz, temp, geo_temp, beta, q64, out=None, dtype=torch.float64, perm=None):
-        """statistics + apply + concat in one call (unsharded database): (N,1280) = [retrieved feature | q64], row n at
+        """statistics + apply + concat in one call (unsharded database): (N,D+256) = [retrieved feature | q64], row n at
         out[perm[n]]"""
         N = q16.shape[0]
-        out = _new_out(N, dtype, self.device) if out is None else out
+        out = _new_out(N, dtype, self.device, self.value_dim) if out is None else out
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
             _lib.check(self.lib.range_retrieve_concat(
                 self.ctx, MODE[mode], N, _ptr(q16), _ptr(qxyz), temp, geo_temp, 0.0 if beta is None else float(beta),
-                _ptr(q64), c_void_p(None) if perm is None else _ptr(perm), _ptr(out), _out_code(out), _ptr(ws), ws.numel(),
-                _stream()))
+                _ptr(q64), c_void_p(None) if perm is None else _ptr(perm), _ptr(out), _out_code(out, self.value_dim),
+                _ptr(ws), ws.numel(), _stream()))
         return out
 
     def concat(self, O, q64, out=None, dtype=torch.float64, perm=None):
-        """[O | q64] -> (N,1280); with perm (from sort_queries) row n is written to out[perm[n]]"""
+        """[O | q64] -> (N,D+256); with perm (from sort_queries) row n is written to out[perm[n]]"""
         N = O.shape[0]
-        out = _new_out(N, dtype, self.device) if out is None else out
-        code = _out_code(out)
+        out = _new_out(N, dtype, self.device, self.value_dim) if out is None else out
+        code = _out_code(out, self.value_dim)
         with torch.cuda.device(self.index):
             _lib.check(self.lib.range_concat_scatter(self.ctx, N, _ptr(O), _ptr(q64),
                                                      c_void_p(None) if perm is None else _ptr(perm), _ptr(out), code,
@@ -368,24 +376,25 @@ class RangeEngine:
             if isinstance(p, int):
                 ptrs.append(p)
                 continue
-            if p.dtype != torch.float32 or p.shape != (N, 1024) or not p.is_contiguous():
-                raise ValueError(f"parts must be contiguous (N,1024) float32, got {p.dtype} {tuple(p.shape)}")
+            if p.dtype != torch.float32 or p.shape != (N, self.value_dim) or not p.is_contiguous():
+                raise ValueError(f"parts must be contiguous (N,{self.value_dim}) float32, got {p.dtype} {tuple(p.shape)}")
             ptrs.append(p.data_ptr())
-        out = _new_out(N, dtype, self.device) if out is None else out
+        out = _new_out(N, dtype, self.device, self.value_dim) if out is None else out
         P = (c_void_p * n)(*ptrs)
         W = None if weights is None else (ctypes.c_float * n)(*[float(w) for w in weights])
         with torch.cuda.device(self.index):
             _lib.check(self.lib.range_combine_concat(self.ctx, N, n, P, W, _ptr(q64),
                                                      c_void_p(None) if perm is None else _ptr(perm), _ptr(out),
-                                                     _out_code(out), _stream()))
+                                                     _out_code(out, self.value_dim), _stream()))
         return out
 
     def sweep_concat(self, geo_parts, sem_parts, betas, q64, out_dtype=torch.float32, perm=None, outs=None):
         """[(1 - beta) G[n] + beta S[n] | q64[n]] at row perm[n] for every beta: G / S = the sum of the slots geo_parts /
-        sem_parts (the geographic and semantic ends of a beta sweep; tensors or raw device addresses, (N,1024) fp32),
-        each slot read once per RANGE_SWEEP_MAX_BETAS beta.  Returns a list of (N,1280) tensors in out_dtype (float64 or
+        sem_parts (the geographic and semantic ends of a beta sweep; tensors or raw device addresses, (N,D) fp32),
+        each slot read once per RANGE_SWEEP_MAX_BETAS beta.  Returns a list of (N,D+256) tensors in out_dtype (float64 or
         float32), or fills `outs` (one per beta)."""
         N = q64.shape[0]
+        D = self.value_dim
         if len(geo_parts) != len(sem_parts):
             raise ValueError(f"{len(geo_parts)} geo slots but {len(sem_parts)} sem slots")
 
@@ -395,8 +404,8 @@ class RangeEngine:
                 if isinstance(p, int):
                     ptrs.append(p)
                     continue
-                if p.dtype != torch.float32 or p.shape != (N, 1024) or not p.is_contiguous():
-                    raise ValueError(f"slots must be contiguous (N,1024) float32, got {p.dtype} {tuple(p.shape)}")
+                if p.dtype != torch.float32 or p.shape != (N, D) or not p.is_contiguous():
+                    raise ValueError(f"slots must be contiguous (N,{D}) float32, got {p.dtype} {tuple(p.shape)}")
                 ptrs.append(p.data_ptr())
             return (c_void_p * len(ptrs))(*ptrs)
 
@@ -405,14 +414,14 @@ class RangeEngine:
         if outs is None:
             if out_dtype not in (torch.float64, torch.float32):
                 raise ValueError(f"out_dtype={out_dtype}: expected torch.float64 or torch.float32")
-            outs = [_new_out(N, out_dtype, self.device) for _ in betas]
+            outs = [_new_out(N, out_dtype, self.device, D) for _ in betas]
         if len(outs) != len(betas):
             raise ValueError(f"{len(outs)} outputs for {len(betas)} beta")
-        codes = {_out_code(o) for o in outs}
+        codes = {_out_code(o, D) for o in outs}
         if len(codes) > 1:
             raise ValueError("every output of a sweep must have the same dtype")
         for o in outs:
-            width = PACKED_ROW_BYTES if _out_code(o) == _lib.RANGE_OUT_PACKED else 1280
+            width = packed_row_bytes(D) if _out_code(o, D) == _lib.RANGE_OUT_PACKED else D + 256
             if o.shape != (N, width) or not o.is_contiguous():
                 raise ValueError(f"outputs must be contiguous ({N}, {width}), got {tuple(o.shape)}")
         if N == 0:
@@ -426,5 +435,5 @@ class RangeEngine:
                 _lib.check(self.lib.range_sweep_concat(
                     self.ctx, N, len(geo_parts), G, S, n, (ctypes.c_float * n)(*[1.0 - b for b in bs]),
                     (ctypes.c_float * n)(*bs), _ptr(q64), c_void_p(None) if perm is None else _ptr(perm),
-                    (c_void_p * n)(*[o.data_ptr() for o in group]), _out_code(group[0]), _stream()))
+                    (c_void_p * n)(*[o.data_ptr() for o in group]), _out_code(group[0], D), _stream()))
         return outs

@@ -3,7 +3,8 @@
 Same constructor contract (an argparse-style namespace with location_model_name, pretrained_path, device,
 range_db, beta), same attributes other code reads (location_feature_dim, args.temp, args.geo_temp,
 args.beta), same forward contract: `model(locs)` with locs (N,2) float64 (lon, lat) degrees returns a
-numpy float64 (N, 1280) array = [retrieved visual feature (1024) | L2-normalised SatCLIP embedding (256)].
+numpy float64 (N, D + 256) array = [retrieved visual feature (D) | L2-normalised SatCLIP embedding (256)], D the width
+of the database's image_embeddings (1024 for SatMAE features: (N, 1280)).
 Only the RANGE branches exist here; every other encoder name raises like the reference's final `else`.
 """
 import os
@@ -14,8 +15,8 @@ import torch.nn as nn
 
 from . import _lib
 from .checkpoint import load_satclip_location_encoder
-from .database import DeviceDatabase, open_npz
-from .engine import RangeEngine
+from .database import DeviceDatabase, open_npz, value_dim_of
+from .engine import RangeEngine, packed_row_bytes
 
 # one round of the producer/consumer apply kernel on 148 SMs: 24 units x 2 query tiles of 128
 ROUND_ROWS = 24 * 256
@@ -43,23 +44,30 @@ class LocationEncoder(nn.Module):
         shard = getattr(args, 'db_shard', None)
         enc = load_satclip_location_encoder(args.pretrained_path) if isinstance(args.pretrained_path, str) \
             else args.pretrained_path
-        self.location_feature_dim = 1024 + 256                                             # range.py:86
         cache = getattr(args, 'db_cache', None)        # optional: prepared device layout on disk (database.py)
         ddb = None
-        if isinstance(args.range_db, DeviceDatabase):   # an already prepared device layout (its own shard, if any)
-            ddb = args.range_db
+        db = args.range_db
+        if isinstance(db, DeviceDatabase):              # an already prepared device layout (its own shard, if any)
+            ddb = db
             if shard is not None and tuple(shard) != ddb.shard:
                 raise ValueError(f'db_shard={tuple(shard)} but the prepared database holds shard {ddb.shard}')
             shard = ddb.shard
         elif cache is not None:
-            # the cache is only used when it was built from this source, for this shard (one file per shard)
-            fp = DeviceDatabase.source_fingerprint(args.range_db)
-            ddb = DeviceDatabase.from_cache(cache, args.device, shard=shard, fingerprint=fp)
+            # the cache is only used when it was built from this source, for this shard (one file per shard) and, for an
+            # in-memory database, for the width of its values (a file's fingerprint already pins them)
+            fp = DeviceDatabase.source_fingerprint(db)
+            width = None if isinstance(db, (str, os.PathLike)) else value_dim_of(np.asarray(db['image_embeddings']))
+            ddb = DeviceDatabase.from_cache(cache, args.device, shard=shard, fingerprint=fp, value_dim=width)
         if ddb is None:
-            db = open_npz(args.range_db) if isinstance(args.range_db, str) else args.range_db      # range.py:78
+            db = open_npz(db) if isinstance(db, str) else db                              # range.py:78
             ddb = DeviceDatabase(db, args.device, shard=shard)
             if cache is not None:
                 ddb.save_cache(cache, fingerprint=fp)
+        # range.py:86 hard-codes 1024 + 256 (SatMAE features): here the width of the database's values + 256
+        self.location_feature_dim = ddb.value_dim + 256
+        if shard is not None and shard[1] > 1 and ddb.value_dim != 1024:
+            raise NotImplementedError(f'an M-sharded database (db_shard={tuple(shard)}) needs 1024-wide values; this '
+                                      f'one has {ddb.value_dim}: load it unsharded')
         self.engine = RangeEngine(args.device, encoder=enc, database=ddb)
         self.chunk = int(getattr(args, 'chunk', DEFAULT_CHUNK))
         self.tail = max(1, min(self.chunk, int(getattr(args, 'tail', DEFAULT_TAIL))))
@@ -71,7 +79,7 @@ class LocationEncoder(nn.Module):
         self.out_dtype = np.dtype(getattr(args, 'out_dtype', np.float64))
         if self.out_dtype not in (np.dtype(np.float64), np.dtype(np.float32)):
             raise ValueError(f'out_dtype={self.out_dtype}: expected float64 (the reference\'s) or float32')
-        # how model(locs) hands the (N,1280) float64 result to the host (see _forward_host)
+        # how model(locs) hands the (N,D+256) float64 result to the host (see _forward_host)
         self.host_path = getattr(args, 'host_path', 'auto')
         if self.host_path not in ('auto', 'copy', 'packed'):
             raise ValueError(f"host_path={self.host_path!r}: expected 'auto', 'copy' or 'packed'")
@@ -100,8 +108,12 @@ class LocationEncoder(nn.Module):
         eng = self.engine
         return self.location_model_name == 'RANGE+' and eng.db is not None and eng.db.caps is not None
 
+    def _width(self):
+        """columns of a result row: D + 256 (an M-sharded model serves 1024-wide values only, __init__)"""
+        return 1280 if self.sharded is not None else self.location_feature_dim
+
     def _retrieve_concat(self, q16, qxyz, q64, out, out_dtype, perm):
-        """statistics, apply and concat: (N,1280) = [retrieved feature | q64] with row n at out[perm[n]]"""
+        """statistics, apply and concat: (N,D+256) = [retrieved feature | q64] with row n at out[perm[n]]"""
         eng, a = self.engine, self.args
         name = self.location_model_name
         beta = getattr(a, 'beta', None)
@@ -110,7 +122,7 @@ class LocationEncoder(nn.Module):
 
     @torch.no_grad()
     def embed(self, coords, out=None, out_dtype=torch.float32):
-        """Device-resident path: coords (N,2) fp64 on the device -> (N,1280) device tensor.
+        """Device-resident path: coords (N,2) fp64 on the device -> (N,D+256) device tensor.
         With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call: every rank passes its own
         queries and gets its own rows (distributed.py)."""
         eng, a = self.engine, self.args
@@ -130,7 +142,7 @@ class LocationEncoder(nn.Module):
         """RANGE+ for several beta on the same queries (multi-resolution use, Readme.md:27-31).  range/range.py:238 is
         linear in beta - O(beta) = (1 - beta) O_geo + beta O_sem - so the encoder, the statistics pass and TWO apply
         passes (the geographic and the semantic end) serve any number of beta; each beta then costs one memory-bound
-        blend + concat kernel.  Returns a list of (N,1280) device tensors.
+        blend + concat kernel.  Returns a list of (N,D+256) device tensors.
         With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call: every rank passes its own queries
         and its own beta list (the lists may differ; every rank takes every step) and gets its own rows for each of its
         beta (distributed.py: two routed apply passes per step, one merge kernel for all beta)."""
@@ -222,7 +234,7 @@ class LocationEncoder(nn.Module):
 
     @torch.no_grad()
     def forward(self, coords):
-        """range.py:206-242.  Returns numpy float64 (N, 1280).  Per super-batch (<= 1M queries): every chunk is
+        """range.py:206-242.  Returns numpy float64 (N, D+256).  Per super-batch (<= 1M queries): every chunk is
         batched spatially, the encoder runs once over the whole super-batch (full-width launches), then chunk after
         chunk is retrieved on the current stream while the previous chunk's rows travel to pinned host memory on a
         copy stream."""
@@ -235,15 +247,16 @@ class LocationEncoder(nn.Module):
 
     @torch.no_grad()
     def embed_into(self, coords, out):
-        """forward() writing into the caller's float64 (N,1280) array - e.g. rows of a memory-mapped .npy
+        """forward() writing into the caller's float64 (N,D+256) array - e.g. rows of a memory-mapped .npy
         (save.embed_to_npy): the rows cross PCIe packed into small page-locked staging buffers and a host thread team
         widens them straight into `out` while the GPU works on the next chunks ('packed' path of _forward_host)."""
         coords = torch.as_tensor(coords)
         if coords.dim() != 2 or coords.shape[1] != 2:
             raise ValueError(f'coords must be (N, 2) (lon, lat) degrees, got {tuple(coords.shape)}')
-        if not (isinstance(out, np.ndarray) and out.dtype == np.float64 and out.shape == (coords.shape[0], 1280)
+        W = self._width()
+        if not (isinstance(out, np.ndarray) and out.dtype == np.float64 and out.shape == (coords.shape[0], W)
                 and out.flags['C_CONTIGUOUS'] and out.flags['WRITEABLE']):
-            raise ValueError('out must be a writable C-contiguous float64 (N, 1280) array')
+            raise ValueError(f'out must be a writable C-contiguous float64 (N, {W}) array')
         return self._forward_host(coords.shape[0], coords=coords, result=out)
 
     # ------------------------------------------------------------------ dense lat/lon rasters
@@ -295,7 +308,7 @@ class LocationEncoder(nn.Module):
     @torch.no_grad()
     def embed_raster(self, lon_axis, lat_axis, rows=None, out=None, out_dtype=torch.float32, tables=None):
         """Device-resident dense-grid path (BASELINE config 5): the points [rows[0], rows[1]) of the lat-major raster
-        lat_axis x lon_axis (point p = i * W + j, like coord_grid) -> (n, 1280) device tensor in raster order.  The
+        lat_axis x lon_axis (point p = i * W + j, like coord_grid) -> (n, D+256) device tensor in raster order.  The
         harmonics are evaluated separably (once per distinct latitude / longitude, csrc/encoder_raster.cu); results
         are bit-identical to embed() on the same coordinates.
         With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call: every rank passes the same axes and
@@ -326,20 +339,21 @@ class LocationEncoder(nn.Module):
 
     @torch.no_grad()
     def forward_raster(self, lon_axis, lat_axis, rows=None, out=None):
-        """model(coord_grid(...)) without building the coordinate list on the host: numpy float64 (H * W, 1280).
-        rows=(p0, p1): only those raster points (a rank's slab); out: the caller's float64 (p1 - p0, 1280) array, e.g.
+        """model(coord_grid(...)) without building the coordinate list on the host: numpy float64 (H * W, D+256).
+        rows=(p0, p1): only those raster points (a rank's slab); out: the caller's float64 (p1 - p0, D+256) array, e.g.
         rows of a memory-mapped .npy (filled through the packed path with bounded page-locked memory).
         With an M-sharded database (db_shard / db_group) this is a COLLECTIVE call like embed_raster: every rank passes
         the same axes and its own rows; its points' rows are computed on the device, then copied to the host."""
         tables = self.raster_tables(lon_axis, lat_axis)
         p0, p1 = (0, tables['H'] * tables['W']) if rows is None else rows
-        if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float64 and out.shape == (p1 - p0, 1280)
+        W = self._width()
+        if out is not None and not (isinstance(out, np.ndarray) and out.dtype == np.float64 and out.shape == (p1 - p0, W)
                                     and out.flags['C_CONTIGUOUS'] and out.flags['WRITEABLE']):
-            raise ValueError('out must be a writable C-contiguous float64 (rows, 1280) array')
+            raise ValueError(f'out must be a writable C-contiguous float64 (rows, {W}) array')
         return self._forward_host(p1 - p0, raster=tables, result=out, raster_p0=p0)
 
     def _forward_host(self, N, coords=None, raster=None, result=None, raster_p0=0):
-        """model(locs) -> numpy float64 (N,1280) (range/range.py:222,240).  Two ways to hand the rows to the host:
+        """model(locs) -> numpy float64 (N,D+256) (range/range.py:222,240).  Two ways to hand the rows to the host:
 
         'copy'    chunk by chunk into device buffers; every chunk's float64 rows travel to the page-locked result on a
                   copy stream while the next chunk is computed (pieces get smaller towards the end: only the last
@@ -354,8 +368,9 @@ class LocationEncoder(nn.Module):
         stores from the SMs to host memory run at ~6 GB/s and stall the consumers: 170 ms per 100 000 queries.)"""
         eng = self.engine
         path = self.host_path
+        W = self._width()
         tdtype = torch.float32 if self.out_dtype == np.dtype(np.float32) and result is None else torch.float64
-        row_bytes = 1280 * (4 if tdtype == torch.float32 else 8)
+        row_bytes = W * (4 if tdtype == torch.float32 else 8)
         if result is not None:
             path = 'packed'
         elif tdtype == torch.float32:
@@ -368,16 +383,16 @@ class LocationEncoder(nn.Module):
             else:
                 dev = self._raster_lonlat(raster, raster_p0, N)
             res = self.embed(dev, out_dtype=tdtype)
-            host = torch.empty((N, 1280), dtype=tdtype, pin_memory=N * row_bytes <= self.pinned_limit)
+            host = torch.empty((N, W), dtype=tdtype, pin_memory=N * row_bytes <= self.pinned_limit)
             host.copy_(res)
             if result is None:
                 return host.numpy()
             result[...] = host.numpy()
             return result
         if path == 'packed':
-            result = np.empty((N, 1280), dtype=np.float64) if result is None else result
+            result = np.empty((N, W), dtype=np.float64) if result is None else result
         else:
-            host = torch.empty((N, 1280), dtype=tdtype, pin_memory=True)
+            host = torch.empty((N, W), dtype=tdtype, pin_memory=True)
             result = host.numpy()
         if N == 0:
             return result
@@ -392,11 +407,12 @@ class LocationEncoder(nn.Module):
             if path == 'copy':
                 # three buffers: with two, piece i + 2 waits for the copy of piece i, which is still running when the
                 # pieces shrink faster than their copies (measured: 0.9 ms stall before the fifth piece of 100 000 rows)
-                bufs = [torch.empty(rows, 1280, dtype=tdtype, device=eng.device) for _ in range(min(3, n_pieces))]
+                bufs = [torch.empty(rows, W, dtype=tdtype, device=eng.device) for _ in range(min(3, n_pieces))]
             elif path == 'packed':
                 depth = min(3, n_pieces)
-                bufs = [torch.empty(rows, 6144, dtype=torch.uint8, device=eng.device) for _ in range(depth)]
-                stage = [torch.empty(rows, 6144, dtype=torch.uint8, pin_memory=True) for _ in range(depth)]
+                packed = packed_row_bytes(W - 256)
+                bufs = [torch.empty(rows, packed, dtype=torch.uint8, device=eng.device) for _ in range(depth)]
+                stage = [torch.empty(rows, packed, dtype=torch.uint8, pin_memory=True) for _ in range(depth)]
                 landed = [None] * depth          # (event, result rows, staging rows) of the piece in each slot
             freed = [None] * len(bufs)
             cur = torch.cuda.current_stream()
@@ -408,8 +424,8 @@ class LocationEncoder(nn.Module):
             def unpack(slot):
                 ev, r0, r1 = landed[slot]
                 ev.synchronize()
-                _check_unpack(eng.lib.range_host_unpack(stage[slot].data_ptr(), r1 - r0, result[r0:r1].ctypes.data,
-                                                        self.host_threads))
+                _check_unpack(eng.lib.range_host_unpack_rows(stage[slot].data_ptr(), r1 - r0, W - 256,
+                                                             result[r0:r1].ctypes.data, self.host_threads))
                 landed[slot] = None
 
             i = 0
@@ -481,4 +497,4 @@ class LocationEncoder(nn.Module):
 
 def _check_unpack(code):
     if code != 0:
-        raise RuntimeError(f'range_host_unpack failed ({code})')
+        raise RuntimeError(f'range_host_unpack_rows failed ({code})')
