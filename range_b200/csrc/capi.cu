@@ -38,8 +38,11 @@ int fail(int code, const char* fmt, ...) {
 constexpr int kDimK = 256, kDimV = 1024, kBlockQ = 128, kBlockKeys = 128;
 constexpr int64_t kEncodeChunk = 131072;   // queries per encoder pass (bounds the feature workspace)
 // apply pass of a database with value width != 1024: queries per chunk are chosen so that the split partials
-// (splits x rows x D fp32) and the scratch O they are reduced into (rows x D) together stay within this many bytes
+// (splits x rows x D fp32) and the scratch O they are reduced into (rows x D) together stay within this many bytes.
+// A chunk never drops below one CTA pair (256 rows): when 256 rows alone need more - the splits that keep <= 256 tiles
+// per accumulator (plan_retrieval) are >= 256 at D = 4096 from 8 355 841 entries on - the chunk is 256 rows anyway.
 constexpr size_t kApplyChunkBytes = size_t(1) << 30;
+std::atomic<size_t> g_apply_chunk_bytes{kApplyChunkBytes};     // the bound in force (range_debug_set_apply_chunk_bytes)
 
 inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
@@ -240,8 +243,9 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   int64_t max_splits = tiles / 8 > 0 ? tiles / 8 : 1;      // at least 8 tiles per split
   if (want > max_splits) want = max_splits;
   if (want > 64) want = 64;
-  // the tensor core's fp32 accumulation truncates (retrieval_pc.cu: kAccWindow): at most 256 tiles per accumulator
-  const int64_t for_accuracy = (tiles + 255) / 256 < 256 ? (tiles + 255) / 256 : 256;
+  // the tensor core's fp32 accumulation truncates (retrieval_pc.cu: kAccWindow): at most 256 tiles per accumulator,
+  // however many splits that takes (grid.z allows 65 535: 2^30 entries need 32 768)
+  const int64_t for_accuracy = (tiles + 255) / 256;
   if (want < for_accuracy) want = for_accuracy;
   p.tiles_per_split = int((tiles + want - 1) / want);
   p.splits = int((tiles + p.tiles_per_split - 1) / p.tiles_per_split);
@@ -290,7 +294,7 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   p.chunk_rows = N;
   if (c->dim_v != kDimV) {      // whole CTA pairs of query tiles per chunk
     const size_t arrays = p.splits > 1 ? p.splits + 1 : 1;     // the split partials and the reduced rows
-    const int64_t rows = int64_t(kApplyChunkBytes / (arrays * c->dim_v * 4)) / 256 * 256;
+    const int64_t rows = int64_t(g_apply_chunk_bytes.load() / (arrays * c->dim_v * 4)) / 256 * 256;
     p.chunk_rows = std::min<int64_t>(N, std::max<int64_t>(rows, 256));
   }
   const int64_t rows = p.chunk_rows;
@@ -374,6 +378,27 @@ int range_version(void) { return 100; }
 int64_t range_launch_count(void) { return g_launches.load(); }
 // not in the public header: work decomposition of the producer/consumer apply kernel (tests/test_capi.py; host code only)
 void range_debug_apply_plan(int sm_count, int64_t N, int64_t M, int32_t* out7) { apply_pc_describe_plan(sm_count, N, M, out7); }
+// not in the public header: the retrieval plan of N queries against an unsharded M-entry database of value width
+// value_dim (with tile caps when has_caps) on sm_count SMs (tests/test_apply_plan.py; host code only).  out8 =
+// {splits, tiles_per_split, stats_splits, stats_tiles_per_split, pc, stats_pc, chunk_rows, total workspace bytes}.
+void range_debug_retrieval_plan(int sm_count, int64_t M, int value_dim, int has_caps, int64_t N, int64_t* out8) {
+  static const float caps_sentinel = 0.f;        // plan_retrieval only asks whether the database has caps
+  range_ctx c;
+  c.sm_count = sm_count;
+  c.M = c.M_total = M;
+  c.Mpad = (M + kBlockKeys - 1) / kBlockKeys * kBlockKeys;
+  c.dim_v = value_dim;
+  c.caps = has_caps ? &caps_sentinel : nullptr;
+  const RetrievalPlan p = plan_retrieval(&c, N);
+  const int64_t v[8] = {p.splits, p.tiles_per_split, p.stats_splits, p.stats_tiles_per_split, p.pc, p.stats_pc,
+                        p.chunk_rows, int64_t(p.total)};
+  std::copy(v, v + 8, out8);
+}
+// not in the public header: replaces the byte bound of the apply pass's query chunks (kApplyChunkBytes; 0 restores
+// it) and returns the previous one, so that tests can run databases of value width != 1024 in several chunks
+size_t range_debug_set_apply_chunk_bytes(size_t bytes) {
+  return g_apply_chunk_bytes.exchange(bytes ? bytes : kApplyChunkBytes);
+}
 // not in the public header: feature layout of the tensor-core encoder's first layer for a harmonics table with these
 // chain offsets (tests/test_capi.py; host code only).  off: n_entries + 1 host ints; perm / fmap: K0 ints each (cap >= K0).
 // Returns K0 (<= 0 on bad arguments or cap too small); *rounds = 0 for the production-order layout.
