@@ -227,21 +227,29 @@ int range_topk_merge(range_ctx* ctx, int n_parts, int64_t N, int k, const float*
  * The softmax-weighted sums of range/range.py:213-217,231-238 are associative in the database axis: with the fixed
  * offset (|s|,|g| <= 1) the per-shard exp-sums of range_retrieve_stats merge by SUM (one all-reduce of 8 B per query),
  * the per-shard maxima stay local (they only scale the fp16 weights), and the per-shard outputs of the apply pass,
- * normalised with the global sums, merge by SUM.  range_retrieve_apply_routed is range_retrieve_apply whose result
- * rows leave the GPU from the apply kernel's epilogue: row n belongs to rank n / slab_rows and is stored as 1024 fp32
- * at   route->peer[n / slab_rows] + ((size_t)route->rank * slab_rows + n % slab_rows) * 1024,
- * (slab_rows a multiple of 128: a 128-query tile has one owner; the stores are warp-transposed into full 128-byte lines)
- * peer[r] being rank r's receive buffer [n_ranks][slab_rows][1024] fp32 mapped into this process (range_peer_open;
- * peer[rank] = the local buffer): the partial rows cross NVLink while the tensor cores work on the next tiles, no
- * collective moves them.  After a barrier across the ranks, the owner sums its n_ranks slots in rank order
- * (range_combine_concat: deterministic) and appends the location columns. */
+ * normalised with the global sums, merge by SUM.  range_retrieve_apply_routed_values is range_retrieve_apply whose
+ * result rows go straight to their owners: row n belongs to rank n / slab_rows and is stored as D fp32 (D the ctx's
+ * value width) at
+ *       route->peer[n / slab_rows] + ((size_t)route->rank * slab_rows + n % slab_rows) * D,
+ * (slab_rows a multiple of 128: a 128-query tile has one owner) peer[r] being rank r's receive buffer
+ * [n_ranks][slab_rows][D] fp32 mapped into this process (range_peer_open; peer[rank] = the local buffer; 16-byte
+ * aligned).  Large batches of a 1024-wide database store from the apply kernel's epilogue (warp-transposed into full
+ * 128-byte lines), so the partial rows cross NVLink while the tensor cores work on the next tiles; otherwise one kernel
+ * per query chunk sums the database splits' partial rows and stores each row once, in 16-byte vectors.  No collective
+ * moves them.  After a barrier across the ranks, the owner sums its n_ranks slots in rank order (range_combine_concat:
+ * deterministic) and appends the location columns.  Needs D % 4 == 0 (RANGE_ERR_UNSUPPORTED otherwise): the slots
+ * stay contiguous (slab_rows, D) arrays that range_combine_concat / range_sweep_concat read as they are. */
 #define RANGE_MAX_RANKS 8
 typedef struct range_route {
   int32_t n_ranks, rank;
   int64_t slab_rows;
   float* peer[RANGE_MAX_RANKS];
 } range_route;
-/* Needs a 1024-wide database: RANGE_ERR_UNSUPPORTED for any other value width. */
+int range_retrieve_apply_routed_values(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz,
+                                       float temp, float geo_temp, float beta, const float* sums, const float* maxs,
+                                       const range_route* route, void* workspace, size_t workspace_bytes, void* stream);
+/* range_retrieve_apply_routed_values for a 1024-wide database (rows 1024 floats apart): RANGE_ERR_UNSUPPORTED for any
+ * other value width. */
 int range_retrieve_apply_routed(range_ctx* ctx, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
                                 float geo_temp, float beta, const float* sums, const float* maxs,
                                 const range_route* route, void* workspace, size_t workspace_bytes, void* stream);

@@ -70,6 +70,8 @@ PROTOTYPES = {
                                  c_void_p]),
     "range_retrieve_apply_routed": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float, c_float,
                                             c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "range_retrieve_apply_routed_values": (c_int, [c_void_p, c_int, c_int64, c_void_p, c_void_p, c_float, c_float,
+                                                   c_float, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "range_combine_concat": (c_int, [c_void_p, c_int64, c_int, POINTER(c_void_p), POINTER(c_float), c_void_p, c_void_p,
                                      c_void_p, c_int, c_void_p]),
     "range_sweep_concat": (c_int, [c_void_p, c_int64, c_int, POINTER(c_void_p), POINTER(c_void_p), c_int, POINTER(c_float),

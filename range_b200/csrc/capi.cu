@@ -883,6 +883,8 @@ static int check_route(const range_route* r, int64_t N, RowRoute* out) {
   out->slab = r->slab_rows;
   for (int i = 0; i < r->n_ranks; ++i) {
     if (!r->peer[i]) return fail(RANGE_ERR_INVALID, "route: receive buffer of rank %d is null", i);
+    if (reinterpret_cast<uintptr_t>(r->peer[i]) % 16)        // rows leave in 16-byte vectors
+      return fail(RANGE_ERR_INVALID, "route: receive buffer of rank %d is not 16-byte aligned", i);
     out->peer[i] = r->peer[i];
   }
   return RANGE_OK;
@@ -901,9 +903,9 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
   if (out && !valid_out_dtype(out_dtype)) return fail(RANGE_ERR_INVALID, "unknown out dtype");
   RowRoute rr;
   if (int r0 = check_route(route, N, &rr)) return r0;
-  if (route && c->dim_v != kDimV)
-    return fail(RANGE_ERR_UNSUPPORTED, "routed apply (M-sharded database) needs 1024-wide values, this database has %d",
-                c->dim_v);
+  if (route && c->dim_v % 4)
+    return fail(RANGE_ERR_UNSUPPORTED, "routed apply (M-sharded database) needs a value width that is a multiple of 4, "
+                "this database has %d", c->dim_v);
   const RetrievalPlan p = plan_retrieval(c, N);
   if (workspace_bytes < p.total + 256) return fail(RANGE_ERR_WORKSPACE, "retrieve workspace too small");
   RetrievalArgs a;
@@ -941,7 +943,8 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
     return RANGE_OK;
   }
   // CTA pairs over ceil(D / 256) value slices, in query chunks (plan_retrieval: chunk_rows) that keep the partials of
-  // the database splits within kApplyChunkBytes; one chunk of all N rows for a 1024-wide database
+  // the database splits within kApplyChunkBytes; one chunk of all N rows for a 1024-wide database.  Routed: every
+  // chunk's partials are summed and stored into the owners' receive buffers by one kernel (no O scratch)
   const int D = c->dim_v;
   const size_t out_row = out_dtype == RANGE_OUT_PACKED ? packed_row_bytes(D)
                                                        : size_t(D + kDimK) * (out_dtype == RANGE_OUT_F64 ? 8 : 4);
@@ -960,14 +963,16 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
     float* part_out = p.splits > 1 ? reinterpret_cast<float*>(ws + p.off_part_out) : Odst;
     CUDA_TRY(launch_apply(ac, rowc + n0 * 8, part_out, size_t(n) * D, D, D, s));
     g_launches += 1;
+    if (route) {
+      CUDA_TRY(launch_reduce_route(part_out, size_t(n) * D, p.splits, n0, int(n), D, rr, s));
+      g_launches += 1;
+      continue;
+    }
     if (p.splits > 1) {
       CUDA_TRY(launch_reduce_out(part_out, size_t(n) * D, p.splits, size_t(n) * D, Odst, s));
       g_launches += 1;
     }
-    if (route) {                  // 1024-wide values only (checked above): one chunk
-      CUDA_TRY(launch_route_rows(Odst, int(N), rr, s));
-      g_launches += 1;
-    } else if (out) {
+    if (out) {
       CombineParts one;
       one.n = 1; one.p[0] = Odst; one.w[0] = 1.f;
       void* dst = perm ? out : static_cast<char*>(out) + size_t(n0) * out_row;
@@ -1075,6 +1080,18 @@ int range_topk_merge(range_ctx* c, int n_parts, int64_t N, int k, const float* p
 int range_retrieve_apply_routed(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz, float temp,
                                 float geo_temp, float beta, const float* sums, const float* maxs, const range_route* route,
                                 void* workspace, size_t workspace_bytes, void* stream) {
+  if (!route) return fail(RANGE_ERR_INVALID, "null route");
+  if (c && c->Kh && c->dim_v != kDimV)
+    return fail(RANGE_ERR_UNSUPPORTED, "range_retrieve_apply_routed needs 1024-wide values, this database has %d "
+                "(range_retrieve_apply_routed_values takes any multiple of 4)", c->dim_v);
+  return apply_impl(c, mode, N, q16, qxyz, temp, geo_temp, beta, sums, maxs, nullptr, nullptr, nullptr, nullptr, 0, route,
+                    workspace, workspace_bytes, stream);
+}
+
+int range_retrieve_apply_routed_values(range_ctx* c, int mode, int64_t N, const void* q16, const float* qxyz,
+                                       float temp, float geo_temp, float beta, const float* sums, const float* maxs,
+                                       const range_route* route, void* workspace, size_t workspace_bytes,
+                                       void* stream) {
   if (!route) return fail(RANGE_ERR_INVALID, "null route");
   return apply_impl(c, mode, N, q16, qxyz, temp, geo_temp, beta, sums, maxs, nullptr, nullptr, nullptr, nullptr, 0, route,
                     workspace, workspace_bytes, stream);

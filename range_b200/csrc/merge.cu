@@ -9,8 +9,9 @@
 //                           last step of a beta sweep on an M-sharded database: G / S = the sums of the partial slots of
 //                           the geographic (beta 0) and semantic (beta 1) ends; every slot is read once for all beta
 //   *_any_kernel            the two above for a value width D other than 1024: parts (N,D), rows [D | 256]
-//   route_rows_kernel       small batches of an M-sharded database: this rank's (N,1024) partial rows -> the owners'
-//                           receive buffers over NVLink (large batches: the apply kernel's epilogue stores there itself)
+//   reduce_route_kernel     an M-sharded database, apply pass on CTA pairs (small batches, value widths other than
+//                           1024): one query chunk's split partials summed and each row stored once into its owner's
+//                           receive buffer over NVLink (large 1024-wide batches: the apply kernel's epilogue stores there)
 //   peer memory             receive buffers are plain cudaMalloc allocations exported / opened with CUDA IPC handles
 #include <cstdint>
 #include <cuda_runtime.h>
@@ -147,11 +148,30 @@ sweep_concat_any_kernel(const SweepParts parts, const double* __restrict__ q64, 
   for (int b = 0; b < parts.n_betas; ++b) store_q<kDtype>(parts.out[b], r, D, t, q);
 }
 
+// One thread per 4 columns of a row of the chunk [n0, n0 + rows): the row's split partials part[k][n][0:D] summed in
+// split order 0 .. splits-1 with the additions of reduce_out_kernel (the same bits), then stored once at
+//   peer[g / slab] + ((size_t)rank * slab + g % slab) * D,   g = n0 + n,
+// the owner computed per row (a chunk of 256-row multiples may span several 128-row-multiple slabs).  D % 4 == 0 and
+// 16-byte aligned buffers (range_retrieve_apply_routed_values checks both).
 __global__ void __launch_bounds__(256)
-route_rows_kernel(const float4* __restrict__ O, int N, const RowRoute route) {
-  const int n = blockIdx.x;
-  if (n >= N) return;
-  reinterpret_cast<float4*>(rangeb200::route_row(route, n))[threadIdx.x] = O[size_t(n) * 256 + threadIdx.x];
+reduce_route_kernel(const float4* __restrict__ part, size_t split_stride4, int splits, long long n0, int rows, int D,
+                    const RowRoute route) {
+  const int D4 = D / 4;
+  const size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= size_t(rows) * D4) return;
+  float4 a = __ldcs(part + i);
+  for (int k = 1; k < splits; ++k) {
+    const float4 b = __ldcs(part + size_t(k) * split_stride4 + i);
+    a.x += b.x; a.y += b.y; a.z += b.z; a.w += b.w;
+  }
+  const long long g = n0 + (long long)(i / D4);
+  const int c4 = int(i % D4);
+  const int owner = int(g / route.slab);
+  float* peer = route.peer[0];
+#pragma unroll
+  for (int r = 1; r < rangeb200::kMaxRanks; ++r) peer = owner == r ? route.peer[r] : peer;   // no local copy of peer[]
+  float* row = peer + (size_t(route.rank) * size_t(route.slab) + size_t(g - owner * route.slab)) * D;
+  reinterpret_cast<float4*>(row)[c4] = a;
 }
 
 }  // namespace
@@ -186,9 +206,12 @@ cudaError_t launch_sweep_concat(const SweepParts& parts, const double* q64, int 
   return cudaGetLastError();
 }
 
-cudaError_t launch_route_rows(const float* O, int N, const RowRoute& route, cudaStream_t s) {
-  if (N <= 0) return cudaSuccess;
-  route_rows_kernel<<<N, 256, 0, s>>>(reinterpret_cast<const float4*>(O), N, route);
+cudaError_t launch_reduce_route(const float* part, size_t split_stride, int splits, long long n0, int rows, int D,
+                                const RowRoute& route, cudaStream_t s) {
+  if (rows <= 0) return cudaSuccess;
+  const size_t total4 = size_t(rows) * (D / 4);
+  reduce_route_kernel<<<unsigned((total4 + 255) / 256), 256, 0, s>>>(reinterpret_cast<const float4*>(part),
+                                                                     split_stride / 4, splits, n0, rows, D, route);
   return cudaGetLastError();
 }
 

@@ -94,9 +94,10 @@ cudaError_t launch_concat_q(const double* q64, int N, int DQ, const int* perm, v
 
 // ---- merging partial retrieved features: M-sharded databases, beta sweeps (merge.cu) ------------------------
 constexpr int kMaxRanks = 8, kMaxParts = 8;
-// Where the rows of an M-sharded apply pass go: row n belongs to rank n / slab and is stored (fp32, 1024 wide) in
-// that rank's receive buffer [n_ranks][slab][1024] at slot `rank` - peer[r] is rank r's buffer as mapped into this
-// process (NVLink peer memory; for r == rank the local buffer).  n_ranks == 0: no routing.
+// Where the rows of an M-sharded apply pass go: row n belongs to rank n / slab and is stored (fp32, D wide) in that
+// rank's receive buffer [n_ranks][slab][D] at slot `rank` - peer[r] is rank r's buffer as mapped into this process
+// (NVLink peer memory; for r == rank the local buffer).  n_ranks == 0: no routing.  route_row: D = 1024 (the
+// producer/consumer epilogue); launch_reduce_route takes D as an argument.
 struct RowRoute {
   int n_ranks = 0, rank = 0;
   long long slab = 0;
@@ -117,8 +118,10 @@ struct CombineParts {
 __host__ __device__ inline size_t packed_row_bytes(int D) { return size_t((D + 3) / 4 * 4) * 4 + 256 * 8; }
 cudaError_t launch_combine_concat(const CombineParts& parts, const double* q64, int N, int D, const int* perm, void* out,
                                   int dtype, cudaStream_t s);
-// O (N,1024) fp32 -> the owners' receive buffers
-cudaError_t launch_route_rows(const float* O, int N, const RowRoute& route, cudaStream_t s);
+// rows [n0, n0 + rows) of an apply pass, value width D (D % 4 == 0): part [splits][rows][D] fp32 (split k at
+// part + k * split_stride floats) summed in split order (reduce_out's additions) -> the owners' receive buffers
+cudaError_t launch_reduce_route(const float* part, size_t split_stride, int splits, long long n0, int rows, int D,
+                                const RowRoute& route, cudaStream_t s);
 // a beta sweep's last step: the geographic (beta 0) and semantic (beta 1) ends, each as n_slots partial slots
 constexpr int kSweepMaxBetas = 8;
 struct SweepParts {

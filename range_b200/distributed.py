@@ -11,13 +11,14 @@ running max and the merge needs no rescaling:
     all_gather          the compact queries: fp16 embedding (512 B) + unit vector (16 B) per query
     every rank          row statistics of all P * slab queries over its shard       (range_retrieve_stats)
     all_reduce(SUM)     the exp-sums, 8 B per query; the maxima stay local (they only scale the fp16 weights)
-    every rank          apply pass over its shard with the global sums; the kernel's epilogue stores row n of the
-                        partial result straight into the receive buffer of its owner, rank n / slab, over NVLink
-                        (range_retrieve_apply_routed) - no collective moves the (N,1024) partial outputs
+    every rank          apply pass over its shard with the global sums; row n of the partial result is stored
+                        straight into the receive buffer of its owner, rank n / slab, over NVLink - by the kernel's
+                        epilogue, or by the kernel that sums the database splits (range_retrieve_apply_routed_values)
+                        - no collective moves the (N,D) partial outputs (D: the width of the database's values)
     barrier             a 4-byte all_reduce: every rank's stores have landed
     every rank          sums its P slots in rank order and appends the location columns (range_combine_concat)
 
-merge='reduce_scatter' replaces the routed epilogue + barrier by a local (N,1024) result and NCCL's reduce_scatter
+merge='reduce_scatter' replaces the routed stores + barrier by a local (N,D) result and NCCL's reduce_scatter
 (the comparison baseline; also what runs if the peers' buffers cannot be mapped).
 
 neighbours() shares the steps up to the SUM of the exp-sums, then:
@@ -53,7 +54,7 @@ def merge_sums(sums, group=None):
 
 
 def _reduce_scatter(O_all, world, rank, group):
-    """(P * slab, 1024) partial rows of every rank -> this rank's (slab, 1024) summed rows"""
+    """(P * slab, D) partial rows of every rank -> this rank's (slab, D) summed rows"""
     slab = O_all.shape[0] // world
     mine = torch.empty(slab, O_all.shape[1], dtype=O_all.dtype, device=O_all.device)
     try:
@@ -65,14 +66,16 @@ def _reduce_scatter(O_all, world, rank, group):
 
 
 class PeerBuffers:
-    """Receive buffers [P][slab][1024] fp32, one per rank, each mapped into every rank's process (CUDA IPC through
-    the C ABI: range_peer_alloc / range_peer_open)."""
+    """Receive buffers [P][slab][width] fp32, one per rank, each mapped into every rank's process (CUDA IPC through
+    the C ABI: range_peer_alloc / range_peer_open); width = D, the width of the database's values."""
 
-    def __init__(self, lib, device_index, slab, group):
-        self.lib, self.slab, self.group = lib, int(slab), group
+    width = 1024
+
+    def __init__(self, lib, device_index, slab, group, width=1024):
+        self.lib, self.slab, self.group, self.width = lib, int(slab), group, int(width)
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
         self.index = device_index
-        nbytes = self.world * self.slab * 1024 * 4
+        nbytes = self.world * self.slab * self.width * 4
         self.local = ctypes.c_void_p()
         handle = (ctypes.c_ubyte * 64)()
         with torch.cuda.device(device_index):
@@ -102,13 +105,13 @@ class PeerBuffers:
         sweep: the two ends of a step, each `slab` <= self.slab / 2 rows per rank): slot r of half h starts at
         (h * P + r) * slab rows"""
         assert (half + 1) * slab <= self.slab
-        base = half * self.world * int(slab) * 4096
+        base = half * self.world * int(slab) * self.width * 4
         return _lib.Route(self.world, self.rank, int(slab),
                           (ctypes.c_void_p * _lib.RANGE_MAX_RANKS)(*[p + base for p in self.ptrs]))
 
     def slots(self, slab, half=0):
         """device addresses of this rank's P slots for a step of `slab` rows per rank (in `half`, see route)"""
-        return [self.local.value + (half * self.world + r) * int(slab) * 4096 for r in range(self.world)]
+        return [self.local.value + (half * self.world + r) * int(slab) * self.width * 4 for r in range(self.world)]
 
     def close(self):
         if getattr(self, "local", None) is None:
@@ -129,13 +132,15 @@ class ShardedRetriever:
     """embed() of a model whose database is sharded along M over the ranks of `group`.  A COLLECTIVE call: every rank
     passes its own queries (the counts may differ) and gets its own rows back."""
 
-    MAX_STEP_ROWS = 131072          # P * slab rows per apply launch (receive buffer: 4 KB per row and rank)
+    MAX_STEP_ROWS = 131072          # P * slab rows per apply launch (receive buffer: 4 D bytes per row and rank; values
+                                    # wider than 1024 take fewer rows, _step_rows)
     TOPK_WORKSPACE_BYTES = 1 << 30  # bound of the top-k workspace of a neighbours step (_topk_step_rows)
 
     def __init__(self, engine, group=None, merge="peer"):
         if merge not in ("peer", "reduce_scatter"):
             raise ValueError(f"merge={merge!r}: expected 'peer' or 'reduce_scatter'")
         self.engine, self.group, self.merge = engine, group, merge
+        self.width = int(getattr(engine, "value_dim", 1024))          # D: result rows are D + 256 wide
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
         if self.world > _lib.RANGE_MAX_RANKS:
             raise ValueError(f"at most {_lib.RANGE_MAX_RANKS} ranks share a database, got {self.world}")
@@ -144,8 +149,13 @@ class ShardedRetriever:
         self.collectives = 0            # NCCL calls issued (bench.py reports them)
         self.trace = None               # developer timing: a list collects CUDA events around neighbours' exchange + merge
 
+    def _step_rows(self):
+        """P * slab rows per step of embed: MAX_STEP_ROWS, or for values wider than 1024 the rows of the same bytes
+        (MAX_STEP_ROWS * 1024 // D), so that the receive buffer stays at MAX_STEP_ROWS * 4 KB (512 MB) for any D"""
+        return self.MAX_STEP_ROWS if self.width <= 1024 else self.MAX_STEP_ROWS * 1024 // self.width
+
     def _slab_for(self, n_max, step_rows=None):
-        cap = max(128, (step_rows or self.MAX_STEP_ROWS) // self.world // 128 * 128)
+        cap = max(128, (step_rows or self._step_rows()) // self.world // 128 * 128)
         return min(cap, (n_max + 127) // 128 * 128)
 
     def _ensure_buffers(self, slab):
@@ -156,7 +166,7 @@ class ShardedRetriever:
         if self.buffers is not None:
             self.buffers.close()
         try:
-            self.buffers = PeerBuffers(self.engine.lib, self.engine.index, slab, self.group)
+            self.buffers = PeerBuffers(self.engine.lib, self.engine.index, slab, self.group, self.width)
             ok = torch.ones(1, device=self.engine.device)
         except _lib.RangeError as e:
             print(f"range_b200: rank {self.rank}: peer buffers unavailable ({e}); merging with reduce_scatter")
@@ -198,7 +208,7 @@ class ShardedRetriever:
             yield lo, rows, perm, q64, q16_all, qxyz_all, sums, maxs
 
     def embed(self, mode, coords, temp, geo_temp, beta, sort, out=None, out_dtype=torch.float32):
-        """coords (n,2) fp64 on the device (this rank's queries) -> (n,1280) device tensor (this rank's rows)"""
+        """coords (n,2) fp64 on the device (this rank's queries) -> (n,D+256) device tensor (this rank's rows)"""
         eng, P, me = self.engine, self.world, self.rank
         dev = eng.device
         n = coords.shape[0]
@@ -206,7 +216,7 @@ class ShardedRetriever:
         dist.all_reduce(n_max, op=dist.ReduceOp.MAX, group=self.group)
         n_max = int(n_max.item())
         self.collectives += 1
-        out = _new_out(n, out_dtype, dev) if out is None else out
+        out = _new_out(n, out_dtype, dev, self.width) if out is None else out
         if n_max == 0:
             return out
         slab = self._slab_for(n_max)
@@ -233,14 +243,14 @@ class ShardedRetriever:
         return out
 
     def embed_sweep(self, coords, temp, geo_temp, sort, betas, out_dtype=torch.float32):
-        """RANGE+ for several beta on this rank's queries: coords (n,2) fp64 on the device -> a list of (n,1280) device
+        """RANGE+ for several beta on this rank's queries: coords (n,2) fp64 on the device -> a list of (n,D+256) device
         tensors, one per beta, in this rank's row order.  A COLLECTIVE call: every rank takes every step, whatever its
         own n and its own beta list (the lists may differ between ranks; an empty one returns []).
 
         The steps of embed (RANGE+ statistics, SUM of the exp-sums), then TWO apply passes per step whatever the number
         of beta, as in the unsharded LocationEncoder.embed_sweep: the geographic end (beta 0) and the semantic end (the
         one-softmax retrieval at temp, with RANGE+'s sums).  Peer merge: the two ends are routed into the two halves of
-        the receive buffer (slot r of half h at row (h P + r) slab, PeerBuffers.route / slots; slab <= MAX_STEP_ROWS / 2P,
+        the receive buffer (slot r of half h at row (h P + r) slab, PeerBuffers.route / slots; slab <= _step_rows() / 2P,
         so the buffer is the one embed allocates), one barrier, then range_sweep_concat over this rank's 2 P slots writes
         every beta.  The buffer is reused across steps for the same reason as embed's: a rank's apply passes of step i + 1
         follow its all_gathers of step i + 1 on its stream, which cannot complete before every rank has enqueued - and so,
@@ -257,10 +267,10 @@ class ShardedRetriever:
         dist.all_reduce(n_max, op=dist.ReduceOp.MAX, group=self.group)
         n_max = int(n_max.item())
         self.collectives += 1
-        outs = [_new_out(n, out_dtype, dev) for _ in betas]
+        outs = [_new_out(n, out_dtype, dev, self.width) for _ in betas]
         if n_max == 0:
             return outs
-        slab = self._slab_for(n_max, self.MAX_STEP_ROWS // 2)
+        slab = self._slab_for(n_max, self._step_rows() // 2)
         self._ensure_buffers(2 * slab)
         if self._token is None:
             self._token = torch.zeros(1, device=dev)
@@ -281,7 +291,8 @@ class ShardedRetriever:
             if not betas:
                 continue
             whole = rows == slab
-            dst = [o[lo:lo + slab] if whole else torch.empty(slab, 1280, dtype=o.dtype, device=dev) for o in outs]
+            dst = [o[lo:lo + slab] if whole else torch.empty(slab, self.width + 256, dtype=o.dtype, device=dev)
+                   for o in outs]
             eng.sweep_concat(geo, sem, betas, q64, perm=perm, outs=dst)
             if not whole and rows > 0:
                 for o, d in zip(outs, dst):

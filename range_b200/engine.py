@@ -357,12 +357,12 @@ class RangeEngine:
         return out
 
     def retrieve_apply_routed(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, route):
-        """apply pass of an M-sharded database: this shard's partial rows leave from the kernel's epilogue into the
-        owner ranks' receive buffers (route: _lib.Route with the mapped peer pointers)"""
+        """apply pass of an M-sharded database: this shard's partial rows (value_dim floats each) go straight into the
+        owner ranks' receive buffers (route: _lib.Route with the mapped peer pointers of [P][slab][value_dim] buffers)"""
         N = q16.shape[0]
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
-            _lib.check(self.lib.range_retrieve_apply_routed(
+            _lib.check(self.lib.range_retrieve_apply_routed_values(
                 self.ctx, MODE[mode], N, _ptr(q16), _ptr(qxyz), temp, geo_temp, 0.0 if beta is None else float(beta),
                 _ptr(sums), _ptr(maxs), ctypes.byref(route), _ptr(ws), ws.numel(), _stream()))
 

@@ -26,6 +26,8 @@ DEFAULT_TAPER = 0.5
 
 
 class LocationEncoder(nn.Module):
+    location_feature_dim = 1280     # __init__ sets D + 256 from the database; SatMAE's 1024 + 256 for one built without it
+
     def __init__(self, args):
         super().__init__()
         self.args = args
@@ -65,9 +67,11 @@ class LocationEncoder(nn.Module):
                 ddb.save_cache(cache, fingerprint=fp)
         # range.py:86 hard-codes 1024 + 256 (SatMAE features): here the width of the database's values + 256
         self.location_feature_dim = ddb.value_dim + 256
-        if shard is not None and shard[1] > 1 and ddb.value_dim != 1024:
-            raise NotImplementedError(f'an M-sharded database (db_shard={tuple(shard)}) needs 1024-wide values; this '
-                                      f'one has {ddb.value_dim}: load it unsharded')
+        if shard is not None and shard[1] > 1 and ddb.value_dim % 4:
+            # the shards' partial rows reach their owners in 16-byte vectors (range_retrieve_apply_routed_values)
+            raise NotImplementedError(f'an M-sharded database (db_shard={tuple(shard)}) needs values whose width is a '
+                                      f'multiple of 4 (512, 768, 1024, 2048, ...); this one has {ddb.value_dim}: load '
+                                      f'it unsharded')
         self.engine = RangeEngine(args.device, encoder=enc, database=ddb)
         self.chunk = int(getattr(args, 'chunk', DEFAULT_CHUNK))
         self.tail = max(1, min(self.chunk, int(getattr(args, 'tail', DEFAULT_TAIL))))
@@ -109,8 +113,8 @@ class LocationEncoder(nn.Module):
         return self.location_model_name == 'RANGE+' and eng.db is not None and eng.db.caps is not None
 
     def _width(self):
-        """columns of a result row: D + 256 (an M-sharded model serves 1024-wide values only, __init__)"""
-        return 1280 if self.sharded is not None else self.location_feature_dim
+        """columns of a result row: D + 256"""
+        return self.location_feature_dim
 
     def _retrieve_concat(self, q16, qxyz, q64, out, out_dtype, perm):
         """statistics, apply and concat: (N,D+256) = [retrieved feature | q64] with row n at out[perm[n]]"""
