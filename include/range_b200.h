@@ -108,6 +108,25 @@ int range_ctx_set_db(range_ctx* ctx, int64_t M, int64_t Mpad, const void* Kh, co
  * whole database when this ctx holds one shard of it.  caps = NULL disables.  Reset by range_ctx_set_db. */
 int range_ctx_set_db_caps(range_ctx* ctx, int64_t n_tiles, const float* caps, int64_t M_total);
 
+/* Optional split-fp16 retrieval: Q.K^T and P'.V with every operand as hi + lo fp16 (x = hi + lo, 22 significant bits)
+ * and three kind::f16 products per term (hi.hi + hi.lo + lo.hi), fp32 accumulation - about three times the tensor
+ * work of the default fp16 operands, which keep 11 significant bits of q, K, P' and V.
+ *   Kl  (Mpad, 256) fp16: rn_f16(K - Kh) of the fp32 keys Kh was rounded from, rows >= M zero
+ *   Vtl (Dp, Mpad)  fp16: rn_f16(vscale V - Vt), the same layout as Vt
+ * Borrowed like Kh / Vt (must outlive the ctx or the next set_db); both null clears them.  Reset by range_ctx_set_db.
+ * range_ctx_set_retrieval_precision(ctx, RANGE_RET_F16X3) then switches every retrieval entry point (stats, apply, the
+ * concat wrappers, topk, topk_rows, the routed applies) to the split operands: their `q16` argument becomes the
+ * (N, 512) fp16 row [hi (256) | lo (256)] that range_split_queries builds from q64 (its hi half is range_encode's q16,
+ * bit for bit), and the workspace functions size for that mode.  RANGE_RET_F16X3 without lo halves is
+ * RANGE_ERR_INVALID.  The statistics and apply passes then always run the single-role kernels, the apply pass in query
+ * chunks as for a value width != 1024. */
+#define RANGE_RET_F16 0
+#define RANGE_RET_F16X3 1
+int range_ctx_set_db_lo(range_ctx* ctx, const void* Kl, const void* Vtl);
+int range_ctx_set_retrieval_precision(range_ctx* ctx, int mode);
+/* q64 (N,256) fp64 -> q16x2 (N,512) fp16: [rn_f16(q) | rn_f16(q - rn_f16(q))] */
+int range_split_queries(range_ctx* ctx, int64_t N, const double* q64, void* q16x2, void* stream);
+
 /* Diagnostic: the skip mask the RANGE+ kernels would use for these queries - mask [rows][words] uint32, bit t of
  * row r set = query tile r (128 rows of qxyz) skips the geo term of database tile t.  Shape from
  * range_geo_mask_shape (rows = query tiles rounded up to even).  sums = NULL: the mask of the statistics pass (bound

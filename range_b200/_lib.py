@@ -14,6 +14,7 @@ RANGE_MODE_RANGE, RANGE_MODE_RANGE_PLUS = 0, 1
 RANGE_OUT_F64, RANGE_OUT_F32, RANGE_OUT_PACKED = 0, 1, 2
 RANGE_MAX_RANKS = 8
 RANGE_ENC_F64, RANGE_ENC_F16X3 = 0, 1
+RANGE_RET_F16, RANGE_RET_F16X3 = 0, 1
 RANGE_TOPK_MAX = 32
 RANGE_SWEEP_MAX_BETAS = 8
 RANGE_MAX_VALUE_DIM = 4096
@@ -35,6 +36,9 @@ PROTOTYPES = {
     "range_ctx_set_db": (c_int, [c_void_p, c_int64, c_int64, c_void_p, c_void_p, c_void_p, c_float]),
     "range_ctx_set_db_values": (c_int, [c_void_p, c_int64, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_float]),
     "range_ctx_set_db_caps": (c_int, [c_void_p, c_int64, c_void_p, c_int64]),
+    "range_ctx_set_db_lo": (c_int, [c_void_p, c_void_p, c_void_p]),
+    "range_ctx_set_retrieval_precision": (c_int, [c_void_p, c_int]),
+    "range_split_queries": (c_int, [c_void_p, c_int64, c_void_p, c_void_p, c_void_p]),
     "range_geo_mask_shape": (c_int, [c_void_p, c_int64, POINTER(c_int32), POINTER(c_int32)]),
     "range_geo_mask": (c_int, [c_void_p, c_int64, c_void_p, c_float, c_void_p, c_void_p, c_void_p]),
     "range_sort_workspace_bytes": (c_size_t, [c_void_p, c_int64]),

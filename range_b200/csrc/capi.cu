@@ -107,6 +107,11 @@ struct range_ctx {
   const float* xyz = nullptr;
   float vscale = 1.f;
   CUtensorMap tmK128, tmK64, tmV128;
+  // split-fp16 retrieval (range_ctx_set_db_lo / range_ctx_set_retrieval_precision): lo halves of K and of Vt
+  const void* Kl = nullptr;
+  const void* Vtl = nullptr;
+  CUtensorMap tmKl128, tmKl64, tmVl128;
+  int ret_precision = RANGE_RET_F16;
   const float* caps = nullptr;     // (Mpad / 128, 4) bounding caps of the database tiles, or null
   int64_t M_total = 0;             // entries of the whole (unsharded) database: sets the geo-skip threshold
   // tensor-core encoder (split fp16): prepared weights live in a caller-provided buffer
@@ -232,6 +237,9 @@ int apply_kernel_override() {
   return v;
 }
 
+// halves per query row of the retrieval entry points: q16 (256), or [hi | lo] (512) with split-fp16 operands
+inline int64_t q_cols(const range_ctx* c) { return c->ret_precision == RANGE_RET_F16X3 ? 2 * kDimK : kDimK; }
+
 // Database splits: enough CTAs to fill the SMs when there are few query tiles.
 RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   RetrievalPlan p{};
@@ -248,6 +256,9 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   const int64_t for_accuracy = (tiles + 255) / 256;
   if (want < for_accuracy) want = for_accuracy;
   p.tiles_per_split = int((tiles + want - 1) / want);
+  // Split-fp16 operands update the accumulator three times per k-step: a third of the tiles per split keeps the
+  // truncation deficit of a split at most that of the fp16 plan's (tests/test_retrieval_precision.py)
+  if (c->ret_precision == RANGE_RET_F16X3) p.tiles_per_split = (p.tiles_per_split + 2) / 3;
   p.splits = int((tiles + p.tiles_per_split - 1) / p.tiles_per_split);
   // stats kernel: one CTA per (query tile, split).  Its partials are tiny, so choose the split count that
   // minimises wave quantisation: waves(s) / s with waves(s) = ceil(qtiles * s / SMs), keeping >= 32 tiles per split.
@@ -260,7 +271,9 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   }
   // large batches: CTA pairs (two query tiles per cluster) -> waves are counted in clusters
   const int64_t qpairs0 = (qtiles + 1) / 2, slots = c->sm_count / 2;
-  p.stats_pc = apply_kernel_override() != 1 && slots > 0 && qpairs0 >= apply_pc_units(c->sm_count);
+  // split-fp16 operands: only the single-role kernels have split variants
+  const bool split = c->ret_precision == RANGE_RET_F16X3;
+  p.stats_pc = !split && apply_kernel_override() != 1 && slots > 0 && qpairs0 >= apply_pc_units(c->sm_count);
   if (p.stats_pc) {
     best = 1;
     best_cost = 1e30;
@@ -286,13 +299,13 @@ RetrievalPlan plan_retrieval(const range_ctx* c, int64_t N) {
   const int64_t qpairs = (qtiles + 1) / 2;
   const int ov = apply_kernel_override();
   // the producer/consumer kernel's consumer pairs cover exactly 1024 value columns: other widths run the CTA pairs
-  p.pc = c->dim_v == kDimV && units > 0 && ov != 1 && (ov == 2 || qpairs >= units);
+  p.pc = !split && c->dim_v == kDimV && units > 0 && ov != 1 && (ov == 2 || qpairs >= units);
   p.off_ring = o;     o += p.pc ? align_up(apply_pc_ring_bytes(c->sm_count), 1024) : 0;
   p.off_flags = o;    o += p.pc ? align_up(apply_pc_flag_bytes(c->sm_count, N, c->M), 256) : 0;
   p.off_pc_part = o;  o += p.pc ? align_up(apply_pc_part_bytes(c->sm_count, N, c->M), 256) : 0;
   p.off_pc_scratch = o; o += p.pc ? align_up(apply_pc_scratch_bytes(c->sm_count), 256) : 0;
   p.chunk_rows = N;
-  if (c->dim_v != kDimV) {      // whole CTA pairs of query tiles per chunk
+  if (!p.pc && (c->dim_v != kDimV || split)) {      // whole CTA pairs of query tiles per chunk
     const size_t arrays = p.splits > 1 ? p.splits + 1 : 1;     // the split partials and the reduced rows
     const int64_t rows = int64_t(g_apply_chunk_bytes.load() / (arrays * c->dim_v * 4)) / 256 * 256;
     p.chunk_rows = std::min<int64_t>(N, std::max<int64_t>(rows, 256));
@@ -310,11 +323,21 @@ int fill_args(range_ctx* c, int mode, int64_t N, const void* q16, const float* q
   if (!c || !c->Kh) return fail(RANGE_ERR_INVALID, "database not set");
   if (mode != RANGE_MODE_RANGE && mode != RANGE_MODE_RANGE_PLUS) return fail(RANGE_ERR_INVALID, "unknown mode %d", mode);
   if (N <= 0 || N > (int64_t(1) << 30)) return fail(RANGE_ERR_INVALID, "N out of range");
-  int r = make_tmap(&a->tmQ, q16, uint64_t(N), kDimK, kBlockQ);
+  int r = make_tmap(&a->tmQ, q16, uint64_t(N), uint64_t(q_cols(c)), kBlockQ);
   if (r) return r;
   a->tmK128 = c->tmK128;
   a->tmK64 = c->tmK64;
   a->tmV128 = c->tmV128;
+  a->split = c->ret_precision == RANGE_RET_F16X3;
+  if (a->split) {
+    a->tmKl128 = c->tmKl128;
+    a->tmKl64 = c->tmKl64;
+    a->tmVl128 = c->tmVl128;
+  } else {          // unused by the fp16 kernels
+    a->tmKl128 = c->tmK128;
+    a->tmKl64 = c->tmK64;
+    a->tmVl128 = c->tmV128;
+  }
   a->q16 = reinterpret_cast<const __half*>(q16);
   a->db_xyz = reinterpret_cast<const float4*>(c->xyz);
   a->q_xyz = reinterpret_cast<const float4*>(qxyz);
@@ -381,7 +404,7 @@ void range_debug_apply_plan(int sm_count, int64_t N, int64_t M, int32_t* out7) {
 // not in the public header: the retrieval plan of N queries against an unsharded M-entry database of value width
 // value_dim (with tile caps when has_caps) on sm_count SMs (tests/test_apply_plan.py; host code only).  out8 =
 // {splits, tiles_per_split, stats_splits, stats_tiles_per_split, pc, stats_pc, chunk_rows, total workspace bytes}.
-void range_debug_retrieval_plan(int sm_count, int64_t M, int value_dim, int has_caps, int64_t N, int64_t* out8) {
+static void debug_plan(int sm_count, int64_t M, int value_dim, int has_caps, int precision, int64_t N, int64_t* out8) {
   static const float caps_sentinel = 0.f;        // plan_retrieval only asks whether the database has caps
   range_ctx c;
   c.sm_count = sm_count;
@@ -389,10 +412,19 @@ void range_debug_retrieval_plan(int sm_count, int64_t M, int value_dim, int has_
   c.Mpad = (M + kBlockKeys - 1) / kBlockKeys * kBlockKeys;
   c.dim_v = value_dim;
   c.caps = has_caps ? &caps_sentinel : nullptr;
+  c.ret_precision = precision;
   const RetrievalPlan p = plan_retrieval(&c, N);
   const int64_t v[8] = {p.splits, p.tiles_per_split, p.stats_splits, p.stats_tiles_per_split, p.pc, p.stats_pc,
                         p.chunk_rows, int64_t(p.total)};
   std::copy(v, v + 8, out8);
+}
+void range_debug_retrieval_plan(int sm_count, int64_t M, int value_dim, int has_caps, int64_t N, int64_t* out8) {
+  debug_plan(sm_count, M, value_dim, has_caps, RANGE_RET_F16, N, out8);
+}
+// not in the public header: the same plan for a ctx in retrieval precision `precision` (RANGE_RET_*; host code only)
+void range_debug_retrieval_plan_precision(int sm_count, int64_t M, int value_dim, int has_caps, int precision, int64_t N,
+                                          int64_t* out8) {
+  debug_plan(sm_count, M, value_dim, has_caps, precision, N, out8);
 }
 // not in the public header: replaces the byte bound of the apply pass's query chunks (kApplyChunkBytes; 0 restores
 // it) and returns the previous one, so that tests can run databases of value width != 1024 in several chunks
@@ -510,6 +542,44 @@ int range_ctx_set_db_values(range_ctx* c, int64_t M, int64_t Mpad, int value_dim
   if (r) return r;
   c->M = M; c->Mpad = Mpad; c->Kh = Kh; c->Vt = Vt; c->xyz = xyz; c->vscale = vscale; c->dim_v = value_dim;
   c->caps = nullptr; c->M_total = M;
+  c->Kl = nullptr; c->Vtl = nullptr;          // the lo halves belonged to the previous database
+  c->ret_precision = RANGE_RET_F16;
+  return RANGE_OK;
+}
+
+int range_ctx_set_db_lo(range_ctx* c, const void* Kl, const void* Vtl) {
+  if (!c || !c->Kh) return fail(RANGE_ERR_INVALID, "database not set");
+  if (!Kl && !Vtl) {
+    c->Kl = c->Vtl = nullptr;
+    c->ret_precision = RANGE_RET_F16;
+    return RANGE_OK;
+  }
+  if (!Kl || !Vtl) return fail(RANGE_ERR_INVALID, "Kl and Vtl must both be set (or both null)");
+  CUDA_TRY(cudaSetDevice(c->device));
+  int r = make_tmap(&c->tmKl128, Kl, uint64_t(c->Mpad), kDimK, 128);
+  if (r) return r;
+  r = make_tmap(&c->tmKl64, Kl, uint64_t(c->Mpad), kDimK, 64);
+  if (r) return r;
+  r = make_tmap(&c->tmVl128, Vtl, uint64_t(c->dim_v + 255) / 256 * 256, uint64_t(c->Mpad), 128);
+  if (r) return r;
+  c->Kl = Kl;
+  c->Vtl = Vtl;
+  return RANGE_OK;
+}
+
+int range_ctx_set_retrieval_precision(range_ctx* c, int mode) {
+  if (!c) return fail(RANGE_ERR_INVALID, "null ctx");
+  if (mode != RANGE_RET_F16 && mode != RANGE_RET_F16X3) return fail(RANGE_ERR_INVALID, "unknown retrieval precision %d", mode);
+  if (mode == RANGE_RET_F16X3 && !c->Kl)
+    return fail(RANGE_ERR_INVALID, "RANGE_RET_F16X3 needs the lo halves of the database (range_ctx_set_db_lo)");
+  c->ret_precision = mode;
+  return RANGE_OK;
+}
+
+int range_split_queries(range_ctx* c, int64_t N, const double* q64, void* q16x2, void* stream) {
+  if (!c || N <= 0 || N > (int64_t(1) << 30) || !q64 || !q16x2) return fail(RANGE_ERR_INVALID, "bad arguments");
+  CUDA_TRY(launch_split_queries(q64, int(N), q16x2, cudaStream_t(stream)));
+  g_launches += 1;
   return RANGE_OK;
 }
 
@@ -952,9 +1022,10 @@ static int apply_impl(range_ctx* c, int mode, int64_t N, const void* q16, const 
     const int64_t n = std::min(p.chunk_rows, N - n0);
     RetrievalArgs ac = a;
     if (n < N) {
-      r = make_tmap(&ac.tmQ, reinterpret_cast<const char*>(q16) + n0 * kDimK * 2, uint64_t(n), kDimK, kBlockQ);
+      r = make_tmap(&ac.tmQ, reinterpret_cast<const char*>(q16) + n0 * q_cols(c) * 2, uint64_t(n), uint64_t(q_cols(c)),
+                    kBlockQ);
       if (r) return r;
-      ac.q16 += n0 * kDimK;
+      ac.q16 += n0 * q_cols(c);
       ac.q_xyz += n0;
       ac.N = int(n);
       if (ac.geo_mask) ac.geo_mask += (n0 / kBlockQ) * ac.mask_words;   // n0 is a multiple of 256: whole pairs

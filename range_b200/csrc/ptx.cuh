@@ -157,11 +157,12 @@ __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.
 // Q tile (rows q0..q0+127 of q16, 256 halves each) -> TMEM columns [tmem_q, tmem_q+128): lane = row,
 // column = dim / 2 (two fp16 per 32-bit column) - the A-operand layout of kind::f16 for M = 128.
 // 16 warps: warp w writes lanes 32 (w%4).., column group w/4 = dims [64 g, 64 g + 64).
+// ld: halves from one row of q16 to the next (512 for the [hi | lo] rows of split-fp16 retrieval).
 __device__ __forceinline__ void load_q_to_tmem16(const __half* __restrict__ q16, int q0, int N, uint32_t tmem_q,
-                                                 int warp, int lane) {
+                                                 int warp, int lane, int ld = 256) {
   const int grp = warp >> 2, quarter = warp & 3;
   const int n = q0 + quarter * 32 + lane;
-  const uint4* src = reinterpret_cast<const uint4*>(q16 + size_t(n < N ? n : 0) * 256 + grp * 64);
+  const uint4* src = reinterpret_cast<const uint4*>(q16 + size_t(n < N ? n : 0) * ld + grp * 64);
   uint32_t v[32];
 #pragma unroll
   for (int i = 0; i < 8; ++i) {

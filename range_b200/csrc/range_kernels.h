@@ -151,6 +151,10 @@ struct RetrievalArgs {
   CUtensorMap tmK128;   // keys, box [128 entries x 64 dims]
   CUtensorMap tmK64;    // keys, box [64 entries x 64 dims]          (CTA-pair kernel: half a K tile per CTA)
   CUtensorMap tmV128;   // values^T, box [128 dims x 64 entries]    (CTA-pair kernel: half a Vt tile per CTA)
+  // split-fp16 retrieval (split != 0): the lo halves Kl / Vtl with the same boxes as tmK128 / tmK64 / tmV128;
+  // q16 rows are then 512 halves [hi | lo] and tmQ covers all 512 columns
+  CUtensorMap tmKl128, tmKl64, tmVl128;
+  int split;
   const __half* q16;
   const float4* db_xyz;
   const float4* q_xyz;
@@ -196,6 +200,8 @@ size_t apply_pc_scratch_bytes(int sm_count);   // consumers' accumulation-window
 cudaError_t launch_stats_pc(const RetrievalArgs& a, float* part_sum, float* part_max, cudaStream_t s);
 cudaError_t launch_reduce_out(const float* part, size_t split_stride, int splits, size_t total, float* out,
                               cudaStream_t s);
+// q64 (N,256) fp64 -> q16x2 (N,512) fp16 rows [hi | lo]: hi = rn_f16(q) (range_encode's q16), lo = rn_f16(q - hi)
+cudaError_t launch_split_queries(const double* q64, int N, void* q16x2, cudaStream_t s);
 
 // ---- retrieval neighbours: the k largest retrieval weights per query (topk.cu) ------------------------------------
 constexpr int kTopkMax = 32, kTopkMaxSplits = 64;

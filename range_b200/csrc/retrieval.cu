@@ -36,6 +36,7 @@
 
 #include "ptx.cuh"
 #include "range_kernels.h"
+#include "split_f16.cuh"
 
 namespace {
 
@@ -56,6 +57,7 @@ constexpr int kPolyModApply = RANGE_POLY_APPLY;
 constexpr int kPolyModStats = RANGE_POLY_STATS;
 constexpr uint32_t kTmemQ = 0;      // column offsets
 constexpr uint32_t kTmemS = 128;
+constexpr uint32_t kTmemQl = 384;   // split-fp16 statistics: Ql after the two S buffers
 
 template <int NS, int NX, int kXyzBytes>
 struct SmemLayout {
@@ -117,9 +119,12 @@ struct StatsSmem {
   static constexpr int dynamic_bytes = total + 1024;
 };
 
-template <bool kGeo>
+// kSplit: split-fp16 operands (q = Qh + Ql, K = Kh + Kl), S = Qh.Kh + Qh.Kl + Ql.Kh in one fp32 accumulator.  Ql sits in
+// TMEM columns [384, 512); a stage holds one 64-dim box of Kh and the same box of Kl, so a tile is four stages.
+template <bool kGeo, bool kSplit = false>
 __global__ void __launch_bounds__(kStatsThreads, 1)
-range_stats_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __restrict__ q16,
+range_stats_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmKl,
+                   const __half* __restrict__ q16,
                    const float4* __restrict__ db_xyz, const float4* __restrict__ q_xyz, int N, int M,
                    int tiles_per_split, float a_sem, float a_geo, float* __restrict__ part_sum,
                    float* __restrict__ part_max, const uint32_t* __restrict__ geo_mask, int mask_words) {
@@ -161,7 +166,14 @@ range_stats_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __rest
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);
   const uint32_t smem_u = __shfl_sync(0xffffffffu, ptx::smem_u32(smem), 0);
   const uint32_t bars_u = smem_u + L::bars;
-  if (warp < kStatsWarps) ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane);
+  if (warp < kStatsWarps) {
+    if constexpr (kSplit) {
+      ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane, 512);
+      ptx::load_q_to_tmem16(q16 + 256, q0, N, tmem_base + kTmemQl, warp, lane, 512);
+    } else {
+      ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane);
+    }
+  }
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();
@@ -170,9 +182,21 @@ range_stats_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __rest
     // ===== TMA producer =====
     if (lane == 0) {
       ptx::prefetch_tmap(&tmK);
+      if (kSplit) ptx::prefetch_tmap(&tmKl);
       PipeState st;
       for (int j = 0; j < T; ++j) {
         const int key0 = (t_begin + j) * kKeys;
+        if constexpr (kSplit) {
+#pragma unroll
+          for (int d = 0; d < 4; ++d) {     // dims [64 d, 64 d + 64): Kh box, then the Kl box
+            ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
+            uint8_t* dst = smem + L::stages + st.idx * kStageBytes;
+            ptx::mbar_expect_tx(&bars[L::b_stage_full + st.idx], kStageBytes);
+            ptx::tma_load_2d(dst, &tmK, &bars[L::b_stage_full + st.idx], d * 64, key0);
+            ptx::tma_load_2d(dst + 16384, &tmKl, &bars[L::b_stage_full + st.idx], d * 64, key0);
+            st.advance<NS>();
+          }
+        } else
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
           ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
@@ -201,6 +225,29 @@ range_stats_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __rest
       const int b = j & 1;
       ptx::mbar_wait(&bars[L::b_s_empty + b], ((j >> 1) & 1) ^ 1);
       ptx::tc_fence_after();
+      if constexpr (kSplit) {
+#pragma unroll
+        for (int d = 0; d < 4; ++d) {
+          ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
+          ptx::tc_fence_after();
+          if (ptx::elect_one()) {
+            const uint32_t b_base = smem_u + L::stages + st.idx * kStageBytes;
+            const uint32_t s_col = tmem_base + kTmemS + b * kKeys;
+#pragma unroll
+            for (int kk = 0; kk < 4; ++kk) {
+              const uint32_t qc = d * 32 + kk * 8;
+              const uint64_t kh = ptx::umma_desc_kmajor_sw128(b_base + kk * 32);
+              const uint64_t kl = ptx::umma_desc_kmajor_sw128(b_base + 16384 + kk * 32);
+              ptx::umma_f16_ts(s_col, tmem_base + kTmemQ + qc, kh, idesc, (d | kk) != 0);
+              ptx::umma_f16_ts(s_col, tmem_base + kTmemQ + qc, kl, idesc, 1);
+              ptx::umma_f16_ts(s_col, tmem_base + kTmemQl + qc, kh, idesc, 1);
+            }
+            ptx::umma_commit_u32(bars_u + 8 * (L::b_stage_empty + st.idx));
+          }
+          __syncwarp();
+          st.advance<NS>();
+        }
+      } else
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
@@ -359,18 +406,46 @@ struct PairSmem : ApplySmem {
 // evaluating part of the exponentials on the FMA pipe (slower: register spills under the 112-register cap).
 // Per tile a warp passes ONE barrier: the entries' xyz bytes are credited to the same mbarrier the MMA
 // completion arrives on.  (Prefetching S(j+1) into a second register array was measured slower: spills.)
+// Split-fp16 variant (kSplit): Q hi and lo in shared memory (8 boxes, 128 KB; TMEM is full with two S/P buffers and
+// the 256-column O slice), a K stage holds 128 dims of this CTA's 64 entries of Kh and of Kl, a V stage this CTA's 128
+// value dims x 64 entries of Vt and of Vtl: two stages per tile each way, and two stages fit beside Q.
+struct PairSplitSmem {
+  static constexpr int NS = 2, NX = 2, kKeys = 128, kXyzBytes = kKeys * 16;
+  static constexpr int q = 0;                                   // 8 x [128 rows x 64 dims] SW128: Qh, then Ql
+  static constexpr int stages = q + 131072;
+  static constexpr int xyz = stages + NS * kStageBytes;
+  static constexpr int bars = xyz + NX * kXyzBytes;
+  static constexpr int b_q_full = 0;
+  static constexpr int b_stage_full = 1;
+  static constexpr int b_stage_empty = b_stage_full + NS;
+  static constexpr int b_s_full = b_stage_empty + NS;
+  static constexpr int b_p_full = b_s_full + 2;
+  static constexpr int b_xyz_full = b_p_full + 2;
+  static constexpr int b_xyz_empty = b_xyz_full + NX;
+  static constexpr int b_o_full = b_xyz_empty + NX;
+  static constexpr int b_q_pair = b_o_full + 1;
+  static constexpr int n_bars2 = b_q_pair + 1;
+  static constexpr int tmem_slot = bars + n_bars2 * 8;
+  static constexpr int total = tmem_slot + 16;
+  static constexpr int dynamic_bytes = total + 1024;
+};
+
 constexpr int kPairSoftmaxWarps = 16;
 constexpr int kPairThreads = (kPairSoftmaxWarps + 2) * 32;
 
-template <bool kGeo, bool kProf = false>
+// kSplit: S = Qh.Kh + Qh.Kl + Ql.Kh (SS mode), P' = P'h + P'l written over S as [16 hi | 16 lo] packed columns per
+// 32-entry group, O += P'h.Vh + P'h.Vl + P'l.Vh (TS mode)
+template <bool kGeo, bool kProf = false, bool kSplit = false>
 __global__ void __launch_bounds__(kPairThreads, 1)
 range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmK64,
-                        const __grid_constant__ CUtensorMap tmV128, const float4* __restrict__ db_xyz,
+                        const __grid_constant__ CUtensorMap tmV128, const __grid_constant__ CUtensorMap tmKl64,
+                        const __grid_constant__ CUtensorMap tmVl128, const float4* __restrict__ db_xyz,
                         const float4* __restrict__ rowc, int N, int M, int tiles_per_split, float a_sem,
                         float* __restrict__ out, size_t out_split_stride, int out_ld, int out_cols,
                         const uint32_t* __restrict__ geo_mask, int mask_words, long long* __restrict__ prof = nullptr) {
-  using L = PairSmem;
+  using L = std::conditional_t<kSplit, PairSplitSmem, PairSmem>;
   constexpr int NS = L::NS, NX = L::NX, kKeys = L::kKeys, kXyzBytes = L::kXyzBytes;
+  constexpr int kQBoxes = kSplit ? 8 : 4;
   long long prof_acc[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   const bool prof_on = kProf && prof != nullptr && blockIdx.x == 2 && blockIdx.y == 0 && blockIdx.z == 0;
   const long long prof_start = kProf ? clock64() : 0;
@@ -424,11 +499,46 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
       ptx::prefetch_tmap(&tmQ);
       ptx::prefetch_tmap(&tmK64);
       ptx::prefetch_tmap(&tmV128);
-      ptx::mbar_expect_tx(&bars[L::b_q_full], 65536);
-      for (int c = 0; c < 4; ++c) ptx::tma_load_2d(smem + L::q + c * 16384, &tmQ, &bars[L::b_q_full], c * 64, q0);
+      if (kSplit) {
+        ptx::prefetch_tmap(&tmKl64);
+        ptx::prefetch_tmap(&tmVl128);
+      }
+      ptx::mbar_expect_tx(&bars[L::b_q_full], kQBoxes * 16384);
+      for (int c = 0; c < kQBoxes; ++c) ptx::tma_load_2d(smem + L::q + c * 16384, &tmQ, &bars[L::b_q_full], c * 64, q0);
       PipeState st;
       for (int j = 0; j <= T; ++j) {
-        if (j < T) {
+        if (kSplit && j < T) {
+          const int key0 = (t_begin + j) * kKeys;
+#pragma unroll
+          for (int d2 = 0; d2 < 2; ++d2) {   // dims [128 d2, 128 d2 + 128) of this CTA's 64 entries: Kh, then Kl
+            ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
+            uint8_t* dst = smem + L::stages + st.idx * kStageBytes;
+            if (leader) ptx::mbar_expect_tx(&bars[L::b_stage_full + st.idx], 2 * kStageBytes);
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+              ptx::tma_load_2d_2sm(dst + c * 8192, &tmK64, &bars[L::b_stage_full + st.idx], (2 * d2 + c) * 64,
+                                   key0 + int(rank) * 64);
+              ptx::tma_load_2d_2sm(dst + 16384 + c * 8192, &tmKl64, &bars[L::b_stage_full + st.idx], (2 * d2 + c) * 64,
+                                   key0 + int(rank) * 64);
+            }
+            st.advance<NS>();
+          }
+        }
+        if (kSplit && j >= 1) {
+          const int key0 = (t_begin + j - 1) * kKeys;
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {      // entries [64 h, 64 h + 64) x this CTA's 128 value dims: Vt, then Vtl
+            ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
+            uint8_t* dst = smem + L::stages + st.idx * kStageBytes;
+            if (leader) ptx::mbar_expect_tx(&bars[L::b_stage_full + st.idx], 2 * kStageBytes);
+            ptx::tma_load_2d_2sm(dst, &tmV128, &bars[L::b_stage_full + st.idx], key0 + h * 64,
+                                 slice * kSliceV + int(rank) * 128);
+            ptx::tma_load_2d_2sm(dst + 16384, &tmVl128, &bars[L::b_stage_full + st.idx], key0 + h * 64,
+                                 slice * kSliceV + int(rank) * 128);
+            st.advance<NS>();
+          }
+        }
+        if (!kSplit && j < T) {
           const int key0 = (t_begin + j) * kKeys;
           PROF_T0();
           ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
@@ -440,7 +550,7 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
             ptx::tma_load_2d_2sm(dst + c * 8192, &tmK64, &bars[L::b_stage_full + st.idx], c * 64, key0 + int(rank) * 64);
           st.advance<NS>();
         }
-        if (j >= 1) {
+        if (!kSplit && j >= 1) {
           const int key0 = (t_begin + j - 1) * kKeys;
           PROF_T0();
           ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
@@ -483,7 +593,59 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
       ptx::mbar_wait_cluster(&bars[L::b_q_pair], 0);
       PipeState st;
       for (int j = 0; j <= T; ++j) {
-        if (j < T) {
+        if (kSplit && j < T) {
+          const uint32_t tmem_s = tmem_base + (j & 1) * kKeys;
+          const uint32_t a_base = smem_u + L::q;
+#pragma unroll
+          for (int d2 = 0; d2 < 2; ++d2) {
+            ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
+            ptx::tc_fence_after();
+            if (ptx::elect_one()) {
+              const uint32_t b_base = smem_u + L::stages + st.idx * kStageBytes;
+#pragma unroll
+              for (int c = 0; c < 2; ++c)
+#pragma unroll
+                for (int kk = 0; kk < 4; ++kk) {
+                  const uint32_t qa = a_base + (2 * d2 + c) * 16384 + kk * 32, kb = b_base + c * 8192 + kk * 32;
+                  const uint64_t qh = ptx::umma_desc_kmajor_sw128(qa), ql = ptx::umma_desc_kmajor_sw128(qa + 65536);
+                  const uint64_t kh = ptx::umma_desc_kmajor_sw128(kb), kl = ptx::umma_desc_kmajor_sw128(kb + 16384);
+                  ptx::umma_f16_ss_2sm(tmem_s, qh, kh, idesc_qk, (d2 | c | kk) != 0);
+                  ptx::umma_f16_ss_2sm(tmem_s, qh, kl, idesc_qk, 1);
+                  ptx::umma_f16_ss_2sm(tmem_s, ql, kh, idesc_qk, 1);
+                }
+              ptx::umma_commit_2sm_u32(bars_u + 8 * (L::b_stage_empty + st.idx));
+              if (d2 == 1) ptx::umma_commit_2sm_u32(bars_u + 8 * (L::b_s_full + (j & 1)));
+            }
+            __syncwarp();
+            st.advance<NS>();
+          }
+        }
+        if (kSplit && j >= 1) {
+          const int jj = j - 1, b = jj & 1;
+          ptx::mbar_wait_cluster(&bars[L::b_p_full + b], (jj >> 1) & 1);
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
+            ptx::tc_fence_after();
+            if (ptx::elect_one()) {
+              const uint32_t b_base = smem_u + L::stages + st.idx * kStageBytes;
+#pragma unroll
+              for (int kk = 0; kk < 4; ++kk) {
+                // P'(jj), 32-entry group g: 16 hi columns at S-buffer column 32 g, the 16 lo columns after them
+                const uint32_t ph = tmem_base + b * kKeys + (2 * h + (kk >> 1)) * 32 + (kk & 1) * 8;
+                const uint64_t vh = ptx::umma_desc_kmajor_sw128(b_base + kk * 32);
+                const uint64_t vl = ptx::umma_desc_kmajor_sw128(b_base + 16384 + kk * 32);
+                ptx::umma_f16_ts_2sm(tmem_o, ph, vh, idesc_pv, (jj > 0) || (h | kk) != 0);
+                ptx::umma_f16_ts_2sm(tmem_o, ph, vl, idesc_pv, 1);
+                ptx::umma_f16_ts_2sm(tmem_o, ph + 16, vh, idesc_pv, 1);
+              }
+              ptx::umma_commit_2sm_u32(bars_u + 8 * (L::b_stage_empty + st.idx));
+            }
+            __syncwarp();
+            st.advance<NS>();
+          }
+        }
+        if (!kSplit && j < T) {
           const uint32_t tmem_s = tmem_base + (j & 1) * kKeys;
           PROF_T0();
           ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
@@ -505,7 +667,7 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
           PROF_ADD(1, 1);
           st.advance<NS>();
         }
-        if (j >= 1) {
+        if (!kSplit && j >= 1) {
           const int jj = j - 1, b = jj & 1;
           PROF_T0();
           ptx::mbar_wait_cluster(&bars[L::b_p_full + b], (jj >> 1) & 1);
@@ -562,7 +724,7 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
       const uint32_t kxyz = ptx::smem_u32(smem + L::xyz + b * kXyzBytes) + grp * 32 * 16;
       const int nvalid = M - key0;            // >= 32 except in the last tile
       const bool with_geo = kGeo && !skip_geo(t_begin + j);
-      uint32_t packed[16];
+      uint32_t packed[kSplit ? 32 : 16];
       // the geo part is selected per TILE (warp-uniform): separate straight-line bodies
       auto body = [&](auto masked, auto geo) {
         constexpr bool kM = decltype(masked)::value, kG = decltype(geo)::value;
@@ -580,7 +742,15 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
             if (kM && i >= nvalid) p = 0.f;
             pv[u] = p;
           }
-          packed[w] = ptx::pack_half2(pv[0], pv[1]);
+          if constexpr (kSplit) {      // p = hi + lo: hi = rn_f16(p), lo = rn_f16(p - hi) (the subtraction is exact)
+            const __half2 hi = __floats2half2_rn(pv[0], pv[1]);
+            const float2 hf = __half22float2(hi);
+            const __half2 lo = __floats2half2_rn(pv[0] - hf.x, pv[1] - hf.y);
+            packed[w] = *reinterpret_cast<const uint32_t*>(&hi);
+            packed[16 + w] = *reinterpret_cast<const uint32_t*>(&lo);
+          } else {
+            packed[w] = ptx::pack_half2(pv[0], pv[1]);
+          }
         }
       };
       if (nvalid >= 32) {
@@ -589,8 +759,10 @@ range_apply_pair_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_co
         if (with_geo) body(std::true_type{}, std::true_type{}); else body(std::true_type{}, std::false_type{});
       }
       PROF_ADD(2, 3);
-      // P'(row, 32 entries) as 16 packed columns over the first half of the 32 S columns it came from
-      ptx::tmem_st16(taddr, packed);
+      // P'(row, 32 entries) as 16 packed columns over the first half of the 32 S columns it came from (split: the lo
+      // parts over the second half)
+      if constexpr (kSplit) ptx::tmem_st32(taddr, packed);
+      else ptx::tmem_st16(taddr, packed);
       ptx::tmem_st_wait();
       ptx::tc_fence_before();
       __syncwarp();
@@ -783,6 +955,17 @@ __global__ void reduce_out1_kernel(const float* __restrict__ part, size_t split_
   out[i] = a;
 }
 
+// q64 (N,256) -> (N,512) fp16 rows [hi | lo]; hi is normalize_kernel's __double2half, bit for bit
+__global__ void split_queries_kernel(const double* __restrict__ q64, int N, __half* __restrict__ q16x2) {
+  const size_t i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= size_t(N) * 256) return;
+  __half hi, lo;
+  rangeb200::split_f16(q64[i], hi, lo);
+  const size_t n = i / 256, d = i % 256;
+  q16x2[n * 512 + d] = hi;
+  q16x2[n * 512 + 256 + d] = lo;
+}
+
 template <class K>
 cudaError_t set_smem(K kernel, int bytes) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
@@ -798,21 +981,27 @@ void set_profile_buffer(long long* p) { g_prof_buffer = p; }
 int retrieval_stats_smem_bytes() { return StatsSmem::dynamic_bytes; }
 int retrieval_apply_smem_bytes() { return PairSmem::dynamic_bytes; }
 
-cudaError_t launch_stats(const RetrievalArgs& a, float* part_sum, float* part_max, cudaStream_t stream) {
-  const int bytes = retrieval_stats_smem_bytes();
+template <bool kSplit>
+cudaError_t launch_stats_variant(const RetrievalArgs& a, float* part_sum, float* part_max, cudaStream_t stream) {
+  const int bytes = StatsSmem::dynamic_bytes;
   cudaError_t e;
-  if ((e = set_smem(range_stats_kernel<true>, bytes)) != cudaSuccess) return e;
-  if ((e = set_smem(range_stats_kernel<false>, bytes)) != cudaSuccess) return e;
+  if ((e = set_smem(range_stats_kernel<true, kSplit>, bytes)) != cudaSuccess) return e;
+  if ((e = set_smem(range_stats_kernel<false, kSplit>, bytes)) != cudaSuccess) return e;
   dim3 grid((a.N + kBlockQ - 1) / kBlockQ, a.stats_splits, 1);
   if (a.geo)
-    range_stats_kernel<true><<<grid, kStatsThreads, bytes, stream>>>(a.tmK128, a.q16, a.db_xyz, a.q_xyz, a.N, a.M,
-                                                               a.stats_tiles_per_split, a.a_sem, a.a_geo, part_sum,
-                                                               part_max, a.geo_mask, a.mask_words);
+    range_stats_kernel<true, kSplit><<<grid, kStatsThreads, bytes, stream>>>(
+        a.tmK128, a.tmKl128, a.q16, a.db_xyz, a.q_xyz, a.N, a.M, a.stats_tiles_per_split, a.a_sem, a.a_geo, part_sum,
+        part_max, a.geo_mask, a.mask_words);
   else
-    range_stats_kernel<false><<<grid, kStatsThreads, bytes, stream>>>(a.tmK128, a.q16, a.db_xyz, a.q_xyz, a.N, a.M,
-                                                                a.stats_tiles_per_split, a.a_sem, a.a_geo, part_sum,
-                                                                part_max, nullptr, 0);
+    range_stats_kernel<false, kSplit><<<grid, kStatsThreads, bytes, stream>>>(
+        a.tmK128, a.tmKl128, a.q16, a.db_xyz, a.q_xyz, a.N, a.M, a.stats_tiles_per_split, a.a_sem, a.a_geo, part_sum,
+        part_max, nullptr, 0);
   return cudaGetLastError();
+}
+
+cudaError_t launch_stats(const RetrievalArgs& a, float* part_sum, float* part_max, cudaStream_t stream) {
+  return a.split ? launch_stats_variant<true>(a, part_sum, part_max, stream)
+                 : launch_stats_variant<false>(a, part_sum, part_max, stream);
 }
 
 cudaError_t launch_geo_mask(const float* q_xyz, int N, int rows, const float* caps, int n_tiles, int M, float delta,
@@ -876,21 +1065,39 @@ cudaError_t launch_apply(const RetrievalArgs& a, const float* rowc, float* out, 
   // CTA pairs: cluster (2,1,1) over the query-tile axis (an odd tile count gets one all-padding CTA)
   const int bytes = PairSmem::dynamic_bytes;
   dim3 grid((qtiles + 1) / 2 * 2, (dim_v + kSliceV - 1) / kSliceV, a.apply_splits);
+  if (a.split) {         // split-fp16 operands (its own shared-memory plan)
+    const int sbytes = PairSplitSmem::dynamic_bytes;
+    if ((e = set_smem(range_apply_pair_kernel<true, false, true>, sbytes)) != cudaSuccess) return e;
+    if ((e = set_smem(range_apply_pair_kernel<false, false, true>, sbytes)) != cudaSuccess) return e;
+    if (a.geo)
+      return launch_pair(range_apply_pair_kernel<true, false, true>, grid, sbytes, stream, a.tmQ, a.tmK64, a.tmV128,
+                         a.tmKl64, a.tmVl128, a.db_xyz, rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out,
+                         out_split_stride, out_ld, dim_v, a.geo_mask, a.mask_words, no_prof);
+    return launch_pair(range_apply_pair_kernel<false, false, true>, grid, sbytes, stream, a.tmQ, a.tmK64, a.tmV128,
+                       a.tmKl64, a.tmVl128, a.db_xyz, rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out,
+                       out_split_stride, out_ld, dim_v, no_mask, 0, no_prof);
+  }
   if (g_prof_buffer) {   // instrumented build of the same kernel (tools/time_apply.py)
     if ((e = set_smem(range_apply_pair_kernel<true, true>, bytes)) != cudaSuccess) return e;
-    return launch_pair(range_apply_pair_kernel<true, true>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.db_xyz,
-                       rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v, a.geo_mask,
-                       a.mask_words, g_prof_buffer);
+    return launch_pair(range_apply_pair_kernel<true, true>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.tmK64,
+                       a.tmV128, a.db_xyz, rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld,
+                       dim_v, a.geo_mask, a.mask_words, g_prof_buffer);
   }
   if ((e = set_smem(range_apply_pair_kernel<true>, bytes)) != cudaSuccess) return e;
   if ((e = set_smem(range_apply_pair_kernel<false>, bytes)) != cudaSuccess) return e;
   if (a.geo)
-    return launch_pair(range_apply_pair_kernel<true>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.db_xyz, rc,
-                       a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v, a.geo_mask,
-                       a.mask_words, no_prof);
-  return launch_pair(range_apply_pair_kernel<false>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.db_xyz, rc,
-                     a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v, no_mask, 0,
-                     no_prof);
+    return launch_pair(range_apply_pair_kernel<true>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.tmK64, a.tmV128,
+                       a.db_xyz, rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v,
+                       a.geo_mask, a.mask_words, no_prof);
+  return launch_pair(range_apply_pair_kernel<false>, grid, bytes, stream, a.tmQ, a.tmK64, a.tmV128, a.tmK64, a.tmV128,
+                     a.db_xyz, rc, a.N, a.M, a.apply_tiles_per_split, a.a_sem, out, out_split_stride, out_ld, dim_v,
+                     no_mask, 0, no_prof);
+}
+
+cudaError_t launch_split_queries(const double* q64, int N, void* q16x2, cudaStream_t stream) {
+  const size_t total = size_t(N) * 256;
+  split_queries_kernel<<<unsigned((total + 255) / 256), 256, 0, stream>>>(q64, N, reinterpret_cast<__half*>(q16x2));
+  return cudaGetLastError();
 }
 
 cudaError_t launch_reduce_out(const float* part, size_t split_stride, int splits, size_t total, float* out,

@@ -37,6 +37,7 @@ constexpr int kTopkThreads = (kTopkWarps + 2) * 32;
 constexpr int kKeyRow = 36;         // floats per thread in the pass-on buffer (32 keys, 16-byte aligned rows)
 constexpr uint32_t kTmemQ = 0;      // TMEM columns: [0,128) Q | [128,256) S buf 0 | [256,384) S buf 1
 constexpr uint32_t kTmemS = 128;
+constexpr uint32_t kTmemQl = 384;   // split-fp16 variant: Ql after the two S buffers
 
 struct TopkSmem {
   static constexpr int NS = 5, kXyzBytes = kKeys * 16;
@@ -68,9 +69,11 @@ struct PipeState {
 };
 
 // part_w / part_idx: [2 * splits][N][k], part = 2 * split + half; unfilled slots have entry -1
-template <bool kGeo, int K>
+// kSplit: split-fp16 operands as in range_stats_kernel<kGeo, true> (Ql in TMEM, four Kh + Kl stages per tile)
+template <bool kGeo, int K, bool kSplit = false>
 __global__ void __launch_bounds__(kTopkThreads, 1)
-range_topk_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __restrict__ q16,
+range_topk_kernel(const __grid_constant__ CUtensorMap tmK, const __grid_constant__ CUtensorMap tmKl,
+                  const __half* __restrict__ q16,
                   const float4* __restrict__ db_xyz, const float4* __restrict__ q_xyz, const float2* __restrict__ sums,
                   int N, int M, int tiles_per_split, float a_sem, float a_geo, float beta, int k,
                   const uint32_t* __restrict__ geo_mask, int mask_words, float* __restrict__ part_w,
@@ -113,8 +116,15 @@ range_topk_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __restr
   const uint32_t smem_u = __shfl_sync(0xffffffffu, ptx::smem_u32(smem), 0);
   const uint32_t bars_u = smem_u + L::bars;
   if (warp < kTopkWarps) {        // the 16-warp Q loader, two column groups per warp
-    ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane);
-    ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp + kTopkWarps, lane);
+    if constexpr (kSplit) {
+      ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane, 512);
+      ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp + kTopkWarps, lane, 512);
+      ptx::load_q_to_tmem16(q16 + 256, q0, N, tmem_base + kTmemQl, warp, lane, 512);
+      ptx::load_q_to_tmem16(q16 + 256, q0, N, tmem_base + kTmemQl, warp + kTopkWarps, lane, 512);
+    } else {
+      ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp, lane);
+      ptx::load_q_to_tmem16(q16, q0, N, tmem_base + kTmemQ, warp + kTopkWarps, lane);
+    }
   }
   ptx::tc_fence_before();
   __syncthreads();
@@ -124,9 +134,21 @@ range_topk_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __restr
     // ===== TMA producer =====
     if (lane == 0) {
       ptx::prefetch_tmap(&tmK);
+      if (kSplit) ptx::prefetch_tmap(&tmKl);
       PipeState st;
       for (int j = 0; j < T; ++j) {
         const int key0 = (t_begin + j) * kKeys;
+        if constexpr (kSplit) {
+#pragma unroll
+          for (int d = 0; d < 4; ++d) {     // dims [64 d, 64 d + 64): Kh box, then the Kl box
+            ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
+            uint8_t* dst = smem + L::stages + st.idx * kStageBytes;
+            ptx::mbar_expect_tx(&bars[L::b_stage_full + st.idx], kStageBytes);
+            ptx::tma_load_2d(dst, &tmK, &bars[L::b_stage_full + st.idx], d * 64, key0);
+            ptx::tma_load_2d(dst + 16384, &tmKl, &bars[L::b_stage_full + st.idx], d * 64, key0);
+            st.advance<NS>();
+          }
+        } else
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
           ptx::mbar_wait(&bars[L::b_stage_empty + st.idx], st.phase ^ 1);
@@ -155,6 +177,29 @@ range_topk_kernel(const __grid_constant__ CUtensorMap tmK, const __half* __restr
       const int b = j & 1;
       ptx::mbar_wait(&bars[L::b_s_empty + b], ((j >> 1) & 1) ^ 1);
       ptx::tc_fence_after();
+      if constexpr (kSplit) {
+#pragma unroll
+        for (int d = 0; d < 4; ++d) {
+          ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
+          ptx::tc_fence_after();
+          if (ptx::elect_one()) {
+            const uint32_t b_base = smem_u + L::stages + st.idx * kStageBytes;
+            const uint32_t s_col = tmem_base + kTmemS + b * kKeys;
+#pragma unroll
+            for (int kk = 0; kk < 4; ++kk) {
+              const uint32_t qc = d * 32 + kk * 8;
+              const uint64_t kh = ptx::umma_desc_kmajor_sw128(b_base + kk * 32);
+              const uint64_t kl = ptx::umma_desc_kmajor_sw128(b_base + 16384 + kk * 32);
+              ptx::umma_f16_ts(s_col, tmem_base + kTmemQ + qc, kh, idesc, (d | kk) != 0);
+              ptx::umma_f16_ts(s_col, tmem_base + kTmemQ + qc, kl, idesc, 1);
+              ptx::umma_f16_ts(s_col, tmem_base + kTmemQl + qc, kh, idesc, 1);
+            }
+            ptx::umma_commit_u32(bars_u + 8 * (L::b_stage_empty + st.idx));
+          }
+          __syncwarp();
+          st.advance<NS>();
+        }
+      } else
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         ptx::mbar_wait(&bars[L::b_stage_full + st.idx], st.phase);
@@ -366,7 +411,7 @@ cudaError_t launch_one(Kern kern, dim3 grid, const rangeb200::RetrievalArgs& a, 
   const int bytes = TopkSmem::dynamic_bytes;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
   if (e != cudaSuccess) return e;
-  kern<<<grid, kTopkThreads, bytes, s>>>(a.tmK128, a.q16, a.db_xyz, a.q_xyz, reinterpret_cast<const float2*>(sums),
+  kern<<<grid, kTopkThreads, bytes, s>>>(a.tmK128, a.tmKl128, a.q16, a.db_xyz, a.q_xyz, reinterpret_cast<const float2*>(sums),
                                          a.N, a.M, tiles_per_split, a.a_sem, a.a_geo, beta, k, a.geo_mask, a.mask_words,
                                          part_w, part_idx);
   return cudaGetLastError();
@@ -375,6 +420,11 @@ cudaError_t launch_one(Kern kern, dim3 grid, const rangeb200::RetrievalArgs& a, 
 template <int K>
 cudaError_t launch_bucket(dim3 grid, const rangeb200::RetrievalArgs& a, int tiles_per_split, const float* sums,
                           float beta, int k, float* part_w, int32_t* part_idx, cudaStream_t s) {
+  if (a.split) {
+    if (a.geo)
+      return launch_one(range_topk_kernel<true, K, true>, grid, a, tiles_per_split, sums, beta, k, part_w, part_idx, s);
+    return launch_one(range_topk_kernel<false, K, true>, grid, a, tiles_per_split, sums, beta, k, part_w, part_idx, s);
+  }
   if (a.geo) return launch_one(range_topk_kernel<true, K>, grid, a, tiles_per_split, sums, beta, k, part_w, part_idx, s);
   return launch_one(range_topk_kernel<false, K>, grid, a, tiles_per_split, sums, beta, k, part_w, part_idx, s);
 }

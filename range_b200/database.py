@@ -10,6 +10,12 @@ Device layout (what include/range_b200.h:range_ctx_set_db takes):
   xyz (Mpad, 4)    fp32  unit vectors of the entry locations (x, y, z, 0)
   caps (Mpad/128, 4) fp32 bounding cap of every 128-entry tile: (unit centre, angular radius [rad])
 Mpad = M rounded up to 128; padding is zero and masked in-kernel.
+Split-fp16 retrieval (retrieval_precision='f16x3', include/range_b200.h: range_ctx_set_db_lo) adds the lo halves of the
+same fp32 arrays Kh and Vt are rounded from - twice the device memory of the keys and values:
+  Kl  (Mpad, 256)  fp16  rn_f16(K - Kh)
+  Vtl (Dp, Mpad)   fp16  rn_f16(vscale V - Vt)
+The lo halves share the hi halves' scale (Kh and Vt stay what the fp16 path reads): every product of the split kernels
+accumulates into one fp32 accumulator, so hi.hi, hi.lo and lo.hi must all carry the same power of two.
 
 Row order: the reference's results do not depend on the order of the database rows (softmax-weighted sums,
 range/range.py:213-238), so the rows are stored sorted along a cube-map Hilbert curve.  Consecutive 128-entry
@@ -152,10 +158,12 @@ def tile_caps(xyz, block=BLOCK):
 class DeviceDatabase:
     STAGING_ROWS = 1 << 18          # rows converted / uploaded at a time (1.3 GB of fp32 staging)
 
-    def __init__(self, db, device, shard=None, spatial_sort=True):
+    def __init__(self, db, device, shard=None, spatial_sort=True, lo=False):
         """db: mapping with locs / satclip_embeddings / image_embeddings (an opened .npz works).
         shard=(rank, world): keep rows [rank*M/world, (rank+1)*M/world) of the (sorted) database only (M-sharding).
-        spatial_sort: store the rows along a Hilbert curve and build the tile caps (geo-term skipping)."""
+        spatial_sort: store the rows along a Hilbert curve and build the tile caps (geo-term skipping).
+        lo: also keep the lo halves Kl / Vtl for split-fp16 retrieval (None otherwise)."""
+        with_lo = lo
         # keys and values stay what they are (ndarrays, or memory maps from open_npz): range.py:85-90's .astype(float32)
         # and row normalisation are applied block by block on the way to the device, in the reference's arithmetic
         locs = np.asarray(db["locs"]).astype(np.float32)                                  # range.py:79
@@ -188,6 +196,7 @@ class DeviceDatabase:
         self.vscale = 1.0 if vmax == 0.0 or not math.isfinite(vmax) else 2.0 ** math.floor(math.log2(256.0 / vmax))
         self.Kh = torch.zeros(Mpad, 256, dtype=torch.float16, device=dev)
         self.Vt = torch.zeros(padded_value_dim(D), Mpad, dtype=torch.float16, device=dev)
+        self._alloc_lo(with_lo)
         step = self.STAGING_ROWS
         for b0 in range(0, M, step):                       # bounded staging memory for 10M-entry databases
             b1 = min(M, b0 + step)
@@ -196,12 +205,33 @@ class DeviceDatabase:
             back = np.searchsorted(idx, want)              # ... then permute into layout order
             k = np.asarray(Kraw[idx]).astype(np.float32)                                  # range.py:85
             k = (k / np.linalg.norm(k, ord=2, axis=1, keepdims=True))[back]               # range.py:89
-            self.Kh[b0:b1] = torch.from_numpy(np.ascontiguousarray(k)).to(dev).half()
             v = np.asarray(V[idx]).astype(np.float32)[back]                               # range.py:90
-            self.Vt[:D, b0:b1] = (torch.from_numpy(np.ascontiguousarray(v)).to(dev) * self.vscale).half().t()
+            self._store_rows(b0, torch.from_numpy(np.ascontiguousarray(k)).to(dev),
+                             torch.from_numpy(np.ascontiguousarray(v)).to(dev) * self.vscale)
         self.xyz = torch.zeros(Mpad, 4, dtype=torch.float32, device=dev)
         self.xyz[:M, :3] = torch.from_numpy(np.ascontiguousarray(xyz)).to(dev)
         self.caps = torch.from_numpy(tile_caps(xyz)).to(dev) if self.order is not None else None
+
+    def _alloc_lo(self, lo):
+        if lo:
+            self.Kl = torch.zeros_like(self.Kh)
+            self.Vtl = torch.zeros_like(self.Vt)
+        else:
+            self.Kl = self.Vtl = None
+
+    def _store_rows(self, b0, k, vs):
+        """rows b0.. of the layout from fp32 device blocks: k (rows, 256) normalised keys, vs (rows, D) = vscale V"""
+        b1, D = b0 + k.shape[0], vs.shape[1]
+        kh, vh = k.half(), vs.half()
+        self.Kh[b0:b1] = kh
+        self.Vt[:D, b0:b1] = vh.t()
+        if self.Kl is not None:                # x - rn_f16(x) is exact in fp32
+            self.Kl[b0:b1] = (k - kh.float()).half()
+            self.Vtl[:D, b0:b1] = (vs - vh.float()).half().t()
+
+    @property
+    def has_lo(self):
+        return getattr(self, "Kl", None) is not None
 
     # ---- device-resident format on disk (SURVEY.md section 8f-1): skips normalisation / sorting / transposition at start-up
     CACHE_VERSION = 2
@@ -237,6 +267,7 @@ class DeviceDatabase:
                          row_range=np.asarray(self.row_range), vscale=self.vscale, shard=np.asarray(shard),
                          fingerprint=np.asarray(fingerprint),
                          Kh=self.Kh.cpu().numpy(), Vt=self.Vt.cpu().numpy(), xyz=self.xyz.cpu().numpy(),
+                         **({"Kl": self.Kl.cpu().numpy(), "Vtl": self.Vtl.cpu().numpy()} if self.has_lo else {}),
                          caps=np.zeros((0, 4), np.float32) if self.caps is None else self.caps.cpu().numpy(),
                          order=np.zeros(0, np.int64) if self.order is None else self.order)
             os.replace(tmp, path)
@@ -246,10 +277,12 @@ class DeviceDatabase:
         return path
 
     @classmethod
-    def from_cache(cls, path, device, shard=None, fingerprint=None, spatial_sort=None, value_dim=None):
+    def from_cache(cls, path, device, shard=None, fingerprint=None, spatial_sort=None, value_dim=None, lo=False):
         """load a cache written by save_cache.  Returns None (the caller rebuilds) when the file is missing or was built
         for another shard, another source (fingerprint, when given), another row order or another value width
-        (value_dim, when given; caches without the field hold 1024-wide values); raises on a malformed file."""
+        (value_dim, when given; caches without the field hold 1024-wide values), or - lo=True, split-fp16 retrieval -
+        holds no lo halves; raises on a malformed file.  lo=False does not load lo halves the file may hold."""
+        need_lo = lo
         path = cls.cache_path(path, shard)
         if not os.path.exists(path):
             return None
@@ -265,6 +298,8 @@ class DeviceDatabase:
             return None
         D = int(z["value_dim"]) if "value_dim" in z else 1024
         if value_dim is not None and D != int(value_dim):
+            return None
+        if need_lo and not ("Kl" in z and "Vtl" in z):
             return None
         self = cls.__new__(cls)
         dev = torch.device(device)
@@ -282,20 +317,25 @@ class DeviceDatabase:
         self.xyz = torch.from_numpy(z["xyz"]).to(dev)
         self.caps = torch.from_numpy(z["caps"]).to(dev) if z["caps"].shape[0] else None
         self.order = z["order"] if z["order"].shape[0] else None
+        self.Kl = torch.from_numpy(z["Kl"]).to(dev) if need_lo else None
+        self.Vtl = torch.from_numpy(z["Vtl"]).to(dev) if need_lo else None
         if self.Kh.shape != (self.Mpad, 256) or self.Vt.shape != (padded_value_dim(D), self.Mpad) \
                 or self.Kh.dtype != torch.float16 or not 1 <= D <= MAX_VALUE_DIM \
-                or self.M != self.row_range[1] - self.row_range[0]:
+                or self.M != self.row_range[1] - self.row_range[0] \
+                or (need_lo and (self.Kl.shape != self.Kh.shape or self.Vtl.shape != self.Vt.shape
+                            or self.Kl.dtype != torch.float16 or self.Vtl.dtype != torch.float16)):
             raise ValueError(f"{path}: malformed database cache")
         return self
 
     @classmethod
-    def synthetic(cls, M, device, seed=0, shard=None, value_dim=1024):
+    def synthetic(cls, M, device, seed=0, shard=None, value_dim=1024, lo=False):
         """Benchmark-only: an iid synthetic database (area-uniform locations, N(0,1) keys and values - the worst case
         for the fp16 operands, SURVEY.md 8d) generated block by block straight into the device layout, so 10 M-entry
         databases (25.7 GB in fp16) do not need their 51 GB of fp32 source arrays on the host.
         shard=(rank, world): rows [rank*M/world, (rank+1)*M/world) of the spatially sorted database only - every rank
         draws the same M locations (same seed) and sorts them the same way, keys / values are iid per entry.
-        value_dim: width D of the values (timing other feature widths)."""
+        value_dim: width D of the values (timing other feature widths); lo: keep the lo halves (split-fp16 retrieval)."""
+        with_lo = lo
         self = cls.__new__(cls)
         dev = torch.device(device)
         rng = np.random.default_rng(seed)
@@ -317,14 +357,14 @@ class DeviceDatabase:
         self.vscale = 2.0 ** math.floor(math.log2(256.0 / 6.0))                      # |N(0,1)| < 6
         self.Kh = torch.zeros(self.Mpad, 256, dtype=torch.float16, device=dev)
         self.Vt = torch.zeros(padded_value_dim(D), self.Mpad, dtype=torch.float16, device=dev)
+        self._alloc_lo(with_lo)
         g = torch.Generator(device=dev).manual_seed(seed if shard is None else seed * 1000003 + 1 + int(shard[0]))
         step = 1 << 18
         for b0 in range(0, m, step):
             b1 = min(m, b0 + step)
             k = torch.randn(b1 - b0, 256, device=dev, generator=g)
-            self.Kh[b0:b1] = (k / k.norm(dim=1, keepdim=True)).half()                 # range.py:89
             v = torch.randn(b1 - b0, D, device=dev, generator=g).clamp_(-6.0, 6.0)
-            self.Vt[:D, b0:b1] = (v * self.vscale).half().t()
+            self._store_rows(b0, k / k.norm(dim=1, keepdim=True), v * self.vscale)     # range.py:89
         self.xyz = torch.zeros(self.Mpad, 4, dtype=torch.float32, device=dev)
         self.xyz[:m, :3] = torch.from_numpy(np.ascontiguousarray(xyz)).to(dev)
         self.caps = torch.from_numpy(tile_caps(xyz)).to(dev)
@@ -350,4 +390,5 @@ class DeviceDatabase:
         return cached[rows]
 
     def nbytes(self):
-        return sum(t.numel() * t.element_size() for t in (self.Kh, self.Vt, self.xyz))
+        lo = (self.Kl, self.Vtl) if self.has_lo else ()
+        return sum(t.numel() * t.element_size() for t in (self.Kh, self.Vt, self.xyz) + lo)

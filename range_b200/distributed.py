@@ -8,7 +8,8 @@ partial softmax state.  Every logit is bounded (|s|,|g| <= 1), so the kernels us
 running max and the merge needs no rescaling:
 
     every rank          sorts + encodes ITS OWN queries (a slab of `slab` rows per step)
-    all_gather          the compact queries: fp16 embedding (512 B) + unit vector (16 B) per query
+    all_gather          the compact queries: fp16 embedding (512 B; 1 024 B of [hi | lo] rows with split-fp16 retrieval)
+                        + unit vector (16 B) per query
     every rank          row statistics of all P * slab queries over its shard       (range_retrieve_stats)
     all_reduce(SUM)     the exp-sums, 8 B per query; the maxima stay local (they only scale the fp16 weights)
     every rank          apply pass over its shard with the global sums; row n of the partial result is stored
@@ -189,7 +190,7 @@ class ShardedRetriever:
         eng, P = self.engine, self.world
         dev = eng.device
         n = coords.shape[0]
-        q16_all = torch.empty(P * slab, 256, dtype=torch.float16, device=dev)
+        q16_all = torch.empty(P * slab, getattr(eng, "q_cols", 256), dtype=torch.float16, device=dev)
         qxyz_all = torch.empty(P * slab, 4, dtype=torch.float32, device=dev)
         for lo in range(0, n_max, slab):
             mine = coords[lo:min(n, lo + slab)] if lo < n else coords[:0]

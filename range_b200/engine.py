@@ -12,6 +12,15 @@ from . import _lib
 from .sh_table import build_table, closed_form_norms
 
 MODE = {"RANGE": _lib.RANGE_MODE_RANGE, "RANGE+": _lib.RANGE_MODE_RANGE_PLUS}
+RETRIEVAL_PRECISIONS = ("fp16", "f16x3")
+
+
+def check_retrieval_precision(p):
+    """'fp16' (the default: fp16 q, K, P' and V) or 'f16x3' (split fp16, hi + lo, three products per term); ValueError
+    otherwise"""
+    if p not in RETRIEVAL_PRECISIONS:
+        raise ValueError(f"retrieval_precision={p!r}: expected 'fp16' or 'f16x3'")
+    return p
 
 
 def _ptr(t):
@@ -50,11 +59,17 @@ def _new_out(N, dtype, device, D=1024):
 
 
 class RangeEngine:
-    def __init__(self, device, encoder=None, database=None, L=None, encoder_precision="auto", harmonics=None):
+    def __init__(self, device, encoder=None, database=None, L=None, encoder_precision="auto", harmonics=None,
+                 retrieval_precision="fp16"):
         """encoder: dict from checkpoint.load_satclip_location_encoder (or None: SH only with `L`);
         database: database.DeviceDatabase or None;
         encoder_precision: 'fp64' (the reference's arithmetic, DMMA), 'f16x3' (tensor cores, split fp16 operands,
-        fp32-class accuracy; 'tf32x3' is accepted as an alias) or 'auto' (= f16x3 when the layer widths allow it, else fp64)."""
+        fp32-class accuracy; 'tf32x3' is accepted as an alias) or 'auto' (= f16x3 when the layer widths allow it, else fp64);
+        retrieval_precision: 'fp16' (fp16 operands of Q.K^T and P'.V) or 'f16x3' (every operand split into hi + lo fp16,
+        three products per term: about 3x the tensor work; the database must carry its lo halves, DeviceDatabase(lo=True)).
+        In 'f16x3' encode() / encode_raster() return q16 as the (N, 512) rows [hi | lo] the retrieval entry points take."""
+        self.retrieval_precision = check_retrieval_precision(retrieval_precision)
+        self.q_cols = 512 if retrieval_precision == "f16x3" else 256
         self.encoder_precision = encoder_precision
         self.device = torch.device(device)
         if self.device.type != "cuda":
@@ -138,6 +153,11 @@ class RangeEngine:
                                                     float(db.vscale)))
         if getattr(db, "caps", None) is not None:
             _lib.check(self.lib.range_ctx_set_db_caps(self.ctx, db.caps.shape[0], _ptr(db.caps), db.M_total))
+        if self.retrieval_precision == "f16x3":
+            if getattr(db, "Kl", None) is None:
+                raise ValueError("retrieval_precision='f16x3' needs a database with its lo halves (DeviceDatabase(lo=True))")
+            _lib.check(self.lib.range_ctx_set_db_lo(self.ctx, _ptr(db.Kl), _ptr(db.Vtl)))
+            _lib.check(self.lib.range_ctx_set_retrieval_precision(self.ctx, _lib.RANGE_RET_F16X3))
         self.db = db
         self.value_dim = D
 
@@ -196,7 +216,26 @@ class RangeEngine:
             ws = self._workspace("enc", nbytes)
             _lib.check(self.lib.range_encode(self.ctx, N, _ptr(lonlat), _ptr(q64), _ptr(q16), _ptr(qxyz), _ptr(ws),
                                              ws.numel(), _stream()))
-        return q64, q16, qxyz
+        return q64, self.query_rows(q64, q16), qxyz
+
+    def split_queries(self, q64):
+        """(N,256) fp64 -> (N,512) fp16 rows [rn_f16(q) | rn_f16(q - rn_f16(q))] (range_split_queries)"""
+        N = q64.shape[0]
+        out = torch.empty(N, 512, dtype=torch.float16, device=self.device)
+        if N:
+            with torch.cuda.device(self.index):
+                _lib.check(self.lib.range_split_queries(self.ctx, N, _ptr(q64), _ptr(out), _stream()))
+        return out
+
+    def query_rows(self, q64, q16):
+        """the query rows of the retrieval entry points: q16 (N,256), or in 'f16x3' the (N,512) [hi | lo] rows of q64"""
+        return self.split_queries(q64) if self.q_cols == 512 else q16
+
+    def _check_q(self, q16):
+        if q16.dim() != 2 or q16.shape[1] != self.q_cols or q16.dtype != torch.float16:
+            raise ValueError(f"query rows must be (N,{self.q_cols}) float16 in retrieval_precision="
+                             f"{self.retrieval_precision!r}, got {q16.dtype} {tuple(q16.shape)}")
+        return q16.shape[0]
 
     def raster_tables(self, lon_axis, lat_axis):
         """Per-axis tables of a lat/lon raster (encoder_raster.cu): the latitude factor of every harmonic for each
@@ -235,7 +274,7 @@ class RangeEngine:
             _lib.check(self.lib.range_encode_raster(self.ctx, tables["H"], tables["W"], _ptr(tables["buf"]), N, _ptr(ij),
                                                     _ptr(lonlat), _ptr(q64), _ptr(q16), _ptr(qxyz), _ptr(ws), ws.numel(),
                                                     _stream()))
-        return lonlat, q64, q16, qxyz
+        return lonlat, q64, self.query_rows(q64, q16), qxyz
 
     def raster_supported(self):
         """the separable raster encoder needs the analytic harmonics and the tensor-core SIREN"""
@@ -245,7 +284,7 @@ class RangeEngine:
         return self._workspace("ret", self.lib.range_retrieve_workspace_bytes(self.ctx, N))
 
     def retrieve(self, mode, q16, qxyz, temp, geo_temp, beta, O=None):
-        N = q16.shape[0]
+        N = self._check_q(q16)
         O = torch.empty(N, self.value_dim, dtype=torch.float32, device=self.device) if O is None else O
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
@@ -255,7 +294,7 @@ class RangeEngine:
         return O
 
     def retrieve_stats(self, mode, q16, qxyz, temp, geo_temp):
-        N = q16.shape[0]
+        N = self._check_q(q16)
         sums = torch.empty(N, 2, dtype=torch.float32, device=self.device)
         maxs = torch.empty(N, 2, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.index):
@@ -267,7 +306,7 @@ class RangeEngine:
     def retrieve_topk(self, mode, q16, qxyz, temp, geo_temp, beta, sums, k, perm=None):
         """the k largest retrieval weights of every query (sums from retrieve_stats): (idx (N,k) int32 device database
         rows, weight (N,k) fp32), descending; row n of the result at row perm[n] (perm from sort_queries)"""
-        N = q16.shape[0]
+        N = self._check_q(q16)
         idx = torch.empty(N, k, dtype=torch.int32, device=self.device)
         weight = torch.empty(N, k, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.index):
@@ -282,7 +321,7 @@ class RangeEngine:
         """retrieve_topk as one shard of an M-sharded database (sums: the global ones): entries are row0 + device row
         (rows of the whole sorted database with row0 = db.row_range[0]), k may exceed this shard's M (unfilled slots:
         entry -1, weight 0), row n of the result is query n"""
-        N = q16.shape[0]
+        N = self._check_q(q16)
         idx = torch.empty(N, k, dtype=torch.int32, device=self.device)
         weight = torch.empty(N, k, dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.index):
@@ -309,7 +348,7 @@ class RangeEngine:
         return idx, weight
 
     def retrieve_apply(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, O=None):
-        N = q16.shape[0]
+        N = self._check_q(q16)
         O = torch.empty(N, self.value_dim, dtype=torch.float32, device=self.device) if O is None else O
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
@@ -321,7 +360,7 @@ class RangeEngine:
     def retrieve_apply_concat(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, q64, out=None,
                               dtype=torch.float64, perm=None):
         """apply pass + concat in one call: (N,D+256) = [retrieved feature | q64], row n at out[perm[n]]"""
-        N = q16.shape[0]
+        N = self._check_q(q16)
         out = _new_out(N, dtype, self.device, self.value_dim) if out is None else out
         code = _out_code(out, self.value_dim)
         with torch.cuda.device(self.index):
@@ -335,7 +374,7 @@ class RangeEngine:
     def retrieve_concat(self, mode, q16, qxyz, temp, geo_temp, beta, q64, out=None, dtype=torch.float64, perm=None):
         """statistics + apply + concat in one call (unsharded database): (N,D+256) = [retrieved feature | q64], row n at
         out[perm[n]]"""
-        N = q16.shape[0]
+        N = self._check_q(q16)
         out = _new_out(N, dtype, self.device, self.value_dim) if out is None else out
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
@@ -359,7 +398,7 @@ class RangeEngine:
     def retrieve_apply_routed(self, mode, q16, qxyz, temp, geo_temp, beta, sums, maxs, route):
         """apply pass of an M-sharded database: this shard's partial rows (value_dim floats each) go straight into the
         owner ranks' receive buffers (route: _lib.Route with the mapped peer pointers of [P][slab][value_dim] buffers)"""
-        N = q16.shape[0]
+        N = self._check_q(q16)
         with torch.cuda.device(self.index):
             ws = self._ret_ws(N)
             _lib.check(self.lib.range_retrieve_apply_routed_values(

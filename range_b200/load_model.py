@@ -6,6 +6,7 @@
 """
 from argparse import Namespace
 
+from .engine import check_retrieval_precision
 from .range import LocationEncoder
 
 
@@ -19,11 +20,16 @@ def load_model(model_name='RANGE+', pretrained_path=None, device='cuda', **kwarg
     collective call: every rank passes its own queries; `db_merge='peer'|'reduce_scatter'`), `db_cache` (path of the
     prepared device layout: written on first use, validated against source and shard, read afterwards), `host_path`
     ('auto' | 'copy' | 'packed': how the float64 result reaches the host, range.py:_forward_host),
-    `out_dtype` (np.float64 like the reference, or np.float32: half the device->host bytes), `pinned_limit` (bytes),
-    `host_threads`.
+    `out_dtype` (np.float64 like the reference, or np.float32: half the device->host bytes), `retrieval_precision`
+    ('fp16', the default: Q.K^T and P'.V on fp16 operands, 11 significant bits of every query, key, weight and value;
+    or 'f16x3': every operand split into hi + lo fp16 and three tensor-core products per term, 22 significant bits at
+    about three times the retrieval's tensor work and twice the device memory of the database's keys and values -
+    for value vectors whose information sits below a large common offset, which fp16 rounds away; the location
+    columns are the same in both), `pinned_limit` (bytes), `host_threads`.
     """
     if pretrained_path is None:
         raise ValueError("Please provide the pretrained model path.")
+    check_retrieval_precision(kwargs.get('retrieval_precision', 'fp16'))
     if 'RANGE' in model_name:
         assert 'db_path' in kwargs, "db_path is required for RANGE model."
         db_path = kwargs.get('db_path')
@@ -33,7 +39,7 @@ def load_model(model_name='RANGE+', pretrained_path=None, device='cuda', **kwarg
     args = Namespace(location_model_name=model_name, pretrained_path=pretrained_path, device=device,
                      range_db=db_path, beta=beta)
     for k in ('chunk', 'db_shard', 'db_group', 'db_cache', 'db_merge', 'tail', 'taper', 'super_batch', 'host_path', 'out_dtype', 'pinned_limit',
-              'host_threads'):
+              'host_threads', 'retrieval_precision'):
         if k in kwargs:
             setattr(args, k, kwargs[k])
     model = LocationEncoder(args)

@@ -16,7 +16,7 @@ import torch.nn as nn
 from . import _lib
 from .checkpoint import load_satclip_location_encoder
 from .database import DeviceDatabase, open_npz, value_dim_of
-from .engine import RangeEngine, packed_row_bytes
+from .engine import RangeEngine, check_retrieval_precision, packed_row_bytes
 
 # one round of the producer/consumer apply kernel on 148 SMs: 24 units x 2 query tiles of 128
 ROUND_ROWS = 24 * 256
@@ -43,6 +43,9 @@ class LocationEncoder(nn.Module):
             print(f'Using RANGE+ with temperatures {self.args.temp} and {self.args.geo_temp}')
         else:
             raise ValueError('Unimplemented RANGE model')                                  # range.py:114
+        # arithmetic of Q.K^T and P'.V: 'fp16' operands, or 'f16x3' (hi + lo fp16, the database keeps its lo halves)
+        self.args.retrieval_precision = check_retrieval_precision(getattr(args, 'retrieval_precision', 'fp16'))
+        lo = self.args.retrieval_precision == 'f16x3'
         shard = getattr(args, 'db_shard', None)
         enc = load_satclip_location_encoder(args.pretrained_path) if isinstance(args.pretrained_path, str) \
             else args.pretrained_path
@@ -59,10 +62,10 @@ class LocationEncoder(nn.Module):
             # in-memory database, for the width of its values (a file's fingerprint already pins them)
             fp = DeviceDatabase.source_fingerprint(db)
             width = None if isinstance(db, (str, os.PathLike)) else value_dim_of(np.asarray(db['image_embeddings']))
-            ddb = DeviceDatabase.from_cache(cache, args.device, shard=shard, fingerprint=fp, value_dim=width)
+            ddb = DeviceDatabase.from_cache(cache, args.device, shard=shard, fingerprint=fp, value_dim=width, lo=lo)
         if ddb is None:
             db = open_npz(db) if isinstance(db, str) else db                              # range.py:78
-            ddb = DeviceDatabase(db, args.device, shard=shard)
+            ddb = DeviceDatabase(db, args.device, shard=shard, lo=lo)
             if cache is not None:
                 ddb.save_cache(cache, fingerprint=fp)
         # range.py:86 hard-codes 1024 + 256 (SatMAE features): here the width of the database's values + 256
@@ -72,7 +75,8 @@ class LocationEncoder(nn.Module):
             raise NotImplementedError(f'an M-sharded database (db_shard={tuple(shard)}) needs values whose width is a '
                                       f'multiple of 4 (512, 768, 1024, 2048, ...); this one has {ddb.value_dim}: load '
                                       f'it unsharded')
-        self.engine = RangeEngine(args.device, encoder=enc, database=ddb)
+        self.engine = RangeEngine(args.device, encoder=enc, database=ddb,
+                                  retrieval_precision=self.args.retrieval_precision)
         self.chunk = int(getattr(args, 'chunk', DEFAULT_CHUNK))
         self.tail = max(1, min(self.chunk, int(getattr(args, 'tail', DEFAULT_TAIL))))
         self.super_batch = max(self.chunk, int(getattr(args, 'super_batch', 1 << 20)) // self.chunk * self.chunk)
