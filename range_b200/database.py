@@ -22,6 +22,7 @@ range/range.py:213-238), so the rows are stored sorted along a cube-map Hilbert 
 tiles are then spatially compact, which lets the RANGE+ kernels skip the geographic term for tiles far from a
 query tile (include/range_b200.h: range_ctx_set_db_caps).
 """
+import copy
 import hashlib
 import math
 import os
@@ -369,6 +370,17 @@ class DeviceDatabase:
         self.xyz[:m, :3] = torch.from_numpy(np.ascontiguousarray(xyz)).to(dev)
         self.caps = torch.from_numpy(tile_caps(xyz)).to(dev)
         return self
+
+    def replicate(self, device):
+        """this layout on another device (or a second copy on the same one): the device tensors copied device to device,
+        the host-side fields (row order, sizes, vscale, value width, row range) shared"""
+        dev = torch.device(device)
+        rep = copy.copy(self)
+        rep.__dict__.pop("_order_t", None)
+        for name in ("Kh", "Vt", "xyz", "caps", "Kl", "Vtl"):
+            t = getattr(self, name, None)
+            setattr(rep, name, None if t is None else t.to(dev, copy=True))
+        return rep
 
     def file_rows(self, idx):
         """device rows (e.g. the entries RangeEngine.retrieve_topk returns) -> rows of the database file, so that

@@ -25,7 +25,13 @@ def load_model(model_name='RANGE+', pretrained_path=None, device='cuda', **kwarg
     or 'f16x3': every operand split into hi + lo fp16 and three tensor-core products per term, 22 significant bits at
     about three times the retrieval's tensor work and twice the device memory of the database's keys and values -
     for value vectors whose information sits below a large common offset, which fp16 rounds away; the location
-    columns are the same in both), `pinned_limit` (bytes), `host_threads`.
+    columns are the same in both), `pinned_limit` (bytes), `host_threads`, `devices` (several GPUs of this host for one
+    model: an int n = the first n visible GPUs, 'all', or a list of indices / 'cuda:i' strings whose first entry is the
+    primary device; None, the default, is `device` alone.  The database is prepared once on the primary and copied to the
+    others; every call of 2 x 6144 rows or more splits its rows into contiguous slabs, one per device, each computed by
+    the single-device code, and returns what it returns today - device-resident results on the primary.  A duplicate
+    entry is a second replica on the same GPU, run after the first: a way to test the path on one GPU, with no speed-up.
+    Not with `db_shard`: ValueError).
     """
     if pretrained_path is None:
         raise ValueError("Please provide the pretrained model path.")
@@ -39,7 +45,7 @@ def load_model(model_name='RANGE+', pretrained_path=None, device='cuda', **kwarg
     args = Namespace(location_model_name=model_name, pretrained_path=pretrained_path, device=device,
                      range_db=db_path, beta=beta)
     for k in ('chunk', 'db_shard', 'db_group', 'db_cache', 'db_merge', 'tail', 'taper', 'super_batch', 'host_path', 'out_dtype', 'pinned_limit',
-              'host_threads', 'retrieval_precision'):
+              'host_threads', 'retrieval_precision', 'devices'):
         if k in kwargs:
             setattr(args, k, kwargs[k])
     model = LocationEncoder(args)

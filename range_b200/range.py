@@ -47,6 +47,16 @@ class LocationEncoder(nn.Module):
         self.args.retrieval_precision = check_retrieval_precision(getattr(args, 'retrieval_precision', 'fp16'))
         lo = self.args.retrieval_precision == 'f16x3'
         shard = getattr(args, 'db_shard', None)
+        devices = getattr(args, 'devices', None)        # queries split over database replicas on several GPUs (devices.py)
+        device = args.device
+        if devices is not None:
+            held = args.range_db.shard if isinstance(args.range_db, DeviceDatabase) else shard
+            if held is not None and held[1] > 1:
+                raise ValueError(f'devices={devices!r} with an M-sharded database (db_shard={tuple(held)}): queries are '
+                                 f'split over local GPUs for a database that fits on one; shard it with one process per GPU')
+            from .devices import check_devices
+            devices = check_devices(devices)
+            device = devices[0]
         enc = load_satclip_location_encoder(args.pretrained_path) if isinstance(args.pretrained_path, str) \
             else args.pretrained_path
         cache = getattr(args, 'db_cache', None)        # optional: prepared device layout on disk (database.py)
@@ -62,10 +72,10 @@ class LocationEncoder(nn.Module):
             # in-memory database, for the width of its values (a file's fingerprint already pins them)
             fp = DeviceDatabase.source_fingerprint(db)
             width = None if isinstance(db, (str, os.PathLike)) else value_dim_of(np.asarray(db['image_embeddings']))
-            ddb = DeviceDatabase.from_cache(cache, args.device, shard=shard, fingerprint=fp, value_dim=width, lo=lo)
+            ddb = DeviceDatabase.from_cache(cache, device, shard=shard, fingerprint=fp, value_dim=width, lo=lo)
         if ddb is None:
             db = open_npz(db) if isinstance(db, str) else db                              # range.py:78
-            ddb = DeviceDatabase(db, args.device, shard=shard, lo=lo)
+            ddb = DeviceDatabase(db, device, shard=shard, lo=lo)
             if cache is not None:
                 ddb.save_cache(cache, fingerprint=fp)
         # range.py:86 hard-codes 1024 + 256 (SatMAE features): here the width of the database's values + 256
@@ -75,7 +85,7 @@ class LocationEncoder(nn.Module):
             raise NotImplementedError(f'an M-sharded database (db_shard={tuple(shard)}) needs values whose width is a '
                                       f'multiple of 4 (512, 768, 1024, 2048, ...); this one has {ddb.value_dim}: load '
                                       f'it unsharded')
-        self.engine = RangeEngine(args.device, encoder=enc, database=ddb,
+        self.engine = RangeEngine(device, encoder=enc, database=ddb,
                                   retrieval_precision=self.args.retrieval_precision)
         self.chunk = int(getattr(args, 'chunk', DEFAULT_CHUNK))
         self.tail = max(1, min(self.chunk, int(getattr(args, 'tail', DEFAULT_TAIL))))
@@ -93,6 +103,8 @@ class LocationEncoder(nn.Module):
             raise ValueError(f"host_path={self.host_path!r}: expected 'auto', 'copy' or 'packed'")
         self.pinned_limit = int(getattr(args, 'pinned_limit', 8 << 30))       # largest page-locked result, bytes
         local_ranks = max(1, int(os.environ.get('LOCAL_WORLD_SIZE', '1')))      # torchrun: ranks sharing this host
+        if devices is not None:                 # the GPUs of this process share the host's cores like ranks would
+            local_ranks *= len({d.index for d in devices})
         self.host_threads = int(getattr(args, 'host_threads', 0)) or max(1, min(16, (os.cpu_count() or 1) // local_ranks))
         self.group = getattr(args, 'db_group', None)       # torch.distributed group when the DB is M-sharded
         self.sharded = None
@@ -101,12 +113,24 @@ class LocationEncoder(nn.Module):
             self.sharded = ShardedRetriever(self.engine, self.group, merge=getattr(args, 'db_merge', 'peer'))
         self._copy_stream = None
         self.trace = None           # developer timeline of _forward_host: a list collects (rows, computed, copied) events
+        self.replicas = None
+        if devices is not None and len(devices) > 1:
+            from .devices import Replicas
+            self.replicas = Replicas(self, enc, devices)
         self.eval()
 
     def close(self):
-        """release the peer receive buffers of an M-sharded model (a collective call: every rank closes)"""
+        """release the peer receive buffers of an M-sharded model (a collective call: every rank closes) or the database
+        replicas of a model on several devices (later calls run on the primary device alone)"""
         if self.sharded is not None:
             self.sharded.close()
+        if self.replicas is not None:
+            self.replicas.close()
+            self.replicas = None
+
+    def _slabs(self, N):
+        """the slabs [lo, hi) of an N-row call split over the devices, or None when it runs on this model's engine"""
+        return None if self.replicas is None else self.replicas.slabs(N)
 
     # the reference calls model.to(device) after construction (load_model.py:50); tensors live in the engine
     def _apply(self, fn, recurse=True):
@@ -138,6 +162,9 @@ class LocationEncoder(nn.Module):
             coords = coords.to(eng.device, torch.float64).contiguous()
             return self.sharded.embed(self.location_model_name, coords, a.temp, float(getattr(a, 'geo_temp', 0.0)),
                                       getattr(a, 'beta', None), self._sorts(), out=out, out_dtype=out_dtype)
+        slabs = self._slabs(coords.shape[0])
+        if slabs is not None:
+            return self.replicas.embed(coords, slabs, out, out_dtype)
         perm = None
         if self._sorts():
             # spatial batching: the geo softmax is local, tiles of nearby queries skip far database tiles
@@ -160,6 +187,9 @@ class LocationEncoder(nn.Module):
         if self.sharded is not None:
             coords = torch.as_tensor(coords).to(eng.device, torch.float64).contiguous()
             return self.sharded.embed_sweep(coords, a.temp, a.geo_temp, self._sorts(), betas, out_dtype=out_dtype)
+        slabs = self._slabs(len(coords))
+        if slabs is not None:
+            return self.replicas.embed_sweep(torch.as_tensor(coords), slabs, betas, out_dtype)
         perm = None
         if self._sorts():
             coords, perm = eng.sort_queries(coords)
@@ -191,6 +221,9 @@ class LocationEncoder(nn.Module):
             rows, weight = self.sharded.neighbours(name, coords, a.temp, geo_temp, getattr(a, 'beta', None),
                                                    self._sorts(), k)
             return eng.db.file_rows_global(rows), weight
+        slabs = self._slabs(coords.shape[0])
+        if slabs is not None:
+            return self.replicas.neighbours(coords, slabs, k)
         perm = None
         if self._sorts():
             coords, perm = eng.sort_queries(coords)
@@ -329,6 +362,9 @@ class LocationEncoder(nn.Module):
         n = p1 - p0
         if self.sharded is not None:
             return self.embed(self._raster_lonlat(tables, p0, n), out=out, out_dtype=out_dtype)
+        slabs = self._slabs(n)
+        if slabs is not None:
+            return self.replicas.embed_raster(tables, p0, slabs, out, out_dtype)
         perm = None
         if tables['buf'] is None:              # no separable evaluation: the per-point encoder on the materialised coordinates
             ij = self._raster_ij(tables['W'], p0, p1)
@@ -360,7 +396,7 @@ class LocationEncoder(nn.Module):
             raise ValueError(f'out must be a writable C-contiguous float64 (rows, {W}) array')
         return self._forward_host(p1 - p0, raster=tables, result=out, raster_p0=p0)
 
-    def _forward_host(self, N, coords=None, raster=None, result=None, raster_p0=0):
+    def _forward_host(self, N, coords=None, raster=None, result=None, raster_p0=0, host=None):
         """model(locs) -> numpy float64 (N,D+256) (range/range.py:222,240).  Two ways to hand the rows to the host:
 
         'copy'    chunk by chunk into device buffers; every chunk's float64 rows travel to the page-locked result on a
@@ -372,6 +408,8 @@ class LocationEncoder(nn.Module):
                   memory for any N, 40 % fewer PCIe bytes, but the host cores must keep up (measured on the 16-core
                   1-GPU box: 6.3 M rows/s with 16 threads, 2.2 M queries/s end to end against 2.9 M for 'copy').
         'auto'    'copy' while the result fits `pinned_limit` (8 GB), else 'packed'.
+        On several devices each writes its slab of the one result: rows of `result` ('packed') or of the page-locked
+        `host` tensor ('copy').
         (Measured and dropped: letting the apply kernel's epilogue store straight into the mapped page-locked result -
         stores from the SMs to host memory run at ~6 GB/s and stall the consumers: 170 ms per 100 000 queries.)"""
         eng = self.engine
@@ -381,8 +419,8 @@ class LocationEncoder(nn.Module):
         row_bytes = W * (4 if tdtype == torch.float32 else 8)
         if result is not None:
             path = 'packed'
-        elif tdtype == torch.float32:
-            path = 'copy'                          # nothing to widen: the rows are copied as they are
+        elif tdtype == torch.float32 or host is not None:
+            path = 'copy'                          # nothing to widen, or a slab of a multi-device call's 'copy' result
         elif path == 'auto':
             path = 'copy' if N * row_bytes <= self.pinned_limit else 'packed'
         if self.sharded is not None:            # collective: distributed.py chunks (every rank must take the same steps)
@@ -400,9 +438,14 @@ class LocationEncoder(nn.Module):
         if path == 'packed':
             result = np.empty((N, W), dtype=np.float64) if result is None else result
         else:
-            host = torch.empty((N, W), dtype=tdtype, pin_memory=True)
+            host = torch.empty((N, W), dtype=tdtype, pin_memory=True) if host is None else host
             result = host.numpy()
         if N == 0:
+            return result
+        slabs = self._slabs(N)
+        if slabs is not None:
+            self.replicas.forward_host(slabs, coords, raster, raster_p0, result if path == 'packed' else None,
+                                       host if path == 'copy' else None)
             return result
         with torch.cuda.device(eng.index):
             if raster is None:
